@@ -1,6 +1,6 @@
 """Benchmark of the caption-generation hot path on BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): ViT-B/32 + 8-layer Transformer
@@ -23,6 +23,10 @@ replicated weights (weak scaling); the only collective is the final all-gather o
 The default line (N = 1, config 2) also carries `other_configs`: short child runs (3 timed steps each) of BASELINE.json's
 configs 3 / 4 / 5 on the same GPU -- context, never part of `value` (--no-other-configs skips them).
 
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0's share) as DIR/<name>.npy in float32:
+tokens, lengths and, for beam search, scores (token ids and lengths are exact in float32).  Weights, images and sampling
+seeds are fixed, so two builds run with the same arguments can be compared output for output.
+
 --config selects another BASELINE.json configuration (the default, 2, is the one the metric is quoted on and the only one
 the CPU arm covers): 3 = nucleus sampling (top_p 0.9, temperature 1.0), batch 256; 4 = beam 5, 102 images per step (two
 micro-batches of 51 = 255 rows, Engine.caption_dataset); 5 = GPT-J-6B + 4096-wide mapper, top_p 0.9, 16 images per GPU (128 on 8).
@@ -41,6 +45,8 @@ _OUT = sys.stdout   # main() points it at the original stdout and redirects fd 1
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree bench.py runs from may be read-only: nothing is written there
+DUMP_LIMIT = 64 << 20            # bytes, all --dump-outputs arrays together
 
 METRIC = "captions/sec (GPT2-XL, prefix 40, 32 tok)"
 UNIT = "captions/s"
@@ -312,7 +318,8 @@ def other_configs_leg():
         try:
             r = subprocess.run([sys.executable, os.path.abspath(__file__), "--config", str(cfg_id), "--steps", "3", "--warmup", "3",
                                 "--no-cpu-baseline"], capture_output=True, text=True, timeout=limit,
-                               env={k: v for k, v in os.environ.items() if k not in ("RANK", "WORLD_SIZE", "LOCAL_RANK")})
+                               env=dict({k: v for k, v in os.environ.items() if k not in ("RANK", "WORLD_SIZE", "LOCAL_RANK")},
+                                        PYTHONDONTWRITEBYTECODE="1"))
             j = json.loads(r.stdout.strip().splitlines()[-1])
             out["config%d" % cfg_id] = {
                 "metric": j["metric"], "workload": j["config"]["workload"], "value": j["value"], "unit": j["unit"],
@@ -322,6 +329,18 @@ def other_configs_leg():
         except Exception as e:   # noqa: BLE001 -- context only
             out["config%d" % cfg_id] = {"unavailable": "%s: %s" % (type(e).__name__, str(e)[:200])}
     return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` (name -> tensor, None skipped) as out_dir/<name>.npy in float32."""
+    import numpy as np
+    host = {k: v.detach().cpu().float().numpy() for k, v in arrays.items() if v is not None}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
@@ -335,7 +354,11 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS))
     ap.add_argument("--no-other-configs", action="store_true",
                     help="skip the short runs of BASELINE.json's configs 3 / 4 / 5 that the default N=1 line reports under `other_configs`")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0: tokens, lengths, beam scores) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     C_ = CONFIGS[args.config]
     BATCH = C_["batch"]
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
@@ -379,10 +402,10 @@ def main():
         return eng.caption_dataset(imgs, params, first_row_id=rank * BATCH)
 
     def step_resident():
-        tokens, lengths, _ = caption(images)
+        tokens, lengths, scores = caption(images)
         if world > 1:
             dist.all_gather(gathered, tokens)      # the only collective: final captions
-        return tokens, lengths
+        return tokens, lengths, scores
 
     def step_e2e():
         dev_images = host_images.to(dev, non_blocking=True)
@@ -422,7 +445,7 @@ def main():
     profiled = os.environ.get("CCB_BENCH_PROFILE") == "1"   # `ncu --profile-from-start off`: the launch list of the timed region
     if profiled:
         torch.cuda.profiler.start()
-    ms_total, (tokens, lengths) = timed(step_resident, args.steps)
+    ms_total, (tokens, lengths, scores) = timed(step_resident, args.steps)
     if profiled:
         torch.cuda.profiler.stop()
     launches = eng.launch_count - l0
@@ -434,6 +457,8 @@ def main():
         step_e2e()
     e2e_ms_total, _ = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tokens": tokens, "lengths": lengths, "scores": scores})
 
     ms_per_step = ms_total / args.steps
     value = world * BATCH / (ms_per_step * 1e-3)
