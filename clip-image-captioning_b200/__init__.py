@@ -6,10 +6,10 @@ creating an `Engine` does, and there is no CPU fallback.
 """
 from . import _lib
 from ._lib import GenParams, ModelDesc
-from .engine import Engine, EngineConfig
+from .engine import CLIP_TOWERS, Engine, EngineConfig
 from . import evaluate_model, inference, lms, model, sampling, sharding, synthetic
 from .lms import GPT2, GPTJ, IdTokenizer
 from .model import CLIPCaptionModel, CLIPCaptionPrefixOnly
 
-__all__ = ["Engine", "EngineConfig", "GenParams", "ModelDesc", "CLIPCaptionModel", "CLIPCaptionPrefixOnly", "GPT2", "GPTJ",
+__all__ = ["CLIP_TOWERS", "Engine", "EngineConfig", "GenParams", "ModelDesc", "CLIPCaptionModel", "CLIPCaptionPrefixOnly", "GPT2", "GPTJ",
            "IdTokenizer", "inference", "evaluate_model", "sampling", "sharding", "synthetic", "lms", "model", "_lib"]

@@ -2,7 +2,8 @@
 //  * attention_prefill: full attention over a short sequence (S <= 256) for one (batch, head) per CTA.  Serves
 //    the ViT (S=50, hd=64, non-causal), the prefix mapper (S=clip_len+P, hd=d/8, non-causal; reference
 //    layers/MultiHeadAttention.py:24-41) and the LM prefill (causal; HF GPT2Attention / GPTJAttention), where
-//    it also writes K/V into the paged cache.
+//    it also writes K/V into the paged cache.  S > 256 (ViT-L towers, the all-features mapper over them) is handed to the
+//    tcgen05 kernel of attention_long.cu.
 //  * attention_decode: one query token per row against the paged KV cache; memory-bound, 16-byte loads,
 //    online softmax, 4 warps per (row, head) each striding over the context, merged through shared memory.
 #include <stdlib.h>
@@ -950,7 +951,11 @@ int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, f
                       const KvCache* cache, int layer, const int* block_table, int pos0, int rotary_dim,
                       const uint8_t* key_mask, cudaStream_t s) {
   if (B <= 0 || S <= 0) return 0;
-  if (S > 256 || hd % 2) return (int)cudaErrorInvalidValue;
+  if (S > 256) {   // the long-sequence tcgen05 kernel (attention_long.cu): plain non-causal attention only
+    if (causal || cache || rotary_dim || key_mask || hd % 8 || hd > 256) return (int)cudaErrorInvalidValue;
+    return attention_prefill_long(qkv, out, B, S, H, hd, scale, s);
+  }
+  if (hd % 2) return (int)cudaErrorInvalidValue;
   static const bool use_mma = [] {
     const char* e = getenv("CCB_ATTN_MMA");
     return !(e && e[0] == '0');

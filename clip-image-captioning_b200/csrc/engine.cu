@@ -252,14 +252,17 @@ int block_forward(ccb_ctx* c, const Block& b, int M, const BlockShape& sh, AttnF
   return 0;
 }
 
+// K of the patch-embedding GEMM: 3 * patch^2 rounded up to the GEMM's 64-element K step (patch 14: 588 -> 640)
+inline int vit_patch_k(int patch) { return (3 * patch * patch + 63) / 64 * 64; }
+
 int vit_forward(ccb_ctx* c, const void* images, int dtype, int B, float* feat_out, cudaStream_t s, bool all_tokens = false) {
   const ccb_model_desc& D = c->desc;
   if (!D.vit_present) return fail(c, "context was created without an image encoder");
   if (B <= 0 || B > D.max_images) return fail(c, "vit_encode: B=%d outside [1, max_images=%d]", B, D.max_images);
   const int g = D.vit_image / D.vit_patch, np = g * g, w = D.vit_width, S = np + 1, M = B * S;
-  const int kdim = 3 * D.vit_patch * D.vit_patch;
-  RUN(vit_patchify(images, dtype, B, 3, D.vit_image, D.vit_image, D.vit_patch, c->patches, s));
-  RUN(linear(c, c->patches, kdim, B * np, c->vit_conv, CCB_ACT_NONE, nullptr, 0, c->patch_emb, w, 0, s));
+  const int kpad = vit_patch_k(D.vit_patch);
+  RUN(vit_patchify(images, dtype, B, 3, D.vit_image, D.vit_image, D.vit_patch, c->patches, kpad, s));
+  RUN(linear(c, c->patches, kpad, B * np, c->vit_conv, CCB_ACT_NONE, nullptr, 0, c->patch_emb, w, 0, s));
   RUN(vit_assemble_lnpre(c->patch_emb, c->vit_cls, c->vit_pos, c->vit_ln_pre.g, c->vit_ln_pre.b, 1e-5f, c->h, B, np, w, s));
   BlockShape sh{w, 4 * w, CCB_ACT_QUICKGELU, 1e-5f, false};
   const int H = D.vit_heads, hd = w / H;
@@ -826,8 +829,17 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
                                             D.map_hidden % 64 || D.map_dim_clip % 64))
     return fail(nullptr, "ccb_create: bad mapper dimensions");
   if (D.map_kind == CCB_MAP_MLP && (D.map_hidden % 64 || D.map_dim_clip % 64)) return fail(nullptr, "ccb_create: bad MLP mapper dimensions");
-  if (D.vit_present && (D.vit_width % 64 || D.vit_width % D.vit_heads || D.vit_image % D.vit_patch || D.vit_patch % 8))
+  // any patch size that divides the image (patch 14: the K of the patch GEMM is padded, see vit_patch_k)
+  if (D.vit_present && (D.vit_width % 64 || D.vit_heads <= 0 || D.vit_width % D.vit_heads || D.vit_patch <= 0 || D.vit_image % D.vit_patch))
     return fail(nullptr, "ccb_create: bad ViT dimensions");
+  if (D.vit_present && (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1 > 256 &&
+      ((D.vit_width / D.vit_heads) % 8 || D.vit_width / D.vit_heads > 256))
+    return fail(nullptr, "ccb_create: ViT of %d tokens with head_dim %d: attention over more than 256 tokens needs head_dim %% 8 == 0 "
+                "and <= 256", (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1, D.vit_width / D.vit_heads);
+  if ((D.map_kind == CCB_MAP_TRANSFORMER || D.map_kind == CCB_MAP_TRANSFORMER_ALL) && D.map_clip_len + D.map_prefix_len > 256 &&
+      ((D.lm_d / D.map_heads) % 8 || D.lm_d / D.map_heads > 256))
+    return fail(nullptr, "ccb_create: mapper sequence of %d tokens with head_dim %d: attention over more than 256 tokens needs "
+                "head_dim %% 8 == 0 and <= 256", D.map_clip_len + D.map_prefix_len, D.lm_d / D.map_heads);
 
   if (D.text_present && (D.text_width % 64 || D.text_heads <= 0 || D.text_width % D.text_heads || (D.text_width / D.text_heads) % 16 ||
                          D.text_ctx <= 0 || D.text_ctx > 128 || D.text_vocab <= 0 || D.text_out <= 0 || D.max_texts <= 0))
@@ -962,8 +974,9 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   if (D.vit_present) {
     const int w = D.vit_width, g = D.vit_image / D.vit_patch, np = g * g, kdim = 3 * D.vit_patch * D.vit_patch;
     vit_S = np + 1;
-    make_linear(c, a, c->vit_conv, w, kdim, false);
-    add_slot(c, "visual.conv1.weight", WeightSlot::MATRIX, c->vit_conv.w, w, kdim, kdim);
+    // conv1 as a [w, kdim] matrix at the padded pitch of the patch rows; the pad columns stay zero (the arena is cleared)
+    make_linear(c, a, c->vit_conv, w, vit_patch_k(D.vit_patch), false);
+    add_slot(c, "visual.conv1.weight", WeightSlot::MATRIX, c->vit_conv.w, w, kdim, vit_patch_k(D.vit_patch));
     c->vit_cls = a.arr<float>(w);
     c->vit_pos = a.arr<float>(static_cast<size_t>(vit_S) * w);
     add_slot(c, "visual.class_embedding", WeightSlot::VECTOR_F32, c->vit_cls, w, 1, 1);
@@ -1047,8 +1060,8 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   c->mlp = a.arr<bf16>(Mz * c->hidden_max);
   if (D.lm_arch == CCB_LM_GPTJ) c->attmlp = a.arr<bf16>(static_cast<size_t>(c->max_rows) * 5 * d);
   if (D.vit_present) {
-    const int g = D.vit_image / D.vit_patch, np = g * g, kdim = 3 * D.vit_patch * D.vit_patch;
-    c->patches = a.arr<bf16>(static_cast<size_t>(D.max_images) * np * kdim);
+    const int g = D.vit_image / D.vit_patch, np = g * g;
+    c->patches = a.arr<bf16>(static_cast<size_t>(D.max_images) * np * vit_patch_k(D.vit_patch));
     c->patch_emb = a.arr<float>(static_cast<size_t>(D.max_images) * np * D.vit_width);
   }
   const int dc = std::max(D.map_dim_clip, D.vit_present ? D.vit_out : 0);

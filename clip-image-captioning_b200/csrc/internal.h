@@ -90,9 +90,10 @@ int layernorm_f32_bf16(const float* x, long long ldx, const float* gamma, const 
 // same but also writes the normalised row as f32 (final ViT ln_post -> proj input kept bf16; f32 copy for debug)
 int layernorm_f32_f32(const float* x, long long ldx, const float* gamma, const float* beta, float eps, float* y,
                       long long ldy, int rows, int d, cudaStream_t s);
-// ViT: NCHW image (f32 or f16 or bf16) -> im2col patches bf16 [B*gh*gw, 3*ps*ps] in conv-weight order (c, ky, kx)
+// ViT: NCHW image (f32 or f16 or bf16) -> im2col patches bf16 [B*gh*gw, 3*ps*ps] in conv-weight order (c, ky, kx), rows at
+// pitch ldp >= 3*ps*ps (columns past 3*ps*ps are written as zeros)
 int vit_patchify(const void* images, int img_dtype /*0 f32, 1 f16, 2 bf16*/, int B, int C, int H, int W, int ps,
-                 bf16* patches, cudaStream_t s);
+                 bf16* patches, int ldp, cudaStream_t s);
 // ViT: x[b,0,:] = cls + pos[0]; x[b,1+p,:] = patch_emb[b*np+p,:] + pos[1+p]; then ln_pre in place -> f32 stream
 int vit_assemble_lnpre(const float* patch_emb, const float* cls, const float* pos, const float* g, const float* b,
                        float eps, float* x, int B, int np, int d, cudaStream_t s);
@@ -133,13 +134,16 @@ struct KvCache {
   size_t layer_stride() const { return 2ull * num_pages * H * page_tokens * hd; }
   size_t kv_stride() const { return 1ull * num_pages * H * page_tokens * hd; }
 };
-// Full attention over a short sequence held in one fused qkv buffer [B*S, 3*d] (q | k | v, head h at h*hd).
+// Full attention over a sequence held in one fused qkv buffer [B*S, 3*d] (q | k | v, head h at h*hd); S > 256 only for
+// non-causal attention without cache, rotary or key mask, with hd % 8 == 0 and hd <= 256.
 // causal=0: ViT / mapper; causal=1: LM prefill, which also stores K/V into cache pages through block_table
 // ([B, max_pages_per_row] int32) at positions pos0..pos0+S-1 and (GPT-J) applies rotary to q/k first.
 // key_mask: optional [B, S] uint8, 0 = key may not be attended (HF attention_mask).
 int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, float scale, int causal,
                       const KvCache* cache, int layer, const int* block_table, int pos0, int rotary_dim,
                       const uint8_t* key_mask, cudaStream_t s);
+// S > 256 part of attention_prefill (attention_long.cu): non-causal, unmasked, no cache / rotary, hd % 8 == 0, hd <= 256
+int attention_prefill_long(const bf16* qkv, bf16* out, int B, int S, int H, int hd, float scale, cudaStream_t s);
 // One new token per row: appends this step's k/v (from qkv [B, 3*d]) at position ctx_len[b] and attends over
 // positions [0, ctx_len[b]] through the block table. ctx_len is device memory (graph-replay friendly).  `out` rows have pitch ldo
 // (elements): H * hd, or wider when the output lands in the [att | mlp] operand of GPT-J's fused out_proj + fc_out GEMM.

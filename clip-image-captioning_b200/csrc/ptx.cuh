@@ -122,7 +122,26 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
                : "r"(taddr)
                : "memory");
 }
+// 32 lanes x 16 consecutive fp32 columns
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32"
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32"
+      " [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
+      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // UMMA shared-memory descriptor for a K-major bf16 tile stored as 128-byte rows with the 128B swizzle
 // (exactly what a TMA box of {64 elements, rows} with CU_TENSOR_MAP_SWIZZLE_128B writes):
@@ -135,6 +154,17 @@ __device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(1024 >> 4) << 32;    // stride byte offset
   d |= static_cast<uint64_t>(1) << 46;            // descriptor version (Blackwell)
   d |= static_cast<uint64_t>(2) << 61;            // SWIZZLE_128B
+  return d;
+}
+// The same tile read as an MN-major operand (e.g. V [keys][dims] as the B operand of P.V, N = dims, K = keys): 128-byte rows
+// along K, 8-row groups SBO = 1024 B apart, successive 64-element blocks along N `lbo` bytes apart.
+__device__ __forceinline__ uint64_t umma_desc_mn_sw128(uint32_t smem_addr, uint32_t lbo) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
+  d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFF) << 16;
+  d |= static_cast<uint64_t>(1024 >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
 // Instruction descriptor, kind::f16: D=f32, A=B=bf16, both K-major, shape M x N (K fixed at 16).

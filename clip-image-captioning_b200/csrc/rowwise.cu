@@ -198,6 +198,30 @@ __global__ void __launch_bounds__(256) patchify_kernel(const InT* __restrict__ i
   }
 }
 
+// Patch sizes whose row is not a multiple of 8 pixels (ViT-L/14: 14): one element per thread, rows written at pitch
+// ldp >= kdim (the GEMM's K, a multiple of 64) with zeros in the pad columns.
+template <typename InT>
+__global__ void __launch_bounds__(256) patchify_any_kernel(const InT* __restrict__ img, int B, int C, int H, int W, int ps,
+                                                           int ldp, bf16* __restrict__ patches) {
+  const int gw = W / ps, gh = H / ps;
+  const int kdim = C * ps * ps;
+  const long long total = static_cast<long long>(B) * gh * gw * ldp;
+  for (long long e = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; e < total;
+       e += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int col = static_cast<int>(e % ldp);
+    const long long prow = e / ldp;
+    float v = 0.f;
+    if (col < kdim) {
+      const int px = static_cast<int>(prow % gw);
+      const int py = static_cast<int>((prow / gw) % gh);
+      const int b = static_cast<int>(prow / (gw * gh));
+      const int kx = col % ps, ky = (col / ps) % ps, c = col / (ps * ps);
+      v = to_f32<InT>(img[((static_cast<long long>(b) * C + c) * H + (py * ps + ky)) * W + px * ps + kx]);
+    }
+    patches[e] = __float2bfloat16_rn(v);
+  }
+}
+
 
 // ---------------------------------------------------------------- weight ingestion (cast / transpose)
 template <typename InT>
@@ -426,10 +450,26 @@ int layernorm_f32_f32(const float* x, long long ldx, const float* gamma, const f
   return 0;
 }
 
-int vit_patchify(const void* images, int img_dtype, int B, int C, int H, int W, int ps, bf16* patches,
+int vit_patchify(const void* images, int img_dtype, int B, int C, int H, int W, int ps, bf16* patches, int ldp,
                  cudaStream_t s) {
   if (B <= 0) return 0;
-  if (ps % 8 || H % ps || W % ps) return (int)cudaErrorInvalidValue;
+  if (ps <= 0 || H % ps || W % ps || ldp < C * ps * ps) return (int)cudaErrorInvalidValue;
+  if (ps % 8 || ldp != C * ps * ps) {
+    const long long total = static_cast<long long>(B) * (H / ps) * (W / ps) * ldp;
+    int blocks = static_cast<int>((total + 255) / 256);
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    if (img_dtype == 0)
+      patchify_any_kernel<float><<<blocks, 256, 0, s>>>(static_cast<const float*>(images), B, C, H, W, ps, ldp, patches);
+    else if (img_dtype == 1)
+      patchify_any_kernel<__half><<<blocks, 256, 0, s>>>(static_cast<const __half*>(images), B, C, H, W, ps, ldp, patches);
+    else if (img_dtype == 2)
+      patchify_any_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(static_cast<const __nv_bfloat16*>(images), B, C, H, W, ps, ldp,
+                                                                patches);
+    else
+      return (int)cudaErrorInvalidValue;
+    CCB_LAUNCH_CHECK();
+    return 0;
+  }
   const long long total8 = static_cast<long long>(B) * (H / ps) * (W / ps) * C * ps * ps / 8;
   int blocks = static_cast<int>((total8 + 255) / 256);
   if (blocks > 148 * 16) blocks = 148 * 16;

@@ -13,6 +13,21 @@ from . import _lib
 from ._lib import GenParams, ModelDesc
 
 
+# The OpenAI CLIP ViT towers by their `clip.load` name (the reference picks its tower that way, inference.py:419): the
+# vision tower (image, patch, width, layers, heads, output) and the matching text tower, as published in
+# openai/CLIP clip/model.py `build_model` (heads = width // 64) and the HF `openai/clip-vit-*` configs.
+CLIP_TOWERS = {
+    "ViT-B/32": dict(vit_image=224, vit_patch=32, vit_width=768, vit_layers=12, vit_heads=12, vit_out=512,
+                     text_width=512, text_layers=12, text_heads=8, text_out=512),
+    "ViT-B/16": dict(vit_image=224, vit_patch=16, vit_width=768, vit_layers=12, vit_heads=12, vit_out=512,
+                     text_width=512, text_layers=12, text_heads=8, text_out=512),
+    "ViT-L/14": dict(vit_image=224, vit_patch=14, vit_width=1024, vit_layers=24, vit_heads=16, vit_out=768,
+                     text_width=768, text_layers=12, text_heads=12, text_out=768),
+    "ViT-L/14@336px": dict(vit_image=336, vit_patch=14, vit_width=1024, vit_layers=24, vit_heads=16, vit_out=768,
+                           text_width=768, text_layers=12, text_heads=12, text_out=768),
+}
+
+
 @dataclass
 class EngineConfig:
     """Shapes of the three networks on the path and the capacities of one context.
@@ -59,6 +74,20 @@ class EngineConfig:
     max_ctx: int = 80
     max_lm_tokens: int = 0           # 0 -> max_images * max_ctx
     page_tokens: int = 16
+
+    @classmethod
+    def for_clip(cls, name: str, **overrides) -> "EngineConfig":
+        """EngineConfig with the image and text towers of `clip.load(name)` ("ViT-B/32", "ViT-B/16", "ViT-L/14",
+        "ViT-L/14@336px"); the mapper takes the tower's output width (`map_dim_clip`) and, with the all-features mapper,
+        one token per ViT token (`map_clip_len` = 1 + patches).  `overrides` win."""
+        if name not in CLIP_TOWERS:
+            raise ValueError("unknown CLIP tower %r (known: %s)" % (name, ", ".join(CLIP_TOWERS)))
+        kw = dict(CLIP_TOWERS[name])
+        kw["map_dim_clip"] = kw["vit_out"]
+        if overrides.get("map_kind", cls.map_kind) == "transformer_all":
+            kw["map_clip_len"] = (kw["vit_image"] // kw["vit_patch"]) ** 2 + 1
+        kw.update(overrides)
+        return cls(**kw)
 
     def desc(self) -> ModelDesc:
         d = ModelDesc()
