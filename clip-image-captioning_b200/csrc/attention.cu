@@ -945,31 +945,66 @@ __global__ void __launch_bounds__(kWideThreads) attention_decode_wide_kernel(
   }
 }
 
+// CCB_ATTN_MMA=0 sends every S <= 256 shape to the scalar kernel, CCB_ATTN_UMMA=0 the head_dim-64 S <= 64 ones to mma.sync
+bool attn_use_mma() {
+  static const bool on = [] {
+    const char* e = getenv("CCB_ATTN_MMA");
+    return !(e && e[0] == '0');
+  }();
+  return on;
+}
+bool attn_use_umma() {
+  static const bool on = [] {
+    const char* e = getenv("CCB_ATTN_UMMA");
+    return !(e && e[0] == '0');
+  }();
+  return on;
+}
+bool attn_mma_wide(int S, int hd, int rotary_dim) {   // head_dim 264..512 on mma.sync (Q fragments streamed)
+  return attn_use_mma() && S <= 80 && hd % 8 == 0 && hd > 256 && hd <= 512 && rotary_dim == 0;
+}
+bool attn_mma(int S, int hd, int rotary_dim) {
+  return attn_use_mma() && S <= 128 && hd % 8 == 0 && hd <= 256 && rotary_dim % 2 == 0;
+}
+// dynamic shared memory of the scalar kernel: K (padded rows) and V of the head, per-warp q row and probability row
+size_t scalar_prefill_smem(int S, int hd) {
+  return (static_cast<size_t>(S) * (hd / 2 + 1) + static_cast<size_t>(S) * (hd / 2) + 1) * 4 +
+         static_cast<size_t>(kPrefillWarps) * (hd + S) * 4;
+}
+constexpr size_t kScalarPrefillSmemCap = 200 * 1024;
+
 }  // namespace
+
+const char* attention_prefill_unsupported(int S, int hd, int causal, bool cache, int rotary_dim, bool key_mask) {
+  if (S <= 0) return nullptr;
+  if (hd <= 0 || hd % 2) return "head_dim must be positive and even";
+  if (S > 256) {   // the long-sequence tcgen05 kernel: plain non-causal attention only
+    if (causal || cache || rotary_dim || key_mask)
+      return "above 256 tokens only non-causal attention without KV cache, rotary or key mask is supported";
+    if (hd % 8 || hd > 256) return "above 256 tokens head_dim must be a multiple of 8 and at most 256";
+    return nullptr;
+  }
+  if (attn_use_mma() && attn_use_umma() && hd == 64 && S <= 64 && rotary_dim == 0) return nullptr;
+  if (attn_mma_wide(S, hd, rotary_dim) || attn_mma(S, hd, rotary_dim)) return nullptr;
+  if (scalar_prefill_smem(S, hd) > kScalarPrefillSmemCap)
+    return "the scalar attention kernel would need more than its 200 KB of shared memory (K and V of the whole sequence)";
+  return nullptr;
+}
 
 int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, float scale, int causal,
                       const KvCache* cache, int layer, const int* block_table, int pos0, int rotary_dim,
                       const uint8_t* key_mask, cudaStream_t s) {
   if (B <= 0 || S <= 0) return 0;
-  if (S > 256) {   // the long-sequence tcgen05 kernel (attention_long.cu): plain non-causal attention only
-    if (causal || cache || rotary_dim || key_mask || hd % 8 || hd > 256) return (int)cudaErrorInvalidValue;
-    return attention_prefill_long(qkv, out, B, S, H, hd, scale, s);
-  }
-  if (hd % 2) return (int)cudaErrorInvalidValue;
-  static const bool use_mma = [] {
-    const char* e = getenv("CCB_ATTN_MMA");
-    return !(e && e[0] == '0');
-  }();
-  static const bool use_umma = [] {
-    const char* e = getenv("CCB_ATTN_UMMA");
-    return !(e && e[0] == '0');
-  }();
-  if (use_mma && use_umma && hd == 64 && S <= 64 && rotary_dim == 0) {   // tcgen05 / TMEM path (ViT, GPT-2 prefill)
+  // the shapes no kernel holds are rejected here, by the same predicate ccb_create and the LM entry points check
+  if (attention_prefill_unsupported(S, hd, causal, cache != nullptr, rotary_dim, key_mask != nullptr))
+    return (int)cudaErrorInvalidValue;
+  if (S > 256) return attention_prefill_long(qkv, out, B, S, H, hd, scale, s);   // attention_long.cu
+  if (attn_use_mma() && attn_use_umma() && hd == 64 && S <= 64 && rotary_dim == 0) {   // tcgen05 / TMEM path (ViT, GPT-2 prefill)
     KvCache c;
     if (cache) c = *cache;
     return launch_prefill_umma(qkv, out, B, S, H, scale, causal, c, layer, block_table, pos0, cache != nullptr ? 1 : 0, key_mask, s);
   }
-  if (use_mma && S <= 80 && hd % 8 == 0 && hd > 256 && hd <= 512 && rotary_dim == 0) {
+  if (attn_mma_wide(S, hd, rotary_dim)) {
     // head_dim 512 (the 4096-wide mapper of config 5): K / V of 80 keys fill 166 KB, Q fragments are streamed
     KvCache c;
     if (cache) c = *cache;
@@ -977,7 +1012,7 @@ int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, f
       return launch_prefill_mma<10, 32, true>(qkv, out, B, S, H, hd, scale, causal, c, layer, block_table, pos0, 0, key_mask, rotary_dim, s);
     return launch_prefill_mma<10, 32>(qkv, out, B, S, H, hd, scale, causal, c, layer, block_table, pos0, 1, key_mask, rotary_dim, s);
   }
-  if (use_mma && S <= 128 && hd % 8 == 0 && hd <= 256 && rotary_dim % 2 == 0) {
+  if (attn_mma(S, hd, rotary_dim)) {
     KvCache c;
     if (cache) c = *cache;
     const int wc = cache != nullptr ? 1 : 0;
@@ -990,16 +1025,15 @@ int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, f
     if (nt <= 10) return dispatch_prefill_mma_ks<10>(ks, qkv, out, B, S, H, hd, scale, causal, c, layer, block_table, pos0, wc, key_mask, rotary_dim, s);
     return dispatch_prefill_mma_ks<16>(ks, qkv, out, B, S, H, hd, scale, causal, c, layer, block_table, pos0, wc, key_mask, rotary_dim, s);
   }
-  const size_t smem = (static_cast<size_t>(S) * (hd / 2 + 1) + static_cast<size_t>(S) * (hd / 2) + 1) * 4 +
-                      static_cast<size_t>(kPrefillWarps) * (hd + S) * 4;
-  if (smem > 200 * 1024) return (int)cudaErrorInvalidValue;
+  // the scalar kernel: every other shape up to 256 tokens (the predicate above checked its shared memory)
+  const size_t smem = scalar_prefill_smem(S, hd);
   static size_t configured_dev[kMaxDevices] = {};
   size_t& configured = configured_dev[current_device_slot()];
   if (smem > 48 * 1024 && smem > configured) {
     cudaError_t e = cudaFuncSetAttribute(attention_prefill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         200 * 1024);
+                                         static_cast<int>(kScalarPrefillSmemCap));
     if (e != cudaSuccess) return (int)e;
-    configured = 200 * 1024;
+    configured = kScalarPrefillSmemCap;
   }
   KvCache c;
   if (cache) c = *cache;

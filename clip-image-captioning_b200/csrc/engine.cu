@@ -660,7 +660,8 @@ int generate_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const float* em
   if (beam < 1 || beam > D.max_beam || beam > 8) return fail(c, "generate: beam_size=%d outside [1, max_beam=%d]", beam, D.max_beam);
   if (T <= 0 || S0 <= 0 || S0 + T > D.max_ctx) return fail(c, "generate: S0=%d + max_new_tokens=%d exceeds max_ctx=%d", S0, T, D.max_ctx);
   if (N * S0 > D.max_lm_tokens) return fail(c, "generate: N*S0=%d exceeds max_lm_tokens=%d", N * S0, D.max_lm_tokens);
-  if (S0 > 256) return fail(c, "generate: prefix longer than 256 tokens is not supported");
+  if (const char* why = attention_prefill_unsupported(S0, D.lm_d / D.lm_heads, 1, true, D.lm_rotary_dim, false))
+    return fail(c, "generate: prefix of S0=%d tokens with head_dim %d: %s", S0, D.lm_d / D.lm_heads, why);
 
   // KV pool geometry for this call
   const int page_tokens = is_beam ? 1 : D.page_tokens;
@@ -832,18 +833,22 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   // any patch size that divides the image (patch 14: the K of the patch GEMM is padded, see vit_patch_k)
   if (D.vit_present && (D.vit_width % 64 || D.vit_heads <= 0 || D.vit_width % D.vit_heads || D.vit_patch <= 0 || D.vit_image % D.vit_patch))
     return fail(nullptr, "ccb_create: bad ViT dimensions");
-  if (D.vit_present && (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1 > 256 &&
-      ((D.vit_width / D.vit_heads) % 8 || D.vit_width / D.vit_heads > 256))
-    return fail(nullptr, "ccb_create: ViT of %d tokens with head_dim %d: attention over more than 256 tokens needs head_dim %% 8 == 0 "
-                "and <= 256", (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1, D.vit_width / D.vit_heads);
-  if ((D.map_kind == CCB_MAP_TRANSFORMER || D.map_kind == CCB_MAP_TRANSFORMER_ALL) && D.map_clip_len + D.map_prefix_len > 256 &&
-      ((D.lm_d / D.map_heads) % 8 || D.lm_d / D.map_heads > 256))
-    return fail(nullptr, "ccb_create: mapper sequence of %d tokens with head_dim %d: attention over more than 256 tokens needs "
-                "head_dim %% 8 == 0 and <= 256", D.map_clip_len + D.map_prefix_len, D.lm_d / D.map_heads);
-
   if (D.text_present && (D.text_width % 64 || D.text_heads <= 0 || D.text_width % D.text_heads || (D.text_width / D.text_heads) % 16 ||
                          D.text_ctx <= 0 || D.text_ctx > 128 || D.text_vocab <= 0 || D.text_out <= 0 || D.max_texts <= 0))
     return fail(nullptr, "ccb_create: bad CLIP text-tower dimensions");
+  // every fixed-length attention of the context must have a kernel (the LM's prefill length is checked per call)
+  {
+    struct { bool present; const char* what; int S, hd, causal; } att[] = {
+        {D.vit_present != 0, "ViT", D.vit_present ? (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1 : 0,
+         D.vit_present ? D.vit_width / D.vit_heads : 0, 0},
+        {D.text_present != 0, "CLIP text tower", D.text_ctx, D.text_present ? D.text_width / D.text_heads : 0, 1},
+        {D.map_kind == CCB_MAP_TRANSFORMER || D.map_kind == CCB_MAP_TRANSFORMER_ALL, "mapper", D.map_clip_len + D.map_prefix_len,
+         D.map_heads > 0 ? D.lm_d / D.map_heads : 0, 0}};
+    for (const auto& a : att) {
+      const char* why = a.present ? attention_prefill_unsupported(a.S, a.hd, a.causal, false, 0, false) : nullptr;
+      if (why) return fail(nullptr, "ccb_create: %s attention over %d tokens with head_dim %d: %s", a.what, a.S, a.hd, why);
+    }
+  }
 
   ccb_ctx* c = new ccb_ctx();
   c->desc = D;
@@ -1285,7 +1290,8 @@ int ccb_lm_forward(ccb_ctx* c, const float* embeds, int B, int S, const uint8_t*
   DeviceGuard dev_guard(c->device);
   if (B <= 0 || S <= 0 || static_cast<long long>(B) * S > c->desc.max_lm_tokens)
     return fail(c, "ccb_lm_forward: B*S=%lld exceeds max_lm_tokens=%d", static_cast<long long>(B) * S, c->desc.max_lm_tokens);
-  if (S > 256) return fail(c, "ccb_lm_forward: S=%d > 256 is not supported", S);
+  if (const char* why = attention_prefill_unsupported(S, c->desc.lm_d / c->desc.lm_heads, 1, false, c->desc.lm_rotary_dim, key_mask != nullptr))
+    return fail(c, "ccb_lm_forward: S=%d with head_dim %d: %s", S, c->desc.lm_d / c->desc.lm_heads, why);
   if (c->desc.lm_arch == CCB_LM_GPT2 && S > c->desc.lm_n_pos)
     return fail(c, "ccb_lm_forward: S=%d exceeds the model's %d learned positions", S, c->desc.lm_n_pos);
   if (ld_logits < c->desc.lm_vocab) return fail(c, "ccb_lm_forward: ld_logits < vocab");

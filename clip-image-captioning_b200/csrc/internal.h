@@ -135,13 +135,19 @@ struct KvCache {
   size_t kv_stride() const { return 1ull * num_pages * H * page_tokens * hd; }
 };
 // Full attention over a sequence held in one fused qkv buffer [B*S, 3*d] (q | k | v, head h at h*hd); S > 256 only for
-// non-causal attention without cache, rotary or key mask, with hd % 8 == 0 and hd <= 256.
+// non-causal attention without cache, rotary or key mask, with hd % 8 == 0 and hd <= 256 (attention_prefill_unsupported).
 // causal=0: ViT / mapper; causal=1: LM prefill, which also stores K/V into cache pages through block_table
 // ([B, max_pages_per_row] int32) at positions pos0..pos0+S-1 and (GPT-J) applies rotary to q/k first.
 // key_mask: optional [B, S] uint8, 0 = key may not be attended (HF attention_mask).
 int attention_prefill(const bf16* qkv, bf16* out, int B, int S, int H, int hd, float scale, int causal,
                       const KvCache* cache, int layer, const int* block_table, int pos0, int rotary_dim,
                       const uint8_t* key_mask, cudaStream_t s);
+// nullptr when attention_prefill has a kernel for the shape, else why not.  attention_prefill rejects exactly these shapes
+// (cudaErrorInvalidValue); ccb_create and the LM entry points call it up front so that a shape no kernel holds fails with
+// this reason before anything is launched.  Above 256 tokens see attention_prefill_long; at most 256 the scalar kernel
+// takes what mma.sync / tcgen05 do not, as long as K and V of the sequence fit its 200 KB of shared memory
+// (S * (4 * hd + 36) + 32 * hd + 4 bytes: GPT-J's head_dim 256 up to S = 185, head_dim 200 up to 237, 512 up to 90).
+const char* attention_prefill_unsupported(int S, int hd, int causal, bool cache, int rotary_dim, bool key_mask);
 // S > 256 part of attention_prefill (attention_long.cu): non-causal, unmasked, no cache / rotary, hd % 8 == 0, hd <= 256
 int attention_prefill_long(const bf16* qkv, bf16* out, int B, int S, int H, int hd, float scale, cudaStream_t s);
 // One new token per row: appends this step's k/v (from qkv [B, 3*d]) at position ctx_len[b] and attends over

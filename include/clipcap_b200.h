@@ -135,7 +135,10 @@ CCB_API int ccb_map_prefix(ccb_ctx* ctx, const float* feat, int B, float* prefix
 CCB_API int ccb_embed_tokens(ccb_ctx* ctx, const int32_t* tokens, int n, float* out, void* stream);
 /* language_model.call(inputs_embeds=E[, attention_mask]) (lms/GPT2.py:17-19 -> HF forward):
  * embeds [B,S,lm_d] f32 -> logits [B,S,ld_logits] (last_only = 0) or [B,ld_logits] for the last position.
- * key_mask: optional [B,S] uint8 (1 = attend), the HF attention_mask on keys; NULL = no mask. */
+ * key_mask: optional [B,S] uint8 (1 = attend), the HF attention_mask on keys; NULL = no mask.
+ * S is at most 256, and at most what the attention kernels hold at the LM's head_dim: 256 for head_dim 64 / 128
+ * (GPT-2 family), 185 for head_dim 256 (GPT-J).  A longer S fails with a message naming S and head_dim before anything
+ * is launched; the same limit applies to the prefix length S0 of ccb_generate / ccb_caption_images. */
 CCB_API int ccb_lm_forward(ccb_ctx* ctx, const float* embeds, int B, int S, const uint8_t* key_mask, float* logits_out,
                    int64_t ld_logits, int last_only, void* stream);
 /* generate_beam / generate_no_beam loops (inference.py:70-148, 219-292; evaluate_model.py:104-179), batched
