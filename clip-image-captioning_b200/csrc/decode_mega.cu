@@ -35,14 +35,454 @@ namespace ccb {
 
 namespace {
 
-#include "mega_common.cuh"
-
 constexpr int kThreads = 384;
 constexpr int kTblMax = 256;
 constexpr int kLnSlots = 14;            // split-K slots a LayerNorm thread keeps in flight per column
 constexpr int kAttnWarps = 11;           // the 8 compute warps + the X-producer, MMA and TMEM-allocator warps (idle then)
 constexpr int kVecScratch = kAttnWarps * 8192;  // vector-phase scratch: the (idle) X ring and what follows it, 8 KB per warp
+constexpr int kComputeThreads = 256;
+constexpr int kComputeWarp0 = 4;
+constexpr int kWStage = 128 * 64 * 2;
 
+__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
+  unsigned v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ float4 ldcg_f4(const float* p) {
+  float4 v;
+  asm volatile("ld.global.cg.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
+  return v;
+}
+__device__ __forceinline__ float2 ldcg_f2(const float* p) {
+  float2 v;
+  asm volatile("ld.global.cg.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
+  return v;
+}
+__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
+// 16-byte asynchronous copy global -> shared; src_bytes == 0 writes zeros
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32_t src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ uint4 lds_u4(uint32_t addr) {
+  uint4 v;
+  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
+  return v;
+}
+
+// wait until the phase counter reaches `target` (bounded: a protocol bug traps instead of hanging the GPU)
+__device__ __forceinline__ void poll_counter(const unsigned* ctr, unsigned target) {
+  if (ld_acquire_u32(ctr) >= target) return;
+  const uint64_t t0 = ptx::globaltimer_ns();
+  uint32_t spins = 0;
+  while (ld_acquire_u32(ctr) < target) {
+    if ((++spins & 0x3ff) == 0 && ptx::globaltimer_ns() - t0 > 4000000000ull) __trap();
+  }
+}
+
+// fine-grained role stamps of layer 1 (tuning only): slot k of CTA c at trace[ncta * 2 * (nbar + 2) + c * 64 + k], nbar = the
+// kernel's grid barriers per step (p.nbar)
+// Compiled in only with -DCCB_TUNING (python tools/build.py --tuning): production builds carry no timeline code.
+#ifdef CCB_TUNING
+#define MEGA_RSTAMP(layer, slot)                                                                         \
+  do {                                                                                                   \
+    if (p.trace != nullptr && (layer) == 1)                                                              \
+      p.trace[static_cast<size_t>(p.ncta) * (2 * (p.nbar + 2)) + static_cast<size_t>(blockIdx.x) * 64 + (slot)] = ptx::globaltimer_ns(); \
+  } while (0)
+#else
+#define MEGA_RSTAMP(layer, slot) do { } while (0)
+#endif
+
+// This CTA's share of one GEMM kind (the same in every layer): n units starting at (tile0, kb0), row-tile major.
+struct KindSched {
+  int n, tile0, kb0, kb;
+};
+
+struct ComputeCtx {
+  int ct, cw, lane;      // thread / warp index among the compute warps
+  int nattn;             // warps per CTA that take attention units
+  float* red;            // [2][8] reduction scratch
+  int red_it;
+  const uint32_t* tbl;   // tile table in shared memory
+  const KindSched* sched;
+  unsigned* ctr;
+  unsigned ncta;
+  uint8_t* vs;           // vector-phase scratch (generic pointer) and its shared-window address
+  uint32_t vs_u32;
+  float* strips;         // [8 warps][192] floats: q (scaled), k_new, v_new of the unit a warp works on
+  bool attn_prefetched;  // the first K/V copies of this warp's attention units are already in flight (a_* say which)
+  int a_k, a_ib, a_h, a_inflight;  // K/V stream position after the prefetch: unit ordinal, batch, batches issued / in flight
+  int u_ctx[4], u_page[4];  // cached tokens / this lane's page id of the warp's first four attention units
+  unsigned long long* trace;
+  int trace_it;
+  unsigned long long* rtrace;   // (tuning) this CTA's 64 role stamps, or null
+  int cur_layer;
+};
+
+__device__ __forceinline__ float compute_sum(ComputeCtx& cc, float v) {
+  v = warp_sum(v);
+  float* buf = cc.red + (cc.red_it & 1) * 8;
+  cc.red_it++;
+  if (cc.lane == 0) buf[cc.cw] = v;
+  ptx::named_bar_sync(2, kComputeThreads);
+  float r = (cc.lane < 8) ? buf[cc.lane] : 0.f;
+  return warp_sum(r);
+}
+
+__device__ __forceinline__ void stamp(ComputeCtx& cc) {
+#ifdef CCB_TUNING
+  if (cc.trace != nullptr && cc.ct == 0) cc.trace[cc.trace_it] = ptx::globaltimer_ns();
+  cc.trace_it++;
+#else
+  (void)cc;
+#endif
+}
+
+// all compute threads: publish this CTA's global writes of the phase and count the CTA in.  The CTA barrier orders
+// every compute thread's stores before thread 0's gpu-scope release (the pattern of a cooperative-groups grid sync).
+// The counter is shared by all barriers (barrier #k is complete at (k + 1) * ncta arrivals), so a CTA must never arrive
+// at #k+1 before #k is complete: a CTA with GEMM work gets that from its own data dependence (epilogue <- MMA <- X
+// tiles <- poll of #k), a CTA without units of a GEMM waits explicitly.
+// proxy: this phase's global writes are read through TMA by other CTAs (x / att / mlp rows): fence them into the async proxy
+__device__ __forceinline__ void grid_arrive(ComputeCtx& cc, uint32_t xgo_bar, uint32_t helpers_bar = 0, uint32_t helpers_parity = 0,
+                                            bool proxy = true) {
+  ptx::fence_proxy_async();  // this thread's generic accesses to the X ring (vector scratch) before TMA reuses it
+  ptx::named_bar_sync(1, kComputeThreads);
+  stamp(cc);
+  if (cc.ct == 0) {
+    if (helpers_bar != 0) {
+      ptx::mbar_wait(helpers_bar, helpers_parity);  // the helper warps' share of the phase is stored
+#ifdef CCB_TUNING
+      if (cc.rtrace != nullptr && cc.cur_layer == 1) cc.rtrace[44] = ptx::globaltimer_ns();
+#endif
+    }
+    if (proxy) fence_proxy_async_all();  // the global writes are read through TMA (async proxy) by other CTAs
+    red_release_add(cc.ctr, 1u);
+    if (xgo_bar != 0) ptx::mbar_arrive(xgo_bar);  // the X producer may start polling for this barrier
+  }
+}
+// all compute threads: wait until every CTA has arrived at the first `n` barriers
+__device__ __forceinline__ void grid_wait(ComputeCtx& cc, unsigned n) {
+  if (cc.ct == 0) poll_counter(cc.ctr, n * cc.ncta);
+  ptx::named_bar_sync(1, kComputeThreads);
+  stamp(cc);
+}
+
+// One warp per (row, head), head_dim 64.  q/k/v = bf16(sum of c_attn partials + bias); the new k/v are appended to
+// the cache; softmax(q K^T) V over the cached tokens and the new one.
+// The phase is latency bound (8 warps per SM, a few dependent memory round trips each), so the K/V rows travel by
+// cp.async into the warp's 8 KB slice of the idle X ring -- no registers are held while they are in flight, which
+// keeps ptxas from serialising the loads -- in batches of 16 tokens, two batches in flight; the sum of the c_attn
+// partials is computed underneath.  lane = (token group g = lane / 8, 16-byte chunk c = lane % 8); the batches are
+// folded with an online softmax.  page_tokens is a power of two (host-checked); offsets are 32-bit element offsets.
+// The K/V batches of ALL units of a warp form one stream with two batches in flight: when a unit has no batch left to
+// request, the freed half is refilled with the first batches of the warp's next unit, so the fold of q/k/v, the output
+// store and the unit change-over run underneath K/V copies (with several units per warp -- 128 / 256 rows -- the phase
+// is bound by these copies: 78 MB of K/V per layer at 256 rows).
+// prefetch_only: issue the first two batches of the stream and return (called between the arrival at the c_attn
+// barrier and the wait for it: cached K/V do not depend on the current step, so their latency hides behind the
+// barrier); the phase proper then continues from there (cc.attn_prefetched, cc.a_*).
+__device__ __noinline__ void attention_phase(const MegaParams& p, ComputeCtx& cc, int cta, int layer, const float* bias, bool prefetch_only) {
+  constexpr int HD = 64;
+  const int d = p.d, H = p.H, lane = cc.lane, ncta = p.ncta, cw = cc.cw;
+  const int grp = lane >> 3, ch = lane & 7;
+  const KvCache cache = p.kv;
+  bf16* const att = p.att;
+  const int* const ctx_len = p.ctx_len;
+  const int* const block_table = p.block_table;
+  const float scale = p.scale;
+  const uint32_t stage_u32 = cc.vs_u32 + cw * 8192;   // [2 halves][K 16 x 128 B | V 16 x 128 B]
+  float* qkvs = cc.strips + cw * 192;
+  const int total = p.R * H;
+  const int lpt = p.log2_page_tokens, ptm = (1 << lpt) - 1;
+  const uint32_t page_stride = static_cast<uint32_t>(H) << (lpt + 6);   // elements per page (all heads)
+  const size_t kv_stride = static_cast<size_t>(cache.num_pages) * page_stride;
+  const bf16* layer_k = cache.base + static_cast<size_t>(layer) * 2 * kv_stride;
+  const uint32_t lane_dst = static_cast<uint32_t>(grp) * 128u + static_cast<uint32_t>(ch) * 16u;
+  // Context length and page ids do not change during the step: those of a warp's first four units were loaded once at
+  // kernel start (cc.u_ctx / cc.u_page); further units (more than 4 * 11 * ncta units) read theirs when they come up.
+  const int maxp = cache.max_pages_per_row;
+  const int stride_u = cc.nattn * ncta, unit_first = cw * ncta + cta;
+  auto unit_state = [&](int k, int unit, int& ctx, int& page) {
+    if (k < 4) {
+      ctx = k == 0 ? cc.u_ctx[0] : k == 1 ? cc.u_ctx[1] : k == 2 ? cc.u_ctx[2] : cc.u_ctx[3];
+      page = k == 0 ? cc.u_page[0] : k == 1 ? cc.u_page[1] : k == 2 ? cc.u_page[2] : cc.u_page[3];
+    } else {
+      const int bb = unit / H;
+      ctx = ctx_len[bb];
+      page = lane < maxp ? block_table[static_cast<uint32_t>(bb) * maxp + lane] : 0;
+    }
+  };
+  // ---- issue side of the K/V stream
+  int i_k = 0, i_ib = 0, i_h = 0, inflight = 0;     // unit ordinal, next batch of it, real batches issued / in flight
+  int i_ctx = 0, i_page = 0, i_nb = 0;
+  bool i_valid = false, i_inwarp = true;
+  const bf16* i_kbase = layer_k;
+  const int* i_bt = block_table;
+  auto issuer_setup = [&](int k) {
+    i_k = k;
+    i_ib = 0;
+    const int unit = unit_first + k * stride_u;
+    i_valid = unit < total;
+    if (!i_valid) return;
+    unit_state(k, unit, i_ctx, i_page);
+    const int bb = unit / H, hh = unit - bb * H;
+    i_nb = (i_ctx + 15) >> 4;
+    i_inwarp = (i_ctx >> lpt) + 1 <= 32;   // page ids held one per lane when they fit a warp, else per-token lookups
+    i_kbase = layer_k + (static_cast<uint32_t>(hh) << (lpt + 6)) + ch * 8;  // + page * page_stride + (t & ptm) * 64
+    i_bt = block_table + static_cast<uint32_t>(bb) * maxp;
+  };
+  auto issue_next = [&]() {   // the next batch of the stream into the half it belongs to; always commits a group
+    while (i_valid && i_ib >= i_nb) issuer_setup(i_k + 1);
+    if (i_valid) {
+      const uint32_t dst = stage_u32 + static_cast<uint32_t>(i_h & 1) * 4096u + lane_dst;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int t = i_ib * 16 + i * 4 + grp;
+        const bool ok = t < i_ctx;
+        const int tt = ok ? t : 0;
+        const int page = i_inwarp ? __shfl_sync(0xffffffffu, i_page, tt >> lpt) : i_bt[tt >> lpt];
+        const bf16* kp = i_kbase + (static_cast<uint32_t>(page) * page_stride + (static_cast<uint32_t>(tt & ptm) << 6));
+        cp_async16(dst + i * 512u, kp, ok ? 16u : 0u);
+        cp_async16(dst + i * 512u + 2048u, kp + kv_stride, ok ? 16u : 0u);
+      }
+      ++i_ib;
+      ++i_h;
+      ++inflight;
+    }
+    cp_async_commit();
+  };
+  if (cc.attn_prefetched) {
+    issuer_setup(cc.a_k);
+    i_ib = cc.a_ib;
+    i_h = cc.a_h;
+    inflight = cc.a_inflight;
+    cc.attn_prefetched = false;
+  } else {
+    issuer_setup(0);
+    issue_next();
+    issue_next();
+  }
+  if (prefetch_only) {
+    cc.attn_prefetched = true;
+    cc.a_k = i_k;
+    cc.a_ib = i_ib;
+    cc.a_h = i_h;
+    cc.a_inflight = inflight;
+    return;
+  }
+  int c_h = 0, ui = 0;   // real batches consumed, unit ordinal
+#pragma unroll 1
+  for (int unit = unit_first; unit < total; unit += stride_u, ++ui) {
+    const int b = unit / H, h = unit - b * H;
+    int ctx, my_page;
+    unit_state(ui, unit, ctx, my_page);
+    const int* bt = block_table + static_cast<uint32_t>(b) * maxp;
+    const bool pages_in_warp = (ctx >> lpt) + 1 <= 32;
+    const bf16* kbase = layer_k + (static_cast<uint32_t>(h) << (lpt + 6)) + ch * 8;
+    const int nb = (ctx + 15) >> 4;
+
+    const bool stamp_me = ui == 0 && cw == 1 && lane == 0;   // (tuning) timeline of one unit: slots 32..43 of the role stamps
+    if (stamp_me) MEGA_RSTAMP(layer, 32);
+    // ---- q / k_new / v_new while the first batches are in flight: lane owns dims (2 lane, 2 lane + 1) of each
+    {
+      const int rows_out = p.g[0].rows_out, tbl_off = p.g[0].tbl_off;
+      const uint32_t* const tbl = cc.tbl;
+      const float* const ws = p.ws;
+      const uint32_t slot_stride = static_cast<uint32_t>(p.R) * rows_out;
+      const int dim = lane * 2;
+      const float* src0 = ws + static_cast<uint32_t>(b) * rows_out + h * HD + dim;
+      float2 w[3][8];
+      int nsl[3];
+      // (the bias of this head's q / k / v slices is requested together with the partials: one round trip, not two)
+      float2 bqkv[3];
+#pragma unroll
+      for (int pz = 0; pz < 3; ++pz) bqkv[pz] = __ldg(reinterpret_cast<const float2*>(bias + pz * d + h * HD + dim));
+#pragma unroll
+      for (int pz = 0; pz < 3; ++pz) {
+        nsl[pz] = static_cast<int>(tbl[tbl_off + ((pz * d + h * HD) >> 7)] >> 16);
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+          w[pz][j] = (j < nsl[pz]) ? ldcg_f2(src0 + pz * d + j * slot_stride) : make_float2(0.f, 0.f);
+      }
+      float2 part[3];
+#pragma unroll
+      for (int pz = 0; pz < 3; ++pz) {
+        float2 acc = make_float2(0.f, 0.f);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          acc.x += w[pz][j].x; acc.y += w[pz][j].y;
+        }
+        for (int sl = 8; sl < nsl[pz]; ++sl) {  // (more than 8 contributors per tile: tiny K only)
+          const float2 e = ldcg_f2(src0 + pz * d + sl * slot_stride);
+          acc.x += e.x; acc.y += e.y;
+        }
+        const float2 bb = bqkv[pz];
+        // the operator-per-kernel path stores c_attn's output as bf16: keep the same rounding
+        part[pz] = unpack_bf16x2(pack_bf16x2(acc.x + bb.x, acc.y + bb.y));
+      }
+      __syncwarp();  // the previous unit's reads of qkvs are complete
+      *reinterpret_cast<float2*>(qkvs + dim) = make_float2(part[0].x * scale, part[0].y * scale);
+      *reinterpret_cast<float2*>(qkvs + HD + dim) = part[1];
+      *reinterpret_cast<float2*>(qkvs + 2 * HD + dim) = part[2];
+      __syncwarp();
+    }
+    if (stamp_me) MEGA_RSTAMP(layer, 33);
+    float q8[8], acc[8];
+    {
+      const float4 a0 = *reinterpret_cast<const float4*>(qkvs + ch * 8), a1 = *reinterpret_cast<const float4*>(qkvs + ch * 8 + 4);
+      q8[0] = a0.x; q8[1] = a0.y; q8[2] = a0.z; q8[3] = a0.w; q8[4] = a1.x; q8[5] = a1.y; q8[6] = a1.z; q8[7] = a1.w;
+    }
+    // the new token: score, and its k / v chunks go to the cache (group 0 writes k, group 1 writes v)
+    float m_run, l_run;
+    {
+      const float4 k0 = *reinterpret_cast<const float4*>(qkvs + HD + ch * 8), k1 = *reinterpret_cast<const float4*>(qkvs + HD + ch * 8 + 4);
+      const float4 v0 = *reinterpret_cast<const float4*>(qkvs + 2 * HD + ch * 8), v1 = *reinterpret_cast<const float4*>(qkvs + 2 * HD + ch * 8 + 4);
+      float sn = q8[0] * k0.x;
+      sn = fmaf(q8[1], k0.y, sn); sn = fmaf(q8[2], k0.z, sn); sn = fmaf(q8[3], k0.w, sn);
+      sn = fmaf(q8[4], k1.x, sn); sn = fmaf(q8[5], k1.y, sn); sn = fmaf(q8[6], k1.z, sn); sn = fmaf(q8[7], k1.w, sn);
+      sn += __shfl_xor_sync(0xffffffffu, sn, 1);
+      sn += __shfl_xor_sync(0xffffffffu, sn, 2);
+      sn += __shfl_xor_sync(0xffffffffu, sn, 4);
+      m_run = sn;
+      const bool g0 = grp == 0;
+      l_run = g0 ? 1.f : 0.f;
+      acc[0] = g0 ? v0.x : 0.f; acc[1] = g0 ? v0.y : 0.f; acc[2] = g0 ? v0.z : 0.f; acc[3] = g0 ? v0.w : 0.f;
+      acc[4] = g0 ? v1.x : 0.f; acc[5] = g0 ? v1.y : 0.f; acc[6] = g0 ? v1.z : 0.f; acc[7] = g0 ? v1.w : 0.f;
+      const int page_new = pages_in_warp ? __shfl_sync(0xffffffffu, my_page, ctx >> lpt) : bt[ctx >> lpt];
+      if (grp < 2) {
+        const float4 s0 = g0 ? k0 : v0, s1 = g0 ? k1 : v1;
+        uint4 pk;
+        pk.x = pack_bf16x2(s0.x, s0.y); pk.y = pack_bf16x2(s0.z, s0.w); pk.z = pack_bf16x2(s1.x, s1.y); pk.w = pack_bf16x2(s1.z, s1.w);
+        const uint32_t off = static_cast<uint32_t>(page_new) * page_stride + (static_cast<uint32_t>(ctx & ptm) << 6);
+        *reinterpret_cast<uint4*>(const_cast<bf16*>(kbase) + off + (g0 ? 0 : kv_stride)) = pk;
+      }
+    }
+    if (stamp_me) MEGA_RSTAMP(layer, 34);
+    // ---- cached tokens, 16 per batch
+#pragma unroll 1
+    for (int bi = 0; bi < nb; ++bi) {
+      // (groups complete in order: with two batches in flight all but the newest group is enough)
+      if (inflight >= 2) cp_async_wait<1>(); else cp_async_wait<0>();
+      __syncwarp();
+      const uint32_t src = stage_u32 + static_cast<uint32_t>(c_h & 1) * 4096u + lane_dst;
+      uint4 kk[4], vv[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        kk[i] = lds_u4(src + i * 512u);
+        vv[i] = lds_u4(src + i * 512u + 2048u);
+      }
+      __syncwarp();                      // every lane has read the half: it may be refilled
+      if (stamp_me && bi < 4) MEGA_RSTAMP(layer, 35 + 2 * bi);
+      ++c_h;
+      --inflight;
+      issue_next();
+      if (stamp_me && bi < 4) MEGA_RSTAMP(layer, 36 + 2 * bi);                      // this unit's batch bi + 2, or the first batches of the warp's next unit
+      float sc[4];
+      float m_b = -INFINITY;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const float2 k0 = unpack_bf16x2(kk[i].x), k1 = unpack_bf16x2(kk[i].y), k2 = unpack_bf16x2(kk[i].z), k3 = unpack_bf16x2(kk[i].w);
+        float s = q8[0] * k0.x;
+        s = fmaf(q8[1], k0.y, s); s = fmaf(q8[2], k1.x, s); s = fmaf(q8[3], k1.y, s);
+        s = fmaf(q8[4], k2.x, s); s = fmaf(q8[5], k2.y, s); s = fmaf(q8[6], k3.x, s); s = fmaf(q8[7], k3.y, s);
+        s += __shfl_xor_sync(0xffffffffu, s, 1);
+        s += __shfl_xor_sync(0xffffffffu, s, 2);
+        s += __shfl_xor_sync(0xffffffffu, s, 4);
+        sc[i] = (bi * 16 + i * 4 + grp < ctx) ? s : -INFINITY;
+        m_b = fmaxf(m_b, sc[i]);
+      }
+      m_b = fmaxf(m_b, __shfl_xor_sync(0xffffffffu, m_b, 8));
+      m_b = fmaxf(m_b, __shfl_xor_sync(0xffffffffu, m_b, 16));
+      const float m_new = fmaxf(m_run, m_b);
+      const float resc = __expf(m_run - m_new);
+      m_run = m_new;
+      l_run *= resc;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc[j] *= resc;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const float pr = __expf(sc[i] - m_new);  // exp(-inf) = 0 for masked tokens (their V rows were zero-filled)
+        l_run += pr;
+        const float2 v0 = unpack_bf16x2(vv[i].x), v1 = unpack_bf16x2(vv[i].y), v2 = unpack_bf16x2(vv[i].z), v3 = unpack_bf16x2(vv[i].w);
+        acc[0] = fmaf(pr, v0.x, acc[0]); acc[1] = fmaf(pr, v0.y, acc[1]); acc[2] = fmaf(pr, v1.x, acc[2]); acc[3] = fmaf(pr, v1.y, acc[3]);
+        acc[4] = fmaf(pr, v2.x, acc[4]); acc[5] = fmaf(pr, v2.y, acc[5]); acc[6] = fmaf(pr, v3.x, acc[6]); acc[7] = fmaf(pr, v3.y, acc[7]);
+      }
+    }
+    if (stamp_me) MEGA_RSTAMP(layer, 43);
+    // fold the 4 token groups
+    l_run += __shfl_xor_sync(0xffffffffu, l_run, 8);
+    l_run += __shfl_xor_sync(0xffffffffu, l_run, 16);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 8);
+      acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 16);
+    }
+    if (grp == 0) {
+      const float inv = 1.f / l_run;
+      uint4 pk;
+      pk.x = pack_bf16x2(acc[0] * inv, acc[1] * inv); pk.y = pack_bf16x2(acc[2] * inv, acc[3] * inv);
+      pk.z = pack_bf16x2(acc[4] * inv, acc[5] * inv); pk.w = pack_bf16x2(acc[6] * inv, acc[7] * inv);
+      *reinterpret_cast<uint4*>(att + static_cast<uint32_t>(b) * d + h * HD + ch * 8) = pk;
+    }
+  }
+}
+
+// attention state of a warp: its unit(s) never change during the step, so context length and page ids are read once
+__device__ __forceinline__ void init_attn_ctx(const MegaParams& p, ComputeCtx& cc, int aw, int nattn, int lane, int cta, const uint32_t* tbl,
+                                              uint8_t* vs, uint32_t vs_u32, float* strips) {
+  cc.cw = aw;
+  cc.nattn = nattn;
+  cc.lane = lane;
+  cc.tbl = tbl;
+  cc.vs = vs;
+  cc.vs_u32 = vs_u32;
+  cc.strips = strips;
+  cc.attn_prefetched = false;
+  cc.a_k = cc.a_ib = cc.a_h = cc.a_inflight = 0;
+  cc.rtrace = p.trace ? p.trace + static_cast<size_t>(p.ncta) * (2 * (p.nbar + 2)) + static_cast<size_t>(cta) * 64 : nullptr;
+  cc.cur_layer = 0;
+#pragma unroll
+  for (int ui = 0; ui < 4; ++ui) {
+    const int unit = (aw + nattn * ui) * p.ncta + cta;
+    cc.u_ctx[ui] = 0;
+    cc.u_page[ui] = 0;
+    if (unit < p.R * p.H) {
+      const int b = unit / p.H;
+      cc.u_ctx[ui] = p.ctx_len[b];
+      cc.u_page[ui] = lane < p.kv.max_pages_per_row ? p.block_table[static_cast<uint32_t>(b) * p.kv.max_pages_per_row + lane] : 0;
+    }
+  }
+}
+
+// The X-producer, MMA and TMEM-allocator warps have nothing to do while the attention phase runs: each takes the
+// attention units of one more "compute warp" (11 instead of 8 warps: GPT2-XL x 64 rows = 1600 units on 148 x 11 warps,
+// one unit per warp instead of two for a third of them).  Their K/V staging lies behind the X ring (up to ~170 rows), so
+// they prefetch as soon as they get here; vgo = c_attn complete everywhere, vdone = this warp's outputs are stored.
+__device__ __forceinline__ void helper_attention(const MegaParams& p, ComputeCtx& hc, int cta, int l, uint32_t vgo, uint32_t vdone,
+                                                 bool early_prefetch) {
+  const float* bias = p.layers[l].b_qkv;
+  // The helpers get here while this CTA's c_attn MMAs may still be reading the X ring.  Their K/V staging (slices 8..10
+  // of the vector scratch, 64..88 KB from the ring's start) lies behind the ring only while the ring is <= 64 KB; above
+  // ~170 rows (three tiles of > 21 KB) it is inside it, and an early prefetch would overwrite live activation tiles
+  // (seen as run-to-run differences of sampled / beam captions at >= 200 rows): then the copies start after vgo.
+  if (early_prefetch) attention_phase(p, hc, cta, l, bias, true);
+  ptx::mbar_wait(vgo, static_cast<uint32_t>(l) & 1u);
+  if (hc.lane == 0 && hc.cw == 8) MEGA_RSTAMP(l, 48);
+  attention_phase(p, hc, cta, l, bias, false);
+  fence_proxy_async_all();   // att rows are fetched by other CTAs through TMA
+  __syncwarp();
+  if (hc.lane == 0) {
+    MEGA_RSTAMP(l, 45 + hc.cw - 8);
+    ptx::mbar_arrive(vdone);
+  }
+}
 
 // h[t] = (embed | h[t] + bias + sum of split-K partials); x[t] = LayerNorm(h[t]) for the rows t = cta, cta + ncta, ...
 // The row is staged in shared memory (each thread re-reads only what it wrote).
@@ -431,7 +871,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_mega_kernel(const __grid_c
     for (int l = 0; l < p.L; ++l) {
 #pragma unroll 1
       for (int kind = 0; kind < 4; ++kind) {
-        if (kind == 1) helper_attention<true>(p, hc, cta, l, vgo, vdone, helper_prefetch);   // between the c_attn and the c_proj tiles
+        if (kind == 1) helper_attention(p, hc, cta, l, vgo, vdone, helper_prefetch);   // between the c_attn and the c_proj tiles
         const CUtensorMap* xm = (kind == 1) ? &xmap_att : (kind == 3) ? &xmap_mlp : &xmap_x;
         const KindSched sc = sched[kind];
         if (sc.n == 0) continue;
@@ -483,7 +923,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_mega_kernel(const __grid_c
     for (int l = 0; l < p.L; ++l) {
 #pragma unroll 1
       for (int kind = 0; kind < 4; ++kind) {
-        if (kind == 1) helper_attention<true>(p, hc, cta, l, vgo, vdone, helper_prefetch);   // all c_attn MMAs of this CTA are issued
+        if (kind == 1) helper_attention(p, hc, cta, l, vgo, vdone, helper_prefetch);   // all c_attn MMAs of this CTA are issued
         const KindSched sc = sched[kind];
         int kb = sc.kb0;          // k block of the next unit inside its row tile
         int seg_left = 0;         // units left in the current segment (0: the next unit opens one)
@@ -557,7 +997,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_mega_kernel(const __grid_c
     prefetch_layer_vectors(p, 0, cta, lane);
     for (int l = 0; l < p.L; ++l) {
       if (l + 1 < p.L) prefetch_layer_vectors(p, l + 1, cta, lane);
-      helper_attention<true>(p, hc, cta, l, vgo, vdone, helper_prefetch);
+      helper_attention(p, hc, cta, l, vgo, vdone, helper_prefetch);
     }
   } else if (warp >= kComputeWarp0) {
     // ------------------------------------------------------------------ compute warps
@@ -594,10 +1034,10 @@ __global__ void __launch_bounds__(kThreads, 1) decode_mega_kernel(const __grid_c
       if (sched[0].n == 0) grid_wait(cc, 8 * l + 1);  // (see grid_arrive: no arrival at #k+1 before #k is complete)
       grid_arrive(cc, 0, 0, 0, false);       // #8l+1 (split-K partials: read with ld.global.cg, no TMA consumer)
       // (warp 0 polls the barrier for the CTA: it goes straight to the wait and fetches its K/V afterwards)
-      if (cc.cw != 0) attention_phase<true>(p, cc, cta, l, ly.b_qkv, true);
+      if (cc.cw != 0) attention_phase(p, cc, cta, l, ly.b_qkv, true);
       grid_wait(cc, 8 * l + 2);
       if (cc.ct == 0) ptx::mbar_arrive(vgo);   // the helper warps start their units
-      attention_phase<true>(p, cc, cta, l, ly.b_qkv, false);
+      attention_phase(p, cc, cta, l, ly.b_qkv, false);
       if (lane == 0) MEGA_RSTAMP(l, 50 + cc.cw);
       grid_arrive(cc, xgo, vdone, static_cast<uint32_t>(l) & 1u);     // #8l+2
       epilogue_phase(p, cc, ec, cta, 1, l);

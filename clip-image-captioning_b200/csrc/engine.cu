@@ -443,60 +443,10 @@ bool mega_enabled() {
   return on;
 }
 
-// the five-phase cluster kernel is opt-in (CCB_MEGA2=1): correct, but measured slower than the eight-phase kernel (DESIGN.md)
-bool mega2_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("CCB_MEGA2");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
-
-// second-generation kernel (decode_mega2.cu, <= 64 rows)
-int lm_decode_layers_mega2(ccb_ctx* c, int rows, cudaStream_t s) {
-  const ccb_model_desc& D = c->desc;
-  const MegaState& m = c->mega;
-  Mega2Params p;
-  memset(&p, 0, sizeof(p));
-  p.L = D.lm_layers;
-  p.d = D.lm_d;
-  p.H = D.lm_heads;
-  p.ff = 4 * D.lm_d;
-  p.R = rows;
-  p.ncl = m.ncl;
-  p.ncta = m.ncl * 4;
-  p.eps = D.lm_ln_eps;
-  p.scale = 1.0f / sqrtf(static_cast<float>(D.lm_d / D.lm_heads));
-  p.layers = m.d_layers;
-  p.wmaps = m.d_wmaps2;
-  for (int k = 0; k < 4; ++k) p.g[k] = m.g2[k];
-  p.h = c->h;
-  p.x = c->x;
-  p.qkv = c->qkv;
-  p.att = c->att;
-  p.mlp = c->mlp;
-  p.stats = m.d_stats;
-  p.wte = c->wte;
-  p.wpe = c->wpe;
-  p.tokens = c->next_tokens;
-  p.ctx_len = c->ctx_len;
-  p.block_table = c->block_table;
-  p.kv = c->kv;
-  p.lnf_g = c->lm_lnf.g;
-  p.lnf_b = c->lm_lnf.b;
-  p.sync = m.d_sync;
-  p.trace = m.trace;
-  p.log2_page_tokens = 0;
-  while ((1 << p.log2_page_tokens) < c->kv.page_tokens) ++p.log2_page_tokens;
-  RUN(mega2_launch(p, s));
-  return 0;
-}
-
 // the whole layer stack of one decode step as ONE persistent kernel (decode_mega.cu): leaves ln_f(h) in c->x
 int lm_decode_layers_mega(ccb_ctx* c, int rows, cudaStream_t s) {
   const ccb_model_desc& D = c->desc;
   const MegaState& m = c->mega;
-  if (m.available2 && m.enabled2 && rows <= kMega2MaxRows) return lm_decode_layers_mega2(c, rows, s);
   MegaParams p;
   memset(&p, 0, sizeof(p));
   p.L = D.lm_layers;
@@ -693,7 +643,7 @@ int generate_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const float* em
 
   // ---- decode: T-1 replays of one captured step (every kernel reads step / ctx_len from device memory)
   if (T > 1) {
-    const std::string key = graph_key(p, N, rows, T, c->mega.enabled ? (c->mega.enabled2 ? 2 : 1) : 0);
+    const std::string key = graph_key(p, N, rows, T, c->mega.enabled ? 1 : 0);
     auto it = c->graphs.find(key);
     if (it == c->graphs.end()) {
       cudaGraph_t graph = nullptr;
@@ -1120,13 +1070,6 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
       mg.d_sync = a.arr<unsigned int>(64);
       mg.available = true;
       mg.enabled = mega_enabled();
-      int ncl = 0;
-      if (mega2_init(&ncl) == 0 && ncl >= 8 && mega2_plan(mg, d, 4 * d, ncl)) {
-        mg.d_stats = a.arr<float>(static_cast<size_t>((d + 63) / 64) * 64 * 2);
-        mg.d_wmaps2 = static_cast<CUtensorMap*>(a.take(sizeof(CUtensorMap) * 4 * D.lm_layers));
-        mg.available2 = true;
-        mg.enabled2 = mega2_enabled();
-      }
     }
   }
 
@@ -1148,16 +1091,6 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
       for (int k = 0; k < 4; ++k)
         ok = ok && gemm_make_tmap(&maps[l * 4 + k], lin[k]->w, lin[k]->features, lin[k]->K, lin[k]->K, 128) == 0;
       lys[l] = MegaLayer{b.ln1.g, b.ln1.b, b.ln2.g, b.ln2.b, b.qkv.bias, b.proj.bias, b.fc.bias, b.fc2.bias};
-    }
-    if (mg.available2) {   // the cluster kernel's weight tiles are 64 features high
-      std::vector<CUtensorMap> maps2(maps.size());
-      for (int l = 0; l < D.lm_layers && ok; ++l) {
-        const Block& b = c->lm[l];
-        const Linear* lin[4] = {&b.qkv, &b.proj, &b.fc, &b.fc2};
-        for (int k = 0; k < 4; ++k)
-          ok = ok && gemm_make_tmap(&maps2[l * 4 + k], lin[k]->w, lin[k]->features, lin[k]->K, lin[k]->K, 64) == 0;
-      }
-      ok = ok && cudaMemcpy(mg.d_wmaps2, maps2.data(), maps2.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice) == cudaSuccess;
     }
     ok = ok && cudaMemcpy(mg.d_wmaps, maps.data(), maps.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice) == cudaSuccess;
     ok = ok && cudaMemcpy(mg.d_layers, lys.data(), lys.size() * sizeof(MegaLayer), cudaMemcpyHostToDevice) == cudaSuccess;
@@ -1472,9 +1405,7 @@ int ccb_debug_gemm_trace(ccb_ctx* c, void* trace_u64, int64_t stride_u64, int la
 
 int ccb_debug_set_mega(ccb_ctx* c, int enable) {
   if (!c) return -1;
-  // 0: operator chain, 1: persistent kernel (default choice), 2: eight-phase kernel only, 3: five-phase cluster kernel up to 64 rows
-  c->mega.enabled = enable != 0;
-  c->mega.enabled2 = (enable == 3 || (enable == 1 && mega2_enabled())) && c->mega.available2;
+  c->mega.enabled = enable != 0;   // 0: operator chain, otherwise the persistent kernel
   return c->mega.available ? 1 : 0;
 }
 
@@ -1492,15 +1423,6 @@ int ccb_debug_copy_buffer(ccb_ctx* c, int which, void* dst, int64_t bytes, void*
     default: return fail(c, "ccb_debug_copy_buffer: unknown buffer %d", which);
   }
   CUDA_OK(cudaMemcpyAsync(dst, src, static_cast<size_t>(bytes), cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
-  return 0;
-}
-
-int ccb_debug_mega_info(ccb_ctx* c, int* out4) {
-  if (!c || !out4) return -1;
-  out4[0] = c->mega.available ? c->mega.ncta : 0;
-  out4[1] = c->mega.available2 ? c->mega.ncl * 4 : 0;
-  out4[2] = c->mega.enabled ? 1 : 0;
-  out4[3] = c->mega.enabled2 ? 1 : 0;
   return 0;
 }
 

@@ -54,37 +54,6 @@ struct MegaParams {
   unsigned long long* trace;   // optional [ncta][2 * (8 * L + 1)] globaltimer stamps of CTA phases
 };
 
-// ---- second generation (decode_mega2.cu): clusters of 4 CTAs own whole row tiles, five phases per layer, <= 64 rows
-struct Mega2Gemm {
-  int rows_out, kb, tiles, off;   // tile t belongs to cluster (t + off) % ncl
-};
-
-struct Mega2Params {
-  int L, d, H, ff, R, ncta, ncl;
-  float eps, scale;
-  const MegaLayer* layers;     // [L]
-  const CUtensorMap* wmaps;    // [L * 4]: qkv, proj, fc, fc2; box {64 k, 64 features}, 128B swizzle
-  Mega2Gemm g[4];
-  float* h;                    // [R, d] residual stream
-  bf16* x;                     // [R, d] ln_f output at exit (operand of lm_head)
-  bf16* qkv;                   // [R, 3d]
-  bf16* att;                   // [R, d]
-  bf16* mlp;                   // [R, ff]
-  float* stats;                // [ceil(d / 64)][64][2]: (mean, M2) of every row of h over a 64-feature tile
-  const bf16* wte;
-  const bf16* wpe;
-  const int* tokens;
-  const int* ctx_len;
-  const int* block_table;
-  KvCache kv;
-  const float *lnf_g, *lnf_b;
-  unsigned int* sync;          // [0] phase counter (zero at entry and at exit)
-  int nW;
-  int log2_page_tokens;
-  int nbar;                    // grid barriers per launch minus the exit barrier (5 * L + 1): sizes the trace rows
-  unsigned long long* trace;   // optional [ncta][2 * (nbar + 2)] globaltimer stamps of CTA phases (+ [ncta][64] role stamps)
-};
-
 // host-side plan, owned by ccb_ctx
 struct MegaState {
   bool available = false;      // model shape supported and buffers allocated
@@ -101,13 +70,6 @@ struct MegaState {
   unsigned long long* trace = nullptr;
   std::vector<uint32_t> h_tbl;
   size_t ws_floats_per_row = 0;
-  // second-generation kernel (rows <= 64)
-  bool available2 = false;
-  bool enabled2 = false;       // CCB_MEGA2=0 in the environment switches it off
-  int ncl = 0;                 // co-resident clusters of 4 CTAs
-  Mega2Gemm g2[4] = {};
-  float* d_stats = nullptr;
-  CUtensorMap* d_wmaps2 = nullptr;   // box {64 k, 64 features}
 };
 
 // fills g[] / table for `ncta` CTAs; returns max over kinds of (max slots * rows_out) = workspace floats per row
@@ -119,12 +81,5 @@ int gemm_make_tmap(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t K, u
 // launches the kernel (cooperative); returns 0 / cudaError / -1 (gemm_last_error)
 int mega_launch(const MegaParams& p, cudaStream_t s);
 int mega_init();  // function attributes
-
-// second generation: function attributes + the number of co-resident 4-CTA clusters; tile -> cluster plan (false: the
-// shape does not fit); launch (cluster + cooperative)
-int mega2_init(int* max_clusters);
-bool mega2_plan(MegaState& m, int d, int ff, int ncl);
-int mega2_launch(const Mega2Params& p, cudaStream_t s);
-constexpr int kMega2MaxRows = 64;
 
 }  // namespace ccb

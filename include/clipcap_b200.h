@@ -205,13 +205,9 @@ CCB_API int ccb_debug_gemm_trace(ccb_ctx* ctx, void* trace_u64, int64_t stride_u
  * Returns the number of CTAs of that kernel (0 when the model shape is not covered by it). */
 CCB_API int ccb_debug_mega_trace(ccb_ctx* ctx, void* trace_u64);
 /* A/B aid: 0 routes decode steps through the operator-per-kernel chain instead of the persistent kernel (CCB_MEGA=0 in
- * the environment), 1 (default) uses the persistent kernel, 2 the eight-phase kernel only, 3 the experimental five-phase
- * cluster kernel up to 64 rows (CCB_MEGA2=1 makes it the choice of mode 1).  Returns 1 when a persistent kernel covers
+ * the environment); any other value (default) uses the persistent kernel.  Returns 1 when the persistent kernel covers
  * this model shape, else 0. */
 CCB_API int ccb_debug_set_mega(ccb_ctx* ctx, int enable);
-/* out4 = { CTAs of the eight-phase kernel (0: shape not covered), CTAs of the five-phase cluster kernel (0: not
- * available), persistent kernels enabled, cluster kernel enabled } */
-CCB_API int ccb_debug_mega_info(ccb_ctx* ctx, int* out4);
 /* test aid: copies the first `bytes` of an internal activation workspace to `dst` (device memory) on `stream`:
  * 0 residual stream h (f32), 1 LayerNorm output x (bf16), 2 attention output (bf16), 3 MLP hidden (bf16),
  * 4 logits (f32, row pitch = vocab rounded up to 64), 5 fused qkv (bf16; operator-per-kernel decode only). */

@@ -157,14 +157,14 @@ def test_row_counts_across_the_ring_configurations(rows):
     embeds = (0.5 * torch.randn(rows, 21, cfg.lm_d, device="cuda")).contiguous()
     p1 = eng.gen_params("greedy", 2, stop_token=-1, max_stops=0)
     buf = {}
-    for tag, on in (("mega", True), ("chain", False), ("mega2", True)):
+    for tag, on in (("mega", True), ("chain", False), ("mega_again", True)):
         assert set_mega(eng, on) == 1
         eng.generate(embeds, p1)
         torch.cuda.synchronize()
         buf[tag] = (grab(eng, 1, rows * cfg.lm_d, torch.bfloat16), grab(eng, 0, rows * cfg.lm_d, torch.float32))
     for k in range(2):
         assert (buf["mega"][k] - buf["chain"][k]).abs().max().item() <= TOL * buf["chain"][k].abs().max().item(), (rows, k)
-        assert torch.equal(buf["mega"][k], buf["mega2"][k]), (rows, k)
+        assert torch.equal(buf["mega"][k], buf["mega_again"][k]), (rows, k)
     eng.close()
 
 
