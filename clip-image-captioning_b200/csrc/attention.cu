@@ -1049,46 +1049,24 @@ int attention_decode(const bf16* qkv, bf16* out, long long ldo, int B, int H, in
   if (B <= 0) return 0;
   if (ldo < static_cast<long long>(H) * hd || (ldo & 1)) return (int)cudaErrorInvalidValue;
   if (!cache) return (int)cudaErrorInvalidValue;
-  // One CTA per (row, head) for head_dim 256 (GPT-J); CCB_ATTN_WIDE=1 / 0 forces it on / off for every head_dim.
-  static const int wide_mode = [] {
-    const char* e = getenv("CCB_ATTN_WIDE");
-    return e ? (e[0] == '0' ? 0 : 1) : -1;
-  }();
-  if (wide_mode == 1 || (wide_mode == -1 && hd == 256)) {
+  // One CTA per (row, head) for head_dim 256 (GPT-J)
+  if (hd == 256) {
     // tile = tokens staged at once: the whole context when it fits (max_pages_per_row >= max_ctx), 96 KB of K + V at most
     int tile = (cache->max_pages_per_row * cache->page_tokens + 15) & ~15;
     const int cap = (96 * 1024) / (hd * 4);
     if (tile > cap) tile = cap;
-    static const int forced_tile = [] {   // testing: a small tile exercises the online-softmax fold across tiles
-      const char* e = getenv("CCB_ATTN_WIDE_TILE");
-      return e ? atoi(e) : 0;
-    }();
-    if (forced_tile > 0 && forced_tile < tile) tile = forced_tile;
     const size_t wsmem = static_cast<size_t>(tile) * hd * 4 + (hd + tile + 2 * (kWideThreads / 32)) * sizeof(float);
-#define CCB_LAUNCH_WIDE(HDV)                                                                                              \
-  do {                                                                                                                    \
-    static size_t configured_dev[kMaxDevices] = {};                                                                       \
-    size_t& configured = configured_dev[current_device_slot()];                                                           \
-    if (wsmem > 48 * 1024 && wsmem > configured) {                                                                        \
-      cudaError_t e = cudaFuncSetAttribute(attention_decode_wide_kernel<HDV>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                           112 * 1024);                                                                   \
-      if (e != cudaSuccess) return (int)e;                                                                                \
-      configured = 112 * 1024;                                                                                            \
-    }                                                                                                                     \
-    cudaError_t le = launch_kernel(attention_decode_wide_kernel<HDV>, dim3(B * H), dim3(kWideThreads), wsmem, s, true, qkv, \
-                                   out, B, H, scale, *cache, layer, block_table, ctx_len, rotary_dim, tile, ldo);              \
-    if (le != cudaSuccess) return (int)le;                                                                                \
-  } while (0)
-    if (hd == 64)
-      CCB_LAUNCH_WIDE(64);
-    else if (hd == 128)
-      CCB_LAUNCH_WIDE(128);
-    else if (hd == 256)
-      CCB_LAUNCH_WIDE(256);
-    else
-      return (int)cudaErrorInvalidValue;
-#undef CCB_LAUNCH_WIDE
-    cudaError_t e = cudaGetLastError();
+    static size_t configured_dev[kMaxDevices] = {};
+    size_t& configured = configured_dev[current_device_slot()];
+    if (wsmem > 48 * 1024 && wsmem > configured) {
+      cudaError_t e = cudaFuncSetAttribute(attention_decode_wide_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           112 * 1024);
+      if (e != cudaSuccess) return (int)e;
+      configured = 112 * 1024;
+    }
+    cudaError_t e = launch_kernel(attention_decode_wide_kernel<256>, dim3(B * H), dim3(kWideThreads), wsmem, s, true, qkv, out,
+                                  B, H, scale, *cache, layer, block_table, ctx_len, rotary_dim, tile, ldo);
+    if (e == cudaSuccess) e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
   }
   // per-warp shared memory: hd floats of q + one score per cached token
@@ -1114,8 +1092,6 @@ int attention_decode(const bf16* qkv, bf16* out, long long ldo, int B, int H, in
     CCB_LAUNCH_DECODE(64);
   else if (hd == 128)
     CCB_LAUNCH_DECODE(128);
-  else if (hd == 256)
-    CCB_LAUNCH_DECODE(256);
   else
     return (int)cudaErrorInvalidValue;
 #undef CCB_LAUNCH_DECODE

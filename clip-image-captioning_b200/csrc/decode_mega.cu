@@ -24,7 +24,6 @@
 // phase kept incrementally, phases as out-of-line functions (the kernel must stay resident in the instruction cache).
 #include <cuda.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -1128,16 +1127,11 @@ int mega_launch(const MegaParams& p_in, cudaStream_t s) {
   // 256 rows (32 KB activation tiles) the X ring holds three single tiles and every unit is handed over on its own
   p.nX = p.N <= 64 ? 8 : p.N <= 128 ? 4 : 3;
   p.grp = p.nX >= 4 ? 2 : 1;
-  if (const char* g = getenv("CCB_MEGA_GRP")) p.grp = atoi(g) == 1 ? 1 : p.grp;   // tuning: single-slot hand-over
   p.xring_bytes = p.nX * xstage > kVecScratch ? p.nX * xstage : kVecScratch;
   p.nW = (total - fixed - p.xring_bytes) / kWStage;
   if (p.nW > 12) p.nW = 12;
   if (p.grp == 2) p.nW &= ~1;
   if (p.nW < 2) return static_cast<int>(cudaErrorInvalidValue);
-  {
-    const char* lay = getenv("CCB_MEGA_LAYERS");  // tuning / debugging only: run the first n layers
-    if (lay && atoi(lay) > 0 && atoi(lay) < p.L) p.L = atoi(lay);
-  }
   p.nbar = 8 * p.L;
   const size_t smem = static_cast<size_t>(p.nW) * kWStage + p.xring_bytes + fixed + 1024;
 

@@ -373,7 +373,7 @@ int map_forward(ccb_ctx* c, const float* feat, int B, float* out, int out_rows_p
     g.rg_in = CL;
     g.rg_out = S;
     g.rg_off = 0;
-    g.force_orientation = 1;   // the row remap lives in the token-major kernels
+    g.force_orientation = 1;   // the row remap exists only in the normal orientation (the persistent kernels)
     g.allow_pdl = 1;
     RUN(gemm_launch(g, c->gemm_ws, s));
   } else {
@@ -496,13 +496,9 @@ int lm_decode_step(ccb_ctx* c, int rows, cudaStream_t s) {
   RUN(embed_tokens(c->wte, D.lm_arch == CCB_LM_GPT2 ? c->wpe : nullptr, c->next_tokens, c->ctx_len, c->h, rows, d, D.lm_vocab, D.lm_n_pos, s));
   const BlockShape sh = lm_shape(D);
   const float scale = 1.0f / sqrtf(static_cast<float>(hd));
-  static const bool fuse_out = [] {   // CCB_GPTJ_FUSE_OUT=0: out_proj and fc_out as two launches (A/B, tests)
-    const char* e = getenv("CCB_GPTJ_FUSE_OUT");
-    return !(e && e[0] == '0');
-  }();
   for (int l = 0; l < D.lm_layers; ++l) {
     const Block& b = c->lm[l];
-    if (sh.parallel && fuse_out && b.projfc2.w != nullptr && c->attmlp != nullptr) {
+    if (sh.parallel) {
       // GPT-J: h += out_proj(att) + fc_out(gelu_new(fc_in(ln_1 h))) + b as ONE GEMM over K = 5 d.  The 32 x 8 CTAs of the
       // stand-alone out_proj stream 33 MB at 2.6 TB/s (launch ramp, cluster reduce and epilogue around 8 k-blocks per CTA);
       // as the first fifth of fc_out's K loop the same bytes move at that GEMM's 4.9 TB/s.

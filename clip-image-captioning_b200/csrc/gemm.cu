@@ -1,7 +1,6 @@
 // Host side of the tcgen05 GEMM: tensor-map encoding, orientation / tile / split-K selection, launch.
 #include <cuda.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <mutex>
@@ -137,11 +136,22 @@ void pick_persist(int tokens, int features, int k_blocks, int num_sms, int force
   *pair_out = pair;
 }
 
-int launch_persist(const GemmArgs& a, const GemmParams& p_in, int bn, bool pair, int num_sms, cudaStream_t s) {
+int launch_persist(const GemmArgs& a, int bn, bool pair, int pdl, int num_sms, cudaStream_t s) {
   PersistParams pp;
   memset(&pp, 0, sizeof(pp));
-  pp.g = p_in;
-  pp.g.split_k = 1;
+  pp.tokens = a.tokens;
+  pp.features = a.features;
+  pp.k_blocks = a.K / 64;
+  pp.out = a.out;
+  pp.out_bf16 = a.out_bf16;
+  pp.ldo = a.ldo;
+  pp.bias = a.bias;
+  pp.residual = a.residual;
+  pp.ldr = a.ldr;
+  pp.act = a.act_fn;
+  pp.rg_in = a.rg_in;
+  pp.rg_out = a.rg_out;
+  pp.rg_off = a.rg_off;
   pp.bn = bn;
   const int stage_bytes = 128 * 128 + bn * (pair ? 64 : 128);
   int stages = (kPersistSmemBytes - 1024 - 512) / stage_bytes;
@@ -169,7 +179,7 @@ int launch_persist(const GemmArgs& a, const GemmParams& p_in, int bn, bool pair,
     attr[na].val.clusterDim.z = 1;
     ++na;
   }
-  if (pp.g.pdl) {
+  if (pdl) {
     attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[na].val.programmaticStreamSerializationAllowed = 1;
     ++na;
@@ -233,58 +243,43 @@ int gemm_launch(const GemmArgs& a, const GemmWorkspace& w, cudaStream_t stream) 
   const bool swapped = a.force_orientation ? (a.force_orientation == 2) : (a.tokens <= 256);
   if (swapped && a.rg_in > 0) return fail("row remap is only supported in the normal orientation");
   if (swapped && a.tokens > 256) return fail("swapped orientation needs tokens <= 256");
+  if (!swapped && a.force_split) return fail("split-K is only available in the swapped orientation");
+  // tuning timelines: every launch takes the next slot, although only the one-tile kernel writes stamps
+  unsigned long long* trace = w.trace ? w.trace + (w.trace_count++ % w.trace_launches) * w.trace_stride : nullptr;
+  const int pdl = (a.allow_pdl && pdl_enabled()) ? 1 : 0;
 
-  int bn;
-  if (a.force_bn) {
-    bn = a.force_bn;
-  } else if (swapped) {
-    bn = a.tokens <= 32 ? 32 : a.tokens <= 64 ? 64 : a.tokens <= 128 ? 128 : 256;
-  } else {
-    bn = a.features >= 256 ? 256 : a.features > 64 ? 128 : 64;
+  if (!swapped) {
+    // token-heavy contractions (ViT / mapper / prefill) take the persistent kernels.  Their vector store path assumes
+    // 16-byte aligned bases; it falls back to scalar stores through odd ldo otherwise.
+    if ((reinterpret_cast<uintptr_t>(a.out) & 15) || (a.residual && (reinterpret_cast<uintptr_t>(a.residual) & 15)) ||
+        (a.bias && (reinterpret_cast<uintptr_t>(a.bias) & 15)))
+      return fail("normal-orientation GEMM needs 16-byte aligned out / residual / bias");
+    bool pair = false;
+    int bn = 0;
+    pick_persist(a.tokens, a.features, a.K / 64, w.num_sms, a.force_orientation, a.force_bn, &pair, &bn);
+    if (bn < 32 || bn > 256 || bn % 32) return fail("unsupported BN for the persistent GEMM");
+    return launch_persist(a, bn, pair, pdl, w.num_sms, stream);
   }
-  // token-heavy contractions (ViT / mapper / prefill) take the persistent kernel; force_split pins the
-  // one-tile-per-CTA kernel (tuning / A-B)
-  const bool persist = !swapped && a.force_split == 0;
-  if (!persist && bn != 32 && bn != 64 && bn != 128 && bn != 256) return fail("unsupported BN");
-  if (swapped && bn < a.tokens) return fail("swapped orientation: BN smaller than token count");
+
+  // swapped: weights on the 128-row side of the one-tile-per-CTA kernel, the tokens fill a BN-wide tile
+  const int bn = a.force_bn ? a.force_bn : a.tokens <= 32 ? 32 : a.tokens <= 64 ? 64 : a.tokens <= 128 ? 128 : 256;
+  if (bn != 32 && bn != 64 && bn != 128 && bn != 256) return fail("unsupported BN");
+  if (bn < a.tokens) return fail("swapped orientation: BN smaller than token count");
 
   GemmParams p;
   memset(&p, 0, sizeof(p));
-  const bf16* A = swapped ? a.weight : a.act;
-  const bf16* B = swapped ? a.act : a.weight;
-  p.Ra = swapped ? a.features : a.tokens;
-  p.Rb = swapped ? a.tokens : a.features;
-  const long long ldw = a.ldw ? a.ldw : a.K;
-  const long long ldA = swapped ? ldw : a.lda;
-  const long long ldB = swapped ? a.lda : ldw;
+  p.Ra = a.features;
+  p.Rb = a.tokens;
   p.k_blocks = a.K / 64;
   p.out = a.out;
   p.out_bf16 = a.out_bf16;
-  p.transposed = swapped ? 1 : 0;
   p.ldo = a.ldo;
   p.bias = a.bias;
   p.residual = a.residual;
   p.ldr = a.ldr;
   p.act = a.act_fn;
-  p.rg_in = a.rg_in;
-  p.rg_out = a.rg_out;
-  p.rg_off = a.rg_off;
-  p.trace = w.trace ? w.trace + (w.trace_count++ % w.trace_launches) * w.trace_stride : nullptr;
-  p.pdl = (a.allow_pdl && pdl_enabled()) ? 1 : 0;
-  // the vector store path assumes 16-byte aligned bases; fall back to scalar stores through odd ldo otherwise
-  if (!swapped) {
-    if ((reinterpret_cast<uintptr_t>(a.out) & 15) || (a.residual && (reinterpret_cast<uintptr_t>(a.residual) & 15)) ||
-        (a.bias && (reinterpret_cast<uintptr_t>(a.bias) & 15)))
-      return fail("normal-orientation GEMM needs 16-byte aligned out / residual / bias");
-  }
-
-  if (persist) {
-    bool pair = false;
-    int pbn = 0;
-    pick_persist(a.tokens, a.features, p.k_blocks, w.num_sms, a.force_orientation, a.force_bn, &pair, &pbn);
-    if (pbn < 32 || pbn > 256 || pbn % 32) return fail("unsupported BN for the persistent GEMM");
-    return launch_persist(a, p, pbn, pair, w.num_sms, stream);
-  }
+  p.trace = trace;
+  p.pdl = pdl;
 
   dim3 grid((p.Ra + 127) / 128, (p.Rb + bn - 1) / bn, 1);
   const int tiles = grid.x * grid.y;
@@ -298,20 +293,12 @@ int gemm_launch(const GemmArgs& a, const GemmWorkspace& w, cudaStream_t stream) 
     const int slots = w.num_sms * (bn == 32 ? 2 : 1);
     if (tiles < slots) {
       split = slots / tiles;
-      static const int min_kb = [] {   // k-blocks a split must own at least (tuning: CCB_GEMM_MINKB)
-        const char* e = getenv("CCB_GEMM_MINKB");
-        return e && atoi(e) > 0 ? atoi(e) : 4;
-      }();
-      const int max_by_k = p.k_blocks / min_kb > 0 ? p.k_blocks / min_kb : 1;
+      const int max_by_k = p.k_blocks / 4 > 0 ? p.k_blocks / 4 : 1;
       if (split > max_by_k) split = max_by_k;
       // with two CTAs per SM, clusters of 3, 5, 6 or 7 CTAs place badly on the GPCs (the 96-tile x 3 q/k/v GEMM of a 16-row
       // GPT-J step: 32 us against 26 us with pairs; GPT-J step 3.02 -> 2.91 ms): round the split down to a power of two.
       // One CTA per SM (64-token tiles: the GPT2-XL operator chain) is 2 % faster with the odd splits, so it keeps them.
-      static const bool pow2 = [] {
-        const char* e = getenv("CCB_GEMM_SPLIT_ANY");
-        return !(e && e[0] == '1');
-      }();
-      if (pow2 && bn == 32)
+      if (bn == 32)
         while (split & (split - 1)) --split;
     }
   }
@@ -323,8 +310,8 @@ int gemm_launch(const GemmArgs& a, const GemmWorkspace& w, cudaStream_t stream) 
   grid.z = split;
 
   CUtensorMap ta, tb;
-  if (make_tmap(&ta, A, p.Ra, a.K, ldA, 128)) return -1;
-  if (make_tmap(&tb, B, p.Rb, a.K, ldB, bn)) return -1;
+  if (make_tmap(&ta, a.weight, a.features, a.K, a.ldw ? a.ldw : a.K, 128)) return -1;
+  if (make_tmap(&tb, a.act, a.tokens, a.K, a.lda, bn)) return -1;
 
   switch (bn) {
     case 32: return launch<32>(ta, tb, p, grid, stream);

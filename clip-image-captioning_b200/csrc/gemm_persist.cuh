@@ -20,7 +20,18 @@
 namespace ccb {
 
 struct PersistParams {
-  GemmParams g;     // Ra = tokens, Rb = features, k_blocks, epilogue description (transposed == 0, split_k == 1)
+  int tokens, features;    // valid rows of X / W (tile rows beyond are zero-filled by TMA and masked at the store)
+  int k_blocks;            // K / 64
+  // epilogue: out[out_row(t) * ldo + f] = act(acc[t, f] + bias[f]) + residual[out_row(t) * ldr + f]
+  void* out;               // f32 or bf16
+  int out_bf16;
+  long long ldo;
+  const float* bias;       // per feature; may be null
+  const float* residual;   // f32; may be null (may alias out)
+  long long ldr;
+  int act;
+  // row remap: out_row(t) = (t / rg_in) * rg_out + rg_off + (t % rg_in); rg_in == 0 -> identity
+  int rg_in, rg_out, rg_off;
   int bn;           // tile width in features (multiple of 32, <= 256)
   int stages;       // TMA ring depth
   int m_tiles, n_tiles;
@@ -29,29 +40,108 @@ struct PersistParams {
 constexpr int kPersistThreads = 224;
 constexpr int kPersistSmemBytes = 227 * 1024;
 
-// Epilogue of one accumulator tile for one warp (thread = token row after tcgen05.ld): 32-column chunks through the
-// fused bias / activation / residual / store of gemm_sm100.cuh; the accumulator buffer is handed back to the MMA
-// issuer (`release`) after the last TMEM read, before the stores of the final chunk.
+// Fused epilogue on the 32 accumulator columns [j0, j0 + 32) of token row out_row (see gemm_apply_act for why it is kept
+// small).
+__device__ __forceinline__ void persist_epilogue_cols(const PersistParams& p, float (&acc)[32], bool i_ok, long long out_row,
+                                                      int j0, bool vec_ok) {
+  if (!i_ok) return;
+  if (p.bias != nullptr) {
+#pragma unroll
+    for (int v = 0; v < 32; ++v) acc[v] += (j0 + v < p.features) ? __ldg(p.bias + j0 + v) : 0.f;
+  }
+  gemm_apply_act(acc, p.act);
+  if (vec_ok && j0 + 32 <= p.features) {
+    if (p.residual) {
+#pragma unroll
+      for (int v = 0; v < 32; v += 4) {
+        const float4 r4 = *reinterpret_cast<const float4*>(p.residual + out_row * p.ldr + j0 + v);
+        acc[v] += r4.x; acc[v + 1] += r4.y; acc[v + 2] += r4.z; acc[v + 3] += r4.w;
+      }
+    }
+    // Whole 32-byte sectors per store instruction where the row allows it (256-bit st.global): a 16-byte store
+    // is a PARTIAL sector write, which L2 has to merge (and, for a sector that is not resident, fill from DRAM first);
+    // with thread = row every lane of a store hits a different sector, so the 16-byte form doubled the write requests
+    // and cost the persistent kernels 20 % although the epilogue runs underneath the main loop.
+    if (p.out_bf16) {
+      __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out) + out_row * p.ldo + j0;
+      if ((reinterpret_cast<uintptr_t>(o) & 31) == 0) {
+#pragma unroll
+        for (int v = 0; v < 32; v += 16) {
+          uint32_t k[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) k[e] = pack_bf16x2(acc[v + 2 * e], acc[v + 2 * e + 1]);
+          ptx::st_global_256(o + v, k);
+        }
+      } else {
+#pragma unroll
+        for (int v = 0; v < 32; v += 8) {
+          uint4 pk;
+          pk.x = pack_bf16x2(acc[v], acc[v + 1]);
+          pk.y = pack_bf16x2(acc[v + 2], acc[v + 3]);
+          pk.z = pack_bf16x2(acc[v + 4], acc[v + 5]);
+          pk.w = pack_bf16x2(acc[v + 6], acc[v + 7]);
+          *reinterpret_cast<uint4*>(o + v) = pk;
+        }
+      }
+    } else {
+      float* o = reinterpret_cast<float*>(p.out) + out_row * p.ldo + j0;
+      if ((reinterpret_cast<uintptr_t>(o) & 31) == 0) {
+#pragma unroll
+        for (int v = 0; v < 32; v += 8) {
+          uint32_t k[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) k[e] = __float_as_uint(acc[v + e]);
+          ptx::st_global_256(o + v, k);
+        }
+      } else {
+#pragma unroll
+        for (int v = 0; v < 32; v += 4)
+          *reinterpret_cast<float4*>(o + v) = make_float4(acc[v], acc[v + 1], acc[v + 2], acc[v + 3]);
+      }
+    }
+  } else {
+    if (p.residual) {
+      float res[32];
+#pragma unroll
+      for (int v = 0; v < 32; ++v) res[v] = (j0 + v < p.features) ? p.residual[out_row * p.ldr + j0 + v] : 0.f;
+#pragma unroll
+      for (int v = 0; v < 32; ++v) acc[v] += res[v];
+    }
+#pragma unroll
+    for (int v = 0; v < 32; ++v) {
+      const int j = j0 + v;
+      if (j < p.features) {
+        if (p.out_bf16)
+          reinterpret_cast<__nv_bfloat16*>(p.out)[out_row * p.ldo + j] = __float2bfloat16_rn(acc[v]);
+        else
+          reinterpret_cast<float*>(p.out)[out_row * p.ldo + j] = acc[v];
+      }
+    }
+  }
+}
+
+// Epilogue of one accumulator tile for one warp (thread = token row after tcgen05.ld): 32-column chunks through
+// persist_epilogue_cols; the accumulator buffer is handed back to the MMA issuer (`release`) after the last TMEM read,
+// before the stores of the final chunk.
 // (Tried and dropped: staging the chunks through shared memory for row-contiguous 128-byte stores.  The main loop
 // already saturates the SM's shared-memory port -- TMA writes 48 KB and the MMAs read 48 KB per k-block, 0.38 us at
 // 128 B/clk -- so the extra ld/st.shared of the epilogue warps starve: 125 us instead of 90 us on 5120 x 6400 x 1600.)
 template <class Release>
-__device__ __forceinline__ void persist_epilogue_tile(const PersistParams& pp, uint32_t taddr, int i, int row_b0, int lane,
+__device__ __forceinline__ void persist_epilogue_tile(const PersistParams& p, uint32_t taddr, int i, int row_b0, int lane,
                                                       Release release) {
-  const GemmParams& p = pp.g;
-  const int BN = pp.bn;
-  const bool i_ok = i < p.Ra;
+  const int BN = p.bn;
+  const bool i_ok = i < p.tokens;
   long long out_row = i;
   if (p.rg_in > 0) out_row = static_cast<long long>(i / p.rg_in) * p.rg_out + p.rg_off + (i % p.rg_in);
   const bool vec_ok = ((p.ldo & 7) == 0) && (p.residual == nullptr || (p.ldr & 3) == 0);
 #pragma unroll 1
   for (int c0 = 0; c0 < BN; c0 += 32) {
     const int j0 = row_b0 + c0;
-    if (j0 >= p.Rb) break;
+    if (j0 >= p.features) break;
     uint32_t r[32];
     ptx::tmem_ld32(taddr + c0, r);
     ptx::tmem_ld_wait();
-    if (c0 + 32 >= BN || j0 + 32 >= p.Rb) {
+    if (c0 + 32 >= BN || j0 + 32 >= p.features) {
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) release();
@@ -59,16 +149,15 @@ __device__ __forceinline__ void persist_epilogue_tile(const PersistParams& pp, u
     float acc[32];
 #pragma unroll
     for (int v = 0; v < 32; ++v) acc[v] = __uint_as_float(r[v]);
-    gemm_epilogue_cols<32>(p, acc, i, i_ok, out_row, 0.f, j0, vec_ok);
+    persist_epilogue_cols(p, acc, i_ok, out_row, j0, vec_ok);
   }
 }
 
 __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const __grid_constant__ CUtensorMap tma_x,
                                                                          const __grid_constant__ CUtensorMap tma_w,
-                                                                         const PersistParams pp) {
+                                                                         const PersistParams p) {
   extern __shared__ uint8_t smem_raw[];
-  const GemmParams& p = pp.g;
-  const int BN = pp.bn, S = pp.stages;
+  const int BN = p.bn, S = p.stages;
   const uint32_t stage_bytes = 128u * 128u + static_cast<uint32_t>(BN) * 128u;
   const uint32_t smem_base = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bar_base = smem_base + static_cast<uint32_t>(S) * stage_bytes;
@@ -100,7 +189,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
   const uint32_t tmem_base = *tmem_slot_ptr;
   ptx::grid_dep_launch();
 
-  const int ntiles = pp.m_tiles * pp.n_tiles;
+  const int ntiles = p.m_tiles * p.n_tiles;
   const int nkb = p.k_blocks;
 
   if (warp == 0 || warp == 6) {
@@ -117,7 +206,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
       uint32_t s = 0, ph = 0;
 #pragma unroll 1
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int row = is_x ? (tile % pp.m_tiles) * 128 : (tile / pp.m_tiles) * BN;
+        const int row = is_x ? (tile % p.m_tiles) * 128 : (tile / p.m_tiles) * BN;
 #pragma unroll 1
         for (int kb = 0; kb < nkb; ++kb) {
           ptx::mbar_wait(empty0 + 8u * s, ph ^ 1);
@@ -172,14 +261,14 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
     const int quad = warp & 3;
     uint32_t it = 0;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-      const int m_blk = tile % pp.m_tiles, n_blk = tile / pp.m_tiles;
+      const int m_blk = tile % p.m_tiles, n_blk = tile / p.m_tiles;
       const uint32_t buf = it & 1, aph = (it >> 1) & 1;
       const int i = m_blk * 128 + quad * 32 + lane;
       ptx::mbar_wait(tfull0 + 8u * buf, aph);
       ptx::tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + buf * 256u;
       const uint32_t rel = tempty0 + 8u * buf;
-      persist_epilogue_tile(pp, taddr, i, n_blk * BN, lane, [rel]() { ptx::mbar_arrive(rel); });
+      persist_epilogue_tile(p, taddr, i, n_blk * BN, lane, [rel]() { ptx::mbar_arrive(rel); });
     }
   }
 
@@ -200,10 +289,9 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
 // barriers; `empty` and `tmem_full` are signalled in both CTAs by multicast commits.
 __global__ void __launch_bounds__(kPersistThreads, 1) gemm_pair_kernel(const __grid_constant__ CUtensorMap tma_x,
                                                                       const __grid_constant__ CUtensorMap tma_w,
-                                                                      const PersistParams pp) {
+                                                                      const PersistParams p) {
   extern __shared__ uint8_t smem_raw[];
-  const GemmParams& p = pp.g;
-  const int BN = pp.bn, S = pp.stages;
+  const int BN = p.bn, S = p.stages;
   const uint32_t w_bytes = static_cast<uint32_t>(BN) * 64u;            // BN / 2 rows x 128 B
   const uint32_t stage_bytes = 128u * 128u + w_bytes;
   const uint32_t smem_base = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -238,7 +326,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_pair_kernel(const __g
   const uint32_t tmem_base = *tmem_slot_ptr;
   ptx::grid_dep_launch();
 
-  const int ntiles = pp.m_tiles * pp.n_tiles;      // m_tiles counts 256-row pair tiles
+  const int ntiles = p.m_tiles * p.n_tiles;       // m_tiles counts 256-row pair tiles
   const int nkb = p.k_blocks;
   const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
 
@@ -254,8 +342,8 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_pair_kernel(const __g
       uint32_t s = 0, ph = 0;
 #pragma unroll 1
       for (int tile = pair; tile < ntiles; tile += npairs) {
-        const int row = is_x ? (tile % pp.m_tiles) * 256 + static_cast<int>(rank) * 128
-                             : (tile / pp.m_tiles) * BN + static_cast<int>(rank) * (BN >> 1);
+        const int row = is_x ? (tile % p.m_tiles) * 256 + static_cast<int>(rank) * 128
+                             : (tile / p.m_tiles) * BN + static_cast<int>(rank) * (BN >> 1);
 #pragma unroll 1
         for (int kb = 0; kb < nkb; ++kb) {
           ptx::mbar_wait(empty0 + 8u * s, ph ^ 1);
@@ -306,14 +394,14 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_pair_kernel(const __g
     const uint32_t ltempty0 = ptx::mapa_shared(tempty0, 0);
     uint32_t it = 0;
     for (int tile = pair; tile < ntiles; tile += npairs, ++it) {
-      const int m_blk = tile % pp.m_tiles, n_blk = tile / pp.m_tiles;
+      const int m_blk = tile % p.m_tiles, n_blk = tile / p.m_tiles;
       const uint32_t buf = it & 1, aph = (it >> 1) & 1;
       const int i = m_blk * 256 + static_cast<int>(rank) * 128 + quad * 32 + lane;
       ptx::mbar_wait(tfull0 + 8u * buf, aph);
       ptx::tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + buf * 256u;
       const uint32_t rel = ltempty0 + 8u * buf;
-      persist_epilogue_tile(pp, taddr, i, n_blk * BN, lane, [rel]() { ptx::mbar_arrive_cluster(rel); });
+      persist_epilogue_tile(p, taddr, i, n_blk * BN, lane, [rel]() { ptx::mbar_arrive_cluster(rel); });
     }
   }
 

@@ -1,12 +1,11 @@
-// bf16 x bf16 -> fp32 GEMM for sm_100a: TMA (128B-swizzled K-major tiles) -> tcgen05.mma with the accumulator
-// in TMEM -> tcgen05.ld epilogue with fused bias / activation / residual and an optional transposed store.
+// bf16 x bf16 -> fp32 GEMM for sm_100a, one output tile per CTA: TMA (128B-swizzled K-major tiles) -> tcgen05.mma with
+// the accumulator in TMEM -> tcgen05.ld epilogue with fused bias / activation / residual and a transposed store.
 //
-//   acc[i, j] = sum_k A[i, k] * B[j, k]          A: [Ra, K] bf16 row-major, B: [Rb, K] bf16 row-major
+//   out[j, i] = sum_k A[i, k] * B[j, k]      A = weights [features, K], B = activations [tokens, K], bf16 row-major
 //
-// "normal" orientation   : A = activations (tokens x K), B = weights (features x K) -> out[token, feature]
-// "swapped" orientation  : A = weights (features x K),  B = activations (tokens x K) -> out[token, feature]
-//                          written through the transposed store.  Used when tokens <= 256 (decode), so the
-//                          128-row MMA tile is filled by weight rows and every weight byte is streamed once.
+// This is the "swapped" orientation of gemm.cu, used when tokens <= 256 (decode): the 128-row MMA tile is filled by
+// weight rows and every weight byte is streamed once.  Token-heavy contractions (tokens on the 128-row side) run on the
+// persistent kernels of gemm_persist.cuh.
 //
 // One CTA computes one 128 x BN tile (optionally one K-split of it).  Warp roles: warp 0 = TMA producer,
 // warp 1 = TMEM allocator + MMA issuer (one elected lane), warps 2..5 = epilogue (one TMEM lane quadrant
@@ -22,20 +21,17 @@
 namespace ccb {
 
 struct GemmParams {
-  int Ra, Rb;        // valid rows of A / B (tile rows beyond are zero-filled by TMA and masked at the store)
+  int Ra, Rb;        // valid rows of A (features) / B (tokens): tile rows beyond are zero-filled by TMA and masked at the store
   int k_blocks;      // K / 64
   int split_k;       // >= 1; == cluster size along z
-  // epilogue
+  // epilogue: out[j * ldo + i] = act(acc[i, j] + bias[i]) + residual[j * ldr + i]
   void* out;         // f32 or bf16
   int out_bf16;
-  int transposed;    // 0: out[i*ldo + j]   1: out[j*ldo + i]
   long long ldo;
-  const float* bias;       // per feature: index j (normal) or i (transposed); may be null
-  const float* residual;   // f32, same indexing as out with leading dim ldr; may be null (may alias out)
+  const float* bias;       // per feature i; may be null
+  const float* residual;   // f32; may be null (may alias out)
   long long ldr;
   int act;
-  // normal-mode row remap: out_row = (i / rg_in) * rg_out + rg_off + (i % rg_in); rg_in == 0 -> identity
-  int rg_in, rg_out, rg_off;
   // 1: launched with programmatic stream serialization inside the engine's chain: weight tiles are fetched
   // before the dependency wait (they are never produced by the preceding kernel)
   int pdl;
@@ -76,24 +72,15 @@ struct GemmCfg {
 #define CCB_TRACE(slot) do { } while (0)
 #endif
 
-// Fused epilogue on CW accumulator columns [c0, c0 + CW) of this thread's row.  Kept small on purpose: it runs
-// once per tile, so its instructions are cold in the instruction cache (a fully unrolled epilogue with the
-// activation switch inlined was 22 K instructions and cost ~15 us per tile in instruction fetches).
+// The fused epilogues (gemm_epilogue_transposed below, persist_epilogue_cols in gemm_persist.cuh) are kept small on
+// purpose: they run once per tile, so their instructions are cold in the instruction cache (a fully unrolled epilogue
+// with the activation switch inlined was 22 K instructions and cost ~15 us per tile in instruction fetches).
 template <int CW>
-__device__ __forceinline__ void gemm_epilogue_cols(const GemmParams& p, float (&acc)[CW], int i, bool i_ok,
-                                                   long long out_row, float bias_i, int j0, bool vec_ok) {
-  if (!i_ok) return;
-  if (p.transposed) {
-#pragma unroll
-    for (int v = 0; v < CW; ++v) acc[v] += bias_i;
-  } else if (p.bias != nullptr) {
-#pragma unroll
-    for (int v = 0; v < CW; ++v) acc[v] += (j0 + v < p.Rb) ? __ldg(p.bias + j0 + v) : 0.f;
-  }
-  if (p.act == ACT_RELU) {
+__device__ __forceinline__ void gemm_apply_act(float (&acc)[CW], int act) {
+  if (act == ACT_RELU) {
 #pragma unroll
     for (int v = 0; v < CW; ++v) acc[v] = fmaxf(acc[v], 0.f);
-  } else if (p.act == ACT_GELU_NEW) {
+  } else if (act == ACT_GELU_NEW) {
     // 0.5 x (1 + tanh(u)) == x - x / (1 + exp(2u)); exp2-based __expf + fast divide: ~1e-6 relative error, far
     // below the bf16 rounding of the stored value, and a handful of instructions (the epilogue has 4 warps)
 #pragma unroll
@@ -102,100 +89,40 @@ __device__ __forceinline__ void gemm_epilogue_cols(const GemmParams& p, float (&
       const float u = 0.7978845608028654f * (x + 0.044715f * x * x * x);
       acc[v] = x - __fdividef(x, 1.f + __expf(2.f * u));
     }
-  } else if (p.act == ACT_QUICKGELU) {
+  } else if (act == ACT_QUICKGELU) {
 #pragma unroll
     for (int v = 0; v < CW; ++v) acc[v] = __fdividef(acc[v], 1.f + __expf(-1.702f * acc[v]));
-  } else if (p.act != ACT_NONE) {
+  } else if (act != ACT_NONE) {
 #pragma unroll
-    for (int v = 0; v < CW; ++v) acc[v] = apply_act_call(acc[v], p.act);  // static indices keep acc in registers
+    for (int v = 0; v < CW; ++v) acc[v] = apply_act_call(acc[v], act);  // static indices keep acc in registers
   }
-  if (p.transposed) {
-    // lanes hold consecutive features i -> coalesced accesses for every token j.  All residual loads are issued
-    // before the first store: out may alias residual (in-place residual stream), so a load placed after a store
-    // could not be hoisted by the compiler and the CW load latencies would serialise.
-    if (p.residual) {
-      float res[CW];
+}
+
+// Epilogue of feature i (this thread's accumulator row) for the 8 tokens [j0, j0 + 8).
+__device__ __forceinline__ void gemm_epilogue_transposed(const GemmParams& p, float (&acc)[8], int i, bool i_ok,
+                                                         float bias_i, int j0) {
+  if (!i_ok) return;
 #pragma unroll
-      for (int v = 0; v < CW; ++v) res[v] = (j0 + v < p.Rb) ? p.residual[static_cast<long long>(j0 + v) * p.ldr + i] : 0.f;
+  for (int v = 0; v < 8; ++v) acc[v] += bias_i;
+  gemm_apply_act(acc, p.act);
+  // lanes hold consecutive features i -> coalesced accesses for every token j.  All residual loads are issued
+  // before the first store: out may alias residual (in-place residual stream), so a load placed after a store
+  // could not be hoisted by the compiler and the 8 load latencies would serialise.
+  if (p.residual) {
+    float res[8];
 #pragma unroll
-      for (int v = 0; v < CW; ++v) acc[v] += res[v];
-    }
+    for (int v = 0; v < 8; ++v) res[v] = (j0 + v < p.Rb) ? p.residual[static_cast<long long>(j0 + v) * p.ldr + i] : 0.f;
 #pragma unroll
-    for (int v = 0; v < CW; ++v) {
-      const int j = j0 + v;
-      if (j < p.Rb) {
-        if (p.out_bf16)
-          reinterpret_cast<__nv_bfloat16*>(p.out)[static_cast<long long>(j) * p.ldo + i] = __float2bfloat16_rn(acc[v]);
-        else
-          reinterpret_cast<float*>(p.out)[static_cast<long long>(j) * p.ldo + i] = acc[v];
-      }
-    }
-  } else if (vec_ok && j0 + CW <= p.Rb) {
-    if (p.residual) {
+    for (int v = 0; v < 8; ++v) acc[v] += res[v];
+  }
 #pragma unroll
-      for (int v = 0; v < CW; v += 4) {
-        const float4 r4 = *reinterpret_cast<const float4*>(p.residual + out_row * p.ldr + j0 + v);
-        acc[v] += r4.x; acc[v + 1] += r4.y; acc[v + 2] += r4.z; acc[v + 3] += r4.w;
-      }
-    }
-    // Whole 32-byte sectors per store instruction where the row allows it (256-bit st.global): a 16-byte store
-    // is a PARTIAL sector write, which L2 has to merge (and, for a sector that is not resident, fill from DRAM first);
-    // with thread = row every lane of a store hits a different sector, so the 16-byte form doubled the write requests
-    // and cost the persistent kernels 20 % although the epilogue runs underneath the main loop.
-    if (p.out_bf16) {
-      __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out) + out_row * p.ldo + j0;
-      if (CW % 16 == 0 && (reinterpret_cast<uintptr_t>(o) & 31) == 0) {
-#pragma unroll
-        for (int v = 0; v + 16 <= CW; v += 16) {
-          uint32_t k[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) k[e] = pack_bf16x2(acc[v + 2 * e], acc[v + 2 * e + 1]);
-          ptx::st_global_256(o + v, k);
-        }
-      } else {
-#pragma unroll
-        for (int v = 0; v < CW; v += 8) {
-          uint4 pk;
-          pk.x = pack_bf16x2(acc[v], acc[v + 1]);
-          pk.y = pack_bf16x2(acc[v + 2], acc[v + 3]);
-          pk.z = pack_bf16x2(acc[v + 4], acc[v + 5]);
-          pk.w = pack_bf16x2(acc[v + 6], acc[v + 7]);
-          *reinterpret_cast<uint4*>(o + v) = pk;
-        }
-      }
-    } else {
-      float* o = reinterpret_cast<float*>(p.out) + out_row * p.ldo + j0;
-      if (CW % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 31) == 0) {
-#pragma unroll
-        for (int v = 0; v + 8 <= CW; v += 8) {
-          uint32_t k[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) k[e] = __float_as_uint(acc[v + e]);
-          ptx::st_global_256(o + v, k);
-        }
-      } else {
-#pragma unroll
-        for (int v = 0; v < CW; v += 4)
-          *reinterpret_cast<float4*>(o + v) = make_float4(acc[v], acc[v + 1], acc[v + 2], acc[v + 3]);
-      }
-    }
-  } else {
-    if (p.residual) {
-      float res[CW];
-#pragma unroll
-      for (int v = 0; v < CW; ++v) res[v] = (j0 + v < p.Rb) ? p.residual[out_row * p.ldr + j0 + v] : 0.f;
-#pragma unroll
-      for (int v = 0; v < CW; ++v) acc[v] += res[v];
-    }
-#pragma unroll
-    for (int v = 0; v < CW; ++v) {
-      const int j = j0 + v;
-      if (j < p.Rb) {
-        if (p.out_bf16)
-          reinterpret_cast<__nv_bfloat16*>(p.out)[out_row * p.ldo + j] = __float2bfloat16_rn(acc[v]);
-        else
-          reinterpret_cast<float*>(p.out)[out_row * p.ldo + j] = acc[v];
-      }
+  for (int v = 0; v < 8; ++v) {
+    const int j = j0 + v;
+    if (j < p.Rb) {
+      if (p.out_bf16)
+        reinterpret_cast<__nv_bfloat16*>(p.out)[static_cast<long long>(j) * p.ldo + i] = __float2bfloat16_rn(acc[v]);
+      else
+        reinterpret_cast<float*>(p.out)[static_cast<long long>(j) * p.ldo + i] = acc[v];
     }
   }
 }
@@ -262,27 +189,18 @@ __global__ void __launch_bounds__(192, GemmCfg<BN>::kMinBlocks) gemm_bf16_tn_ker
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
     if (lane == 0) {
-      // weights are streamed once (evict-first); activations are re-read by many CTAs (evict-last)
-      const uint64_t hint_a = p.transposed ? ptx::kEvictFirst : ptx::kEvictLast;
-      const uint64_t hint_b = p.transposed ? ptx::kEvictLast : ptx::kEvictNormal;
-      // Weights (A when transposed, else B) do not depend on the preceding kernel: with PDL their first
-      // kStages tiles are requested before the dependency wait, the activation tiles right after it.
-      const CUtensorMap* w_map = p.transposed ? &tma_a : &tma_b;
-      const CUtensorMap* x_map = p.transposed ? &tma_b : &tma_a;
-      const uint32_t w_off = p.transposed ? 0u : static_cast<uint32_t>(Cfg::kABytes);
-      const uint32_t x_off = p.transposed ? static_cast<uint32_t>(Cfg::kABytes) : 0u;
-      const int w_row = p.transposed ? row_a0 : row_b0;
-      const int x_row = p.transposed ? row_b0 : row_a0;
-      const uint64_t w_hint = p.transposed ? hint_a : hint_b;
-      const uint64_t x_hint = p.transposed ? hint_b : hint_a;
+      // weights (A) are streamed once (evict-first); activations (B) are re-read by many CTAs (evict-last).  The weights
+      // do not depend on the preceding kernel: with PDL their first kStages tiles are requested before the dependency
+      // wait, the activation tiles right after it.
       const int pre = p.pdl ? (nkb < kStages ? nkb : kStages) : 0;
       for (int it = 0; it < pre; ++it) {
         ptx::mbar_arrive_expect_tx(full_bar(it), Cfg::kStageBytes);
-        ptx::tma_load_2d(smem_base + it * Cfg::kStageBytes + w_off, w_map, full_bar(it), (kb_begin + it) * Cfg::BK, w_row, w_hint);
+        ptx::tma_load_2d(smem_base + it * Cfg::kStageBytes, &tma_a, full_bar(it), (kb_begin + it) * Cfg::BK, row_a0, ptx::kEvictFirst);
       }
       ptx::grid_dep_wait();
       for (int it = 0; it < pre; ++it)
-        ptx::tma_load_2d(smem_base + it * Cfg::kStageBytes + x_off, x_map, full_bar(it), (kb_begin + it) * Cfg::BK, x_row, x_hint);
+        ptx::tma_load_2d(smem_base + it * Cfg::kStageBytes + Cfg::kABytes, &tma_b, full_bar(it), (kb_begin + it) * Cfg::BK, row_b0,
+                         ptx::kEvictLast);
       for (int it = pre; it < nkb; ++it) {
         const int s = it % kStages;
         const uint32_t ph = (it / kStages) & 1;
@@ -290,8 +208,8 @@ __global__ void __launch_bounds__(192, GemmCfg<BN>::kMinBlocks) gemm_bf16_tn_ker
         const uint32_t st = smem_base + s * Cfg::kStageBytes;
         ptx::mbar_arrive_expect_tx(full_bar(s), Cfg::kStageBytes);
         const int kcoord = (kb_begin + it) * Cfg::BK;
-        ptx::tma_load_2d(st + w_off, w_map, full_bar(s), kcoord, w_row, w_hint);
-        ptx::tma_load_2d(st + x_off, x_map, full_bar(s), kcoord, x_row, x_hint);
+        ptx::tma_load_2d(st, &tma_a, full_bar(s), kcoord, row_a0, ptx::kEvictFirst);
+        ptx::tma_load_2d(st + Cfg::kABytes, &tma_b, full_bar(s), kcoord, row_b0, ptx::kEvictLast);
       }
     }
     __syncwarp();
@@ -328,10 +246,6 @@ __global__ void __launch_bounds__(192, GemmCfg<BN>::kMinBlocks) gemm_bf16_tn_ker
     if (warp == 2) CCB_TRACE(4);  // accumulator ready
   }
 
-  long long out_row = i;
-  if (!p.transposed && p.rg_in > 0) out_row = static_cast<long long>(i / p.rg_in) * p.rg_out + p.rg_off + (i % p.rg_in);
-  const bool vec_ok = !p.transposed && ((p.ldo & 7) == 0) && (p.residual == nullptr || (p.ldr & 3) == 0);
-
   if (p.split_k > 1) {
     // ------------------------------------------------------------ split-K: push-based cluster reduction
     // The BN/8 groups of 8 columns are dealt round-robin to the S CTAs of the cluster (owner of group c = c % S).
@@ -365,7 +279,7 @@ __global__ void __launch_bounds__(192, GemmCfg<BN>::kMinBlocks) gemm_bf16_tn_ker
     ptx::cluster_wait();
     if (warp == 2) CCB_TRACE(5);
     if (warp >= 2) {
-      const float bias_i = (p.transposed && p.bias != nullptr && i_ok) ? p.bias[i] : 0.f;
+      const float bias_i = (p.bias != nullptr && i_ok) ? p.bias[i] : 0.f;
       const uint32_t row_off = static_cast<uint32_t>(quad * 32 + lane) * 4u;
 #pragma unroll 1
       for (uint32_t c = my_rank, li = 0; c < NC; c += S, ++li) {
@@ -380,38 +294,23 @@ __global__ void __launch_bounds__(192, GemmCfg<BN>::kMinBlocks) gemm_bf16_tn_ker
 #pragma unroll
           for (int v = 0; v < 8; ++v) acc[v] += ptx::ld_shared_f32(src + v * 512u);
         }
-        gemm_epilogue_cols<8>(p, acc, i, i_ok, out_row, bias_i, j0, vec_ok);
+        gemm_epilogue_transposed(p, acc, i, i_ok, bias_i, j0);
       }
       if (warp == 2) CCB_TRACE(6);  // epilogue done
     }
   } else if (warp >= 2) {
-    const float bias_i = (p.transposed && p.bias != nullptr && i_ok) ? p.bias[i] : 0.f;
-    if (p.transposed) {
+    const float bias_i = (p.bias != nullptr && i_ok) ? p.bias[i] : 0.f;
 #pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 8) {
-        const int j0 = row_b0 + c0;
-        if (j0 >= p.Rb) break;
-        uint32_t r[8];
-        ptx::tmem_ld8(taddr + c0, r);
-        ptx::tmem_ld_wait();
-        float acc[8];
+    for (int c0 = 0; c0 < BN; c0 += 8) {
+      const int j0 = row_b0 + c0;
+      if (j0 >= p.Rb) break;
+      uint32_t r[8];
+      ptx::tmem_ld8(taddr + c0, r);
+      ptx::tmem_ld_wait();
+      float acc[8];
 #pragma unroll
-        for (int v = 0; v < 8; ++v) acc[v] = __uint_as_float(r[v]);
-        gemm_epilogue_cols<8>(p, acc, i, i_ok, out_row, bias_i, j0, vec_ok);
-      }
-    } else {
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 32) {
-        const int j0 = row_b0 + c0;
-        if (j0 >= p.Rb) break;
-        uint32_t r[32];
-        ptx::tmem_ld32(taddr + c0, r);
-        ptx::tmem_ld_wait();
-        float acc[32];
-#pragma unroll
-        for (int v = 0; v < 32; ++v) acc[v] = __uint_as_float(r[v]);
-        gemm_epilogue_cols<32>(p, acc, i, i_ok, out_row, bias_i, j0, vec_ok);
-      }
+      for (int v = 0; v < 8; ++v) acc[v] = __uint_as_float(r[v]);
+      gemm_epilogue_transposed(p, acc, i, i_ok, bias_i, j0);
     }
     if (warp == 2) CCB_TRACE(6);  // epilogue done
   }

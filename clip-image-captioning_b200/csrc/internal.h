@@ -72,9 +72,12 @@ struct GemmArgs {
   long long ldo = 0;
   int out_bf16 = 0;
   int rg_in = 0, rg_out = 0, rg_off = 0;  // out_row = (t / rg_in) * rg_out + rg_off + t % rg_in (0 = identity)
-  int force_orientation = 0;     // 0 auto, 1 normal, 2 swapped
+  // 0 auto (swapped when tokens <= 256), 1 normal (tokens on the 128-row MMA side: the persistent kernels, single-CTA or
+  // CTA pair picked from the shape), 2 swapped (weights on the 128-row side: the one-tile-per-CTA kernel),
+  // 3 normal on the CTA-pair persistent kernel, 4 normal on the single-CTA persistent kernel
+  int force_orientation = 0;
   int force_bn = 0;              // 0 auto
-  int force_split = 0;           // 0 auto
+  int force_split = 0;           // 0 auto; split-K exists in the swapped orientation only (an error otherwise)
   int allow_pdl = 0;             // 1: launched inside the engine's own chain (weights are never produced by the
                                  // preceding kernel, so their loads may start before the dependency wait)
 };

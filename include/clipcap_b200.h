@@ -191,7 +191,10 @@ CCB_API int ccb_beam_step(ccb_ctx* ctx, const float* logits, int64_t ld, int N, 
 /* ---- single operators on caller tensors (used by the parity tests and micro-benchmarks) ------------------ */
 /* out[t, f] = act(sum_k x[t,k] * w[f,k] + bias[f]) + residual[t, f]; x [tokens, K] bf16 (ld lda), w [features, K]
  * bf16, bias f32 or NULL, residual f32 [tokens, ldr] or NULL, out f32 or bf16 [tokens, ldo].
- * orientation: 0 auto, 1 normal (tokens on the 128-row MMA side), 2 swapped (weights on the 128-row side). */
+ * orientation: 0 auto (swapped when tokens <= 256), 1 normal (tokens on the 128-row MMA side), 2 swapped (weights on the
+ * 128-row side, tokens <= 256), 3 normal on the CTA-pair persistent kernel, 4 normal on the single-CTA persistent kernel.
+ * bn: 0 auto, else the tile width in tokens (swapped) or features (normal).  split_k: 0 auto, else the number of K splits;
+ * the swapped orientation only: with the normal orientation a non-zero split_k is an error. */
 CCB_API int ccb_op_linear(ccb_ctx* ctx, const void* x, int64_t lda, int tokens, const void* w, int features, int K,
                   const float* bias, int act, const float* residual, int64_t ldr, void* out, int64_t ldo,
                   int out_bf16, int orientation, int bn, int split_k, void* stream);

@@ -26,11 +26,9 @@ def _ref_linear(x, w, bias, act, residual):
 
 # (tokens, features, K, orientation, bn, split_k)
 LINEAR_CASES = [
-    (128, 256, 64, 1, 0, 1),
-    (128, 128, 128, 1, 128, 1),
-    (300, 520, 256, 1, 0, 1),        # ragged rows / features, normal orientation
-    (300, 520, 256, 1, 64, 1),
-    (2560, 4800, 1600, 1, 256, 1),   # GPT2-XL prefill c_attn
+    (128, 256, 64, 1, 0, 0),
+    (128, 128, 128, 1, 128, 0),
+    (2560, 4800, 1600, 1, 256, 0),   # GPT2-XL prefill c_attn
     (2560, 1600, 6400, 1, 0, 0),     # c_proj of the MLP, auto split
     (64, 4800, 1600, 2, 64, 1),      # decode, swapped orientation
     (64, 4800, 1600, 0, 0, 0),       # decode, auto
@@ -38,10 +36,10 @@ LINEAR_CASES = [
     (1, 768, 768, 0, 0, 0),          # batch 1
     (5, 2304, 768, 2, 32, 3),
     (256, 50257, 128, 2, 256, 1),    # lm_head shape, swapped with odd vocab
-    (200, 1000, 512, 1, 128, 2),     # split-K normal
+    (200, 1000, 512, 1, 128, 0),
     (49, 768, 3072, 0, 0, 0),        # ViT patch embed at batch 1
-    # persistent kernel (normal orientation, split_k = 0): auto and forced tile widths, ragged edges, many tiles per CTA
-    (300, 520, 256, 1, 0, 0),
+    # persistent kernel (normal orientation): auto and forced tile widths, ragged edges, many tiles per CTA
+    (300, 520, 256, 1, 0, 0),        # ragged rows / features
     (300, 520, 256, 1, 64, 0),
     (1000, 100, 128, 1, 96, 0),
     (130, 96, 64, 1, 0, 0),
@@ -74,6 +72,21 @@ def test_linear_matches_torch(tiny_engine, tokens, features, K, orientation, bn,
         err = (out.float() - ref).abs().max().item()
         scale = ref.abs().max().item()
         assert err <= tol * scale + 1e-5, (act, err, scale)
+
+
+def test_linear_split_k_needs_the_swapped_orientation(tiny_engine):
+    """Split-K exists only in the one-tile kernel (weights on the 128-row side): asked for with tokens on that side, it is
+    rejected, not run some other way, and the context keeps working."""
+    g = torch.Generator().manual_seed(7)
+    x = torch.randn(300, 256, generator=g).bfloat16()
+    w = (torch.randn(520, 256, generator=g) * 0.05).bfloat16()
+    with pytest.raises(RuntimeError, match="split-K"):
+        tiny_engine.op_linear(x[:64], w, orientation=1, split_k=2)
+    with pytest.raises(RuntimeError, match="split-K"):
+        tiny_engine.op_linear(x, w, orientation=0, split_k=2)     # 300 tokens: normal orientation
+    out = tiny_engine.op_linear(x, w)
+    ref = _ref_linear(x.cuda(), w.cuda(), None, "none", None)
+    assert (out - ref).abs().max().item() <= 2e-3 * ref.abs().max().item()
 
 
 def test_linear_no_bias_in_place_residual(tiny_engine):

@@ -1,5 +1,6 @@
 """Micro-benchmark of the decode-shaped (weight-streaming) GEMM: rotates over enough weight matrices to stay HBM-cold.
-usage: python tools/bench_gemm.py [tokens] [features] [K] [split_k] [bn] [orientation]"""
+usage: python tools/bench_gemm.py [tokens] [features] [K] [split_k] [bn] [orientation]
+split_k 0 times the forced single split and the automatic choice; split-K needs the swapped orientation (tokens <= 256)."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
