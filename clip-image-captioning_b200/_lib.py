@@ -69,8 +69,10 @@ PROTOTYPES = {
     "ccb_debug_mega_trace": (_I, [_P, _P]),
     "ccb_debug_set_mega": (_I, [_P, _I]),
     "ccb_debug_copy_buffer": (_I, [_P, _I, _P, _L, _P]),
+    "ccb_debug_kv_layout": (_I, [_P, C.POINTER(_L)]),
     "ccb_op_layernorm": (_I, [_P, _P, _P, _P, _F, _P, _I, _I, _P]),
     "ccb_op_attention": (_I, [_P, _P, _P, _I, _I, _I, _I, _F, _I, _I, _P]),
+    "ccb_op_attention_decode": (_I, [_P, _P, _P, _L, _I, _I, _I, _F, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P]),
 }
 
 _lib = None

@@ -1409,6 +1409,7 @@ int ccb_debug_copy_buffer(ccb_ctx* c, int which, void* dst, int64_t bytes, void*
   if (!c || !dst) return -1;
   DeviceGuard dev_guard(c->device);
   const void* src = nullptr;
+  int64_t size = -1;   // known for the KV pool and the block table
   switch (which) {
     case 0: src = c->h; break;
     case 1: src = c->x; break;
@@ -1416,9 +1417,23 @@ int ccb_debug_copy_buffer(ccb_ctx* c, int which, void* dst, int64_t bytes, void*
     case 3: src = c->mlp; break;
     case 4: src = c->logits; break;
     case 5: src = c->qkv; break;
+    case 6: src = c->kv.base; size = static_cast<int64_t>(2) * c->desc.lm_layers * c->kv_pool_tokens * c->desc.lm_d * sizeof(bf16); break;
+    case 7: src = c->block_table; size = static_cast<int64_t>(c->max_rows) * c->max_pages_per_row * sizeof(int); break;
     default: return fail(c, "ccb_debug_copy_buffer: unknown buffer %d", which);
   }
+  if (size >= 0 && (bytes < 0 || bytes > size))
+    return fail(c, "ccb_debug_copy_buffer: %lld bytes requested from buffer %d of %lld bytes", static_cast<long long>(bytes), which,
+                static_cast<long long>(size));
   CUDA_OK(cudaMemcpyAsync(dst, src, static_cast<size_t>(bytes), cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
+int ccb_debug_kv_layout(ccb_ctx* c, int64_t out[6]) {
+  if (!c || !out) return fail(c, "ccb_debug_kv_layout: null argument");
+  if (c->kv.page_tokens <= 0) return fail(c, "ccb_debug_kv_layout: no generate call yet");
+  const KvCache& k = c->kv;
+  const int64_t v[6] = {k.L, k.H, k.hd, k.page_tokens, k.num_pages, k.max_pages_per_row};
+  for (int i = 0; i < 6; ++i) out[i] = v[i];
   return 0;
 }
 
@@ -1442,6 +1457,31 @@ int ccb_op_attention(ccb_ctx* c, const void* qkv_bf16, void* out_bf16, int B, in
   DeviceGuard dev_guard(c->device);
   RUN(attention_prefill(static_cast<const bf16*>(qkv_bf16), static_cast<bf16*>(out_bf16), B, S, H, hd, scale, causal,
                         nullptr, 0, nullptr, 0, rotary_dim, nullptr, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
+int ccb_op_attention_decode(ccb_ctx* c, const void* qkv_bf16, void* out_bf16, int64_t ldo, int rows, int H, int hd, float scale,
+                            void* kv_bf16, int layers, int layer, int num_pages, int page_tokens, int max_pages_per_row,
+                            const int32_t* block_table, const int32_t* ctx_len, int rotary_dim, void* stream) {
+  if (!c || !qkv_bf16 || !out_bf16 || !kv_bf16 || !block_table || !ctx_len)
+    return fail(c, "ccb_op_attention_decode: null argument");
+  if (layers <= 0 || layer < 0 || layer >= layers) return fail(c, "ccb_op_attention_decode: layer %d outside [0, %d)", layer, layers);
+  if (page_tokens <= 0 || num_pages <= 0 || max_pages_per_row <= 0)
+    return fail(c, "ccb_op_attention_decode: page_tokens=%d, num_pages=%d, max_pages_per_row=%d must be positive", page_tokens,
+                num_pages, max_pages_per_row);
+  if (hd != 64 && hd != 128 && hd != 256) return fail(c, "ccb_op_attention_decode: head_dim %d unsupported (64/128/256)", hd);
+  if (rows < 0 || H <= 0) return fail(c, "ccb_op_attention_decode: rows=%d, H=%d", rows, H);
+  DeviceGuard dev_guard(c->device);
+  KvCache kv;
+  kv.base = static_cast<bf16*>(kv_bf16);
+  kv.L = layers;
+  kv.H = H;
+  kv.hd = hd;
+  kv.page_tokens = page_tokens;
+  kv.num_pages = num_pages;
+  kv.max_pages_per_row = max_pages_per_row;
+  RUN(attention_decode(static_cast<const bf16*>(qkv_bf16), static_cast<bf16*>(out_bf16), ldo, rows, H, hd, scale, &kv, layer,
+                       block_table, ctx_len, rotary_dim, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 

@@ -538,3 +538,36 @@ class Engine:
                                               scale if scale is not None else hd ** -0.5, 1 if causal else 0, rotary_dim,
                                               self._stream()))
         return out
+
+    def op_attention_decode(self, qkv, kv, layer, page_tokens, block_table, ctx_len, H, hd, rotary_dim=0, scale=None,
+                            ldo=None):
+        """One decode step over a paged KV cache (ccb_op_attention_decode): qkv [rows, 3*H*hd] bf16 (the new tokens),
+        kv [layers, 2, num_pages, H, page_tokens, hd] bf16 (the new k / v are written into it), block_table
+        [rows, max_pages_per_row] int32, ctx_len [rows] int32.  Returns out [rows, ldo] bf16 (ldo defaults to H*hd); the
+        columns past H*hd are left as allocated."""
+        if kv.dtype != torch.bfloat16 or not kv.is_contiguous() or kv.dim() != 6 or tuple(kv.shape[3:]) != (H, page_tokens, hd):
+            raise ValueError("kv must be a contiguous bf16 [layers, 2, num_pages, %d, %d, %d] tensor" % (H, page_tokens, hd))
+        qkv = self._dev(qkv, torch.bfloat16)
+        bt = self._dev(block_table, torch.int32)
+        cl = self._dev(ctx_len, torch.int32)
+        rows = qkv.shape[0]
+        ldo = ldo or H * hd
+        out = torch.zeros(rows, ldo, device=self.device, dtype=torch.bfloat16)
+        self._check(self.lib.ccb_op_attention_decode(self._h, _ptr(qkv), _ptr(out), ldo, rows, H, hd,
+                                                     scale if scale is not None else hd ** -0.5, _ptr(kv), kv.shape[0], layer,
+                                                     kv.shape[2], page_tokens, bt.shape[1], _ptr(bt), _ptr(cl), rotary_dim,
+                                                     self._stream()))
+        self._keep = [qkv, bt, cl]
+        return out
+
+    def debug_kv_layout(self):
+        """(layers, heads, head_dim, page_tokens, num_pages, max_pages_per_row) of the last generate call's KV pool."""
+        out = (C.c_int64 * 6)()
+        self._check(self.lib.ccb_debug_kv_layout(self._h, out))
+        return tuple(int(v) for v in out)
+
+    def debug_copy_buffer(self, which: int, numel: int, dtype) -> torch.Tensor:
+        """The first `numel` elements of internal buffer `which` (ccb_debug_copy_buffer), copied on the current stream."""
+        out = torch.empty(numel, dtype=dtype, device=self.device)
+        self._check(self.lib.ccb_debug_copy_buffer(self._h, which, _ptr(out), out.numel() * out.element_size(), self._stream()))
+        return out

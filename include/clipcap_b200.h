@@ -211,16 +211,37 @@ CCB_API int ccb_debug_mega_trace(ccb_ctx* ctx, void* trace_u64);
  * the environment); any other value (default) uses the persistent kernel.  Returns 1 when the persistent kernel covers
  * this model shape, else 0. */
 CCB_API int ccb_debug_set_mega(ccb_ctx* ctx, int enable);
-/* test aid: copies the first `bytes` of an internal activation workspace to `dst` (device memory) on `stream`:
+/* test aid: copies the first `bytes` of an internal buffer to `dst` (device memory) on `stream`:
  * 0 residual stream h (f32), 1 LayerNorm output x (bf16), 2 attention output (bf16), 3 MLP hidden (bf16),
- * 4 logits (f32, row pitch = vocab rounded up to 64), 5 fused qkv (bf16; operator-per-kernel decode only). */
+ * 4 logits (f32, row pitch = vocab rounded up to 64), 5 fused qkv (bf16; operator-per-kernel decode only),
+ * 6 KV pool (bf16 [layers][2][num_pages][heads][page_tokens][head_dim], geometry of ccb_debug_kv_layout),
+ * 7 block table (int32 [max_images * max_beam][max_pages_per_row]).  For 6 and 7 more bytes than the buffer holds is an
+ * error. */
 CCB_API int ccb_debug_copy_buffer(ccb_ctx* ctx, int which, void* dst, int64_t bytes, void* stream);
+/* test aid: the KV pool geometry of the last ccb_generate / ccb_caption_images call: out = {layers, heads, head_dim,
+ * page_tokens, num_pages, max_pages_per_row}.  An error before the first such call. */
+CCB_API int ccb_debug_kv_layout(ccb_ctx* ctx, int64_t out[6]);
 /* y = LayerNorm(x) over the last dim: x f32 [rows, d] -> y bf16 [rows, d] */
 CCB_API int ccb_op_layernorm(ccb_ctx* ctx, const float* x, const float* gamma, const float* beta, float eps, void* y_bf16,
                      int rows, int d, void* stream);
 /* softmax(q k^T * scale [causal]) v for a fused qkv buffer [B*S, 3*H*hd] bf16 -> out [B*S, H*hd] bf16 */
 CCB_API int ccb_op_attention(ccb_ctx* ctx, const void* qkv_bf16, void* out_bf16, int B, int S, int H, int hd, float scale,
                      int causal, int rotary_dim, void* stream);
+/* One decode step of attention over a paged KV cache in caller memory, on the kernels the operator-per-kernel decode
+ * chain runs (head_dim 64 / 128: one warp per (row, head); 256: one CTA per (row, head)).  qkv [rows, 3*H*hd] holds each
+ * row's new token; row r attends over positions [0, ctx_len[r]] with the token at ctx_len[r] being the new one: its k
+ * (GPT-J rotary at position ctx_len[r] on the first rotary_dim dims, as on q; 0 = none) and v are first stored into the
+ * cache.  out row r starts at r * ldo (ldo >= H*hd, even).
+ * kv [layers][2][num_pages][H][page_tokens][hd] (k then v); block_table [rows, max_pages_per_row]: position t of row r is
+ * slot t % page_tokens of page block_table[r][t / page_tokens].  The caller keeps the contract the engine keeps:
+ *   - every ctx_len[r] < max_pages_per_row (the engine's block table is sized for token-granular pages, and the kernels
+ *     size their per-row score buffer and K/V tile from max_pages_per_row);
+ *   - every page id that positions [0, ctx_len[r]] of row r use lies in [0, num_pages).
+ * Null pointers, `layer` outside [0, layers), non-positive page geometry and an unsupported head_dim are rejected. */
+CCB_API int ccb_op_attention_decode(ccb_ctx* ctx, const void* qkv_bf16, void* out_bf16, int64_t ldo, int rows, int H, int hd,
+                                    float scale, void* kv_bf16, int layers, int layer, int num_pages, int page_tokens,
+                                    int max_pages_per_row, const int32_t* block_table, const int32_t* ctx_len, int rotary_dim,
+                                    void* stream);
 
 #ifdef __cplusplus
 }
