@@ -65,6 +65,7 @@ PROTOTYPES = {
     "ccb_cross_entropy": (_I, [_P, _P, _L, _I, _I, _P, _P, _I, _P, _P, _P]),
     "ccb_beam_step": (_I, [_P, _P, _L, _I, _I, _I, _F, _I, _I, _P, _P, _P, _P, _I, _P, _P, _P]),
     "ccb_op_linear": (_I, [_P, _P, _L, _I, _P, _I, _I, _P, _I, _P, _L, _P, _L, _I, _I, _I, _I, _P]),
+    "ccb_op_linear_ex": (_I, [_P, _P, _L, _I, _P, _L, _I, _I, _P, _I, _P, _L, _P, _L, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ccb_debug_gemm_trace": (_I, [_P, _P, _L, _I]),
     "ccb_debug_mega_trace": (_I, [_P, _P]),
     "ccb_debug_set_mega": (_I, [_P, _I]),

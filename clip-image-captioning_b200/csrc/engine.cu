@@ -1362,6 +1362,13 @@ int ccb_beam_step(ccb_ctx* c, const float* logits, int64_t ld, int N, int beam, 
 int ccb_op_linear(ccb_ctx* c, const void* x, int64_t lda, int tokens, const void* w, int features, int K,
                   const float* bias, int act, const float* residual, int64_t ldr, void* out, int64_t ldo, int out_bf16,
                   int orientation, int bn, int split_k, void* stream) {
+  return ccb_op_linear_ex(c, x, lda, tokens, w, 0, features, K, bias, act, residual, ldr, out, ldo, out_bf16, 0, 0, 0,
+                          orientation, bn, split_k, stream);
+}
+
+int ccb_op_linear_ex(ccb_ctx* c, const void* x, int64_t lda, int tokens, const void* w, int64_t ldw, int features, int K,
+                     const float* bias, int act, const float* residual, int64_t ldr, void* out, int64_t ldo, int out_bf16,
+                     int rg_in, int rg_out, int rg_off, int orientation, int bn, int split_k, void* stream) {
   if (!c || !x || !w || !out) return fail(c, "ccb_op_linear: null argument");
   DeviceGuard dev_guard(c->device);
   GemmArgs g;
@@ -1369,6 +1376,10 @@ int ccb_op_linear(ccb_ctx* c, const void* x, int64_t lda, int tokens, const void
   g.lda = lda;
   g.tokens = tokens;
   g.weight = static_cast<const bf16*>(w);
+  g.ldw = ldw;
+  g.rg_in = rg_in;
+  g.rg_out = rg_out;
+  g.rg_off = rg_off;
   g.features = features;
   g.K = K;
   g.bias = bias;

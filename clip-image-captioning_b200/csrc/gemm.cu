@@ -238,6 +238,23 @@ int gemm_launch(const GemmArgs& a, const GemmWorkspace& w, cudaStream_t stream) 
   if (!g_encode) return fail("gemm_init() was not called");
   if (a.K <= 0 || a.K % 64 != 0) return fail("GEMM K must be a positive multiple of 64");
   if (a.tokens <= 0 || a.features <= 0) return fail("GEMM with empty extent");
+  // the epilogue knows activations 0..7 only (GEGLU is a separate kernel on the GEMM's output); an unknown code would
+  // silently run as the identity
+  if (a.act_fn < ACT_NONE || a.act_fn > ACT_TANH) {
+    snprintf(g_err, sizeof(g_err), "GEMM activation %d is not an epilogue activation (0..7)", a.act_fn);
+    return -1;
+  }
+  // pitches shorter than a row would make rows overlap: a tile would read its neighbour's K range or two rows would be
+  // written to the same elements.  A remap must keep the groups' rows apart: rg_off + rg_in <= rg_out.
+  if (a.lda < a.K || (a.ldw != 0 && a.ldw < a.K) || a.ldo < a.features || (a.residual && a.ldr < a.features) ||
+      ((a.rg_in | a.rg_out | a.rg_off) != 0 && (a.rg_in <= 0 || a.rg_off < 0 || a.rg_off + a.rg_in > a.rg_out))) {
+    snprintf(g_err, sizeof(g_err),
+             "GEMM pitches out of range: K=%d features=%d lda=%lld ldw=%lld ldo=%lld ldr=%lld, remap rg_in=%d rg_out=%d "
+             "rg_off=%d (need lda >= K, ldw 0 or >= K, ldo >= features, ldr >= features with a residual, and for a remap "
+             "rg_in > 0, rg_off >= 0, rg_off + rg_in <= rg_out)",
+             a.K, a.features, a.lda, a.ldw, a.ldo, a.ldr, a.rg_in, a.rg_out, a.rg_off);
+    return -1;
+  }
 
   // force_orientation: 0 auto, 1 normal, 2 swapped, 3 normal + CTA-pair persistent kernel, 4 normal + single-CTA persistent
   const bool swapped = a.force_orientation ? (a.force_orientation == 2) : (a.tokens <= 256);

@@ -507,20 +507,50 @@ class Engine:
         return nxt, src
 
     # ------------------------------------------------------------------------------------------ single ops
+    def _rows(self, t, dtype, tma):
+        """t as a [rows, cols] GEMM operand on this device.  A view with unit column stride is passed as it is, its
+        stride(0) becoming the row pitch, when the kernels can address it (16-byte aligned base; for operands read through
+        a tensor map (`tma`) also a pitch of whole 16 bytes); anything else is copied contiguous."""
+        if (t.device == self.device and t.dtype == dtype and t.dim() == 2 and t.stride(1) == 1 and
+                t.stride(0) >= t.shape[1] and t.data_ptr() % 16 == 0 and
+                (not tma or t.stride(0) * t.element_size() % 16 == 0)):
+            return t
+        return self._dev(t, dtype)
+
     def op_linear(self, x, w, bias=None, act="none", residual=None, out_dtype=torch.float32, orientation=0, bn=0,
-                  split_k=0):
-        """act(x @ w.T + bias) + residual with x [tokens, K] bf16, w [features, K] bf16 (tcgen05 GEMM)."""
-        x = self._dev(x, torch.bfloat16)
-        w = self._dev(w, torch.bfloat16)
+                  split_k=0, *, out=None, residual_is_out=False, row_remap=None):
+        """act(x @ w.T + bias) + residual with x [tokens, K] bf16, w [features, K] bf16 (tcgen05 GEMM,
+        ccb_op_linear_ex).  x, w and residual may be row-strided views: their row pitches go to the kernel.
+
+        out: a caller-owned [rows, features] f32 or bf16 view (row pitch stride(0), any offset) written in place and
+        returned; by default a new [tokens, features] tensor of out_dtype.  residual_is_out: the residual is read from
+        `out` itself (f32), as the engine's residual stream does.  row_remap (rg_in, rg_out, rg_off): token row t lands in
+        out row (t // rg_in) * rg_out + rg_off + t % rg_in (normal orientation only)."""
+        x = self._rows(x, torch.bfloat16, True)
+        w = self._rows(w, torch.bfloat16, True)
         tokens, K = x.shape
         features = w.shape[0]
+        rg_in, rg_out, rg_off = row_remap or (0, 0, 0)
         bias = self._dev(bias, torch.float32) if bias is not None else None
-        residual = self._dev(residual, torch.float32) if residual is not None else None
-        out = torch.empty(tokens, features, device=self.device, dtype=out_dtype)
-        self._check(self.lib.ccb_op_linear(self._h, _ptr(x), x.stride(0), tokens, _ptr(w), features, K, _ptr(bias),
-                                           _lib.ACT[act], _ptr(residual), residual.stride(0) if residual is not None else 0,
-                                           _ptr(out), out.stride(0), 1 if out_dtype == torch.bfloat16 else 0, orientation,
-                                           bn, split_k, self._stream()))
+        if residual_is_out and (out is None or residual is not None or out.dtype != torch.float32):
+            raise ValueError("residual_is_out needs an f32 `out` and no separate residual")
+        if out is None:
+            out = torch.empty(tokens, features, device=self.device, dtype=out_dtype)
+        elif (out.device != self.device or out.dtype not in (torch.float32, torch.bfloat16) or out.dim() != 2 or
+              out.stride(1) != 1 or out.shape[1] != features):
+            raise ValueError("out must be a [rows, %d] f32 or bf16 view on %s with unit column stride" % (features, self.device))
+        last = tokens - 1 if not rg_in else (tokens - 1) // rg_in * rg_out + rg_off + (tokens - 1) % rg_in
+        if out.shape[0] <= last:
+            raise ValueError("out has %d rows; token row %d lands in row %d" % (out.shape[0], tokens - 1, last))
+        if residual_is_out:
+            residual = out
+        elif residual is not None:
+            residual = self._rows(residual, torch.float32, False)
+        self._check(self.lib.ccb_op_linear_ex(self._h, _ptr(x), x.stride(0), tokens, _ptr(w), w.stride(0), features, K,
+                                              _ptr(bias), _lib.ACT[act], _ptr(residual),
+                                              residual.stride(0) if residual is not None else 0, _ptr(out), out.stride(0),
+                                              1 if out.dtype == torch.bfloat16 else 0, rg_in, rg_out, rg_off, orientation,
+                                              bn, split_k, self._stream()))
         return out
 
     def op_layernorm(self, x, gamma, beta, eps=1e-5):

@@ -198,7 +198,24 @@ CCB_API int ccb_beam_step(ccb_ctx* ctx, const float* logits, int64_t ld, int N, 
 CCB_API int ccb_op_linear(ccb_ctx* ctx, const void* x, int64_t lda, int tokens, const void* w, int features, int K,
                   const float* bias, int act, const float* residual, int64_t ldr, void* out, int64_t ldo,
                   int out_bf16, int orientation, int bn, int split_k, void* stream);
-/* tuning aid: when non-NULL, GEMM launch n of this context writes 8 globaltimer stamps per CTA to
+/* ccb_op_linear with the addressing the engine's own GEMMs use (ccb_op_linear is this call with ldw = 0 and no remap):
+ *   out[r(t), f] = act(sum_k x[t * lda + k] * w[f * ldw + k] + bias[f]) + residual[r(t) * ldr + f]
+ *   r(t) = (t / rg_in) * rg_out + rg_off + t % rg_in   (identity when rg_in = rg_out = rg_off = 0)
+ * out element (row r, column f) is at out + r * ldo + f.  ldw is the weight row pitch in elements (0: K), so w may be a
+ * column range of a wider matrix.  residual may equal out (read before the element is written: an in-place residual
+ * stream); no other overlap of out with x, w, bias or residual is allowed.  The row remap lays groups of rg_in token
+ * rows into groups of rg_out output rows at offset rg_off (the all-features mapper's visual tokens inside each
+ * sequence); it exists only in the normal orientation (orientation 1, 3 or 4, or 0 with tokens > 256).
+ * Rejected with a message, nothing launched: act outside 0..7 (CCB_ACT_GEGLU is not an epilogue), K not a positive
+ * multiple of 64, lda < K, ldw != 0 and ldw < K, ldo < features, a residual with ldr < features, a remap with
+ * rg_in <= 0, rg_off < 0 or rg_off + rg_in > rg_out, x / w not 16-byte aligned or their row pitches not multiples of
+ * 8 elements, and in the normal orientation out / residual / bias not 16-byte aligned.  The caller owns the extents:
+ * x holds `tokens` rows, w `features` rows, out and residual every row r(t) for t < tokens. */
+CCB_API int ccb_op_linear_ex(ccb_ctx* ctx, const void* x, int64_t lda, int tokens, const void* w, int64_t ldw, int features,
+                  int K, const float* bias, int act, const float* residual, int64_t ldr, void* out, int64_t ldo,
+                  int out_bf16, int rg_in, int rg_out, int rg_off, int orientation, int bn, int split_k, void* stream);
+/* tuning aid, inert unless the library was built with -DCCB_TUNING (`python tools/build.py --tuning`): when non-NULL,
+ * one-tile GEMM launch n of this context writes 8 globaltimer stamps per CTA to
  * trace[(n % launches) * stride_u64 + cta * 8 + k] (entry, setup, first tile landed, MMAs issued, accumulator ready,
  * cluster reduction reached, epilogue done, exit).  NULL (the default) disables it. */
 CCB_API int ccb_debug_gemm_trace(ccb_ctx* ctx, void* trace_u64, int64_t stride_u64, int launches);
