@@ -593,6 +593,45 @@ std::string graph_key(const ccb_gen_params* p, int N, int rows, int T, int c_meg
   return buf;
 }
 
+// the graph cached under `key`, captured from what body() enqueues on s when it is not cached yet; null after a failure
+template <class Body>
+const GraphEntry* captured_graph(ccb_ctx* c, const std::string& key, cudaStream_t s, Body body) {
+  auto it = c->graphs.find(key);
+  if (it != c->graphs.end()) return &it->second;
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
+  if (e != cudaSuccess) {
+    fail(c, "cudaStreamBeginCapture: %s", cudaGetErrorString(e));
+    return nullptr;
+  }
+  c->capturing = true;
+  c->capture_launches = 0;
+  const int r = body();
+  c->capturing = false;
+  e = cudaStreamEndCapture(s, &graph);
+  if (r != 0) {
+    if (graph) cudaGraphDestroy(graph);
+    return nullptr;
+  }
+  if (e != cudaSuccess) {
+    fail(c, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
+    return nullptr;
+  }
+  GraphEntry ge;
+  ge.nodes = c->capture_launches;
+  e = cudaGraphInstantiate(&ge.exec, graph, 0);
+  cudaGraphDestroy(graph);
+  if (e != cudaSuccess) {
+    fail(c, "cudaGraphInstantiate: %s", cudaGetErrorString(e));
+    return nullptr;
+  }
+  if (c->graphs.size() >= 32) {  // bound the cache
+    for (auto& kvp : c->graphs) cudaGraphExecDestroy(kvp.second.exec);
+    c->graphs.clear();
+  }
+  return &c->graphs.emplace(key, ge).first->second;
+}
+
 int generate_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const float* embeds, int N, int S0,
                             int32_t* tokens_out, int32_t* lengths_out, float* scores_out) {
   const ccb_model_desc& D = c->desc;
@@ -639,35 +678,12 @@ int generate_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const float* em
 
   // ---- decode: T-1 replays of one captured step (every kernel reads step / ctx_len from device memory)
   if (T > 1) {
-    const std::string key = graph_key(p, N, rows, T, c->mega.enabled ? 1 : 0);
-    auto it = c->graphs.find(key);
-    if (it == c->graphs.end()) {
-      cudaGraph_t graph = nullptr;
-      CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      c->capturing = true;
-      c->capture_launches = 0;
-      const int r = decode_iteration(c, p, N, rows, T, s);
-      c->capturing = false;
-      const cudaError_t e = cudaStreamEndCapture(s, &graph);
-      if (r != 0) {
-        if (graph) cudaGraphDestroy(graph);
-        return -1;
-      }
-      if (e != cudaSuccess) return fail(c, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
-      GraphEntry ge;
-      ge.nodes = c->capture_launches;
-      const cudaError_t e2 = cudaGraphInstantiate(&ge.exec, graph, 0);
-      cudaGraphDestroy(graph);
-      if (e2 != cudaSuccess) return fail(c, "cudaGraphInstantiate: %s", cudaGetErrorString(e2));
-      if (c->graphs.size() >= 32) {  // bound the cache
-        for (auto& kvp : c->graphs) cudaGraphExecDestroy(kvp.second.exec);
-        c->graphs.clear();
-      }
-      it = c->graphs.emplace(key, ge).first;
-    }
+    const GraphEntry* ge = captured_graph(c, graph_key(p, N, rows, T, c->mega.enabled ? 1 : 0), s,
+                                          [&]() { return decode_iteration(c, p, N, rows, T, s); });
+    if (!ge) return -1;
     for (int t = 1; t < T; ++t) {
-      CUDA_OK(cudaGraphLaunch(it->second.exec, s));
-      c->launches += it->second.nodes;
+      CUDA_OK(cudaGraphLaunch(ge->exec, s));
+      c->launches += ge->nodes;
     }
   }
   CUDA_OK(cudaEventRecord(c->ev_t2[slot], s));
@@ -682,6 +698,235 @@ int generate_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const float* em
   } else if (lengths_out) {
     CUDA_OK(cudaMemcpyAsync(lengths_out, c->lengths, sizeof(int) * rows, cudaMemcpyDeviceToDevice, s));
   }
+  return 0;
+}
+
+// why images cannot be captioned with this context and this append_bos, or null
+const char* image_path_unsupported(ccb_ctx* c, int append_bos) {
+  const ccb_model_desc& D = c->desc;
+  if (!D.vit_present) return "context was created without an image encoder";
+  if (D.map_kind == CCB_MAP_NONE) return "context was created without a prefix mapper";
+  if (D.map_kind == CCB_MAP_TRANSFORMER_ALL && D.map_clip_len != (D.vit_image / D.vit_patch) * (D.vit_image / D.vit_patch) + 1)
+    return "map_clip_len does not match the ViT's token count";
+  if (append_bos >= D.lm_vocab) return "BOS id outside the vocabulary";
+  return nullptr;
+}
+
+// ViT + mapper of B images (+ the BOS embedding appended when append_bos >= 0, evaluate_model.py:124-133) -> c->prefix
+// [B, map_prefix_len + (append_bos >= 0), lm_d]
+int image_prefix(ccb_ctx* c, const void* images, int dtype, int B, int append_bos, cudaStream_t s) {
+  const int P = c->desc.map_prefix_len, d = c->desc.lm_d;
+  const int extra = append_bos >= 0 ? 1 : 0;
+  if (vit_forward(c, images, dtype, B, c->feat, s, c->desc.map_kind == CCB_MAP_TRANSFORMER_ALL)) return -1;
+  if (map_forward(c, c->feat, B, c->prefix, P + extra, s)) return -1;
+  if (extra) {
+    token_rows_kernel<<<B, 256, 0, s>>>(c->wte, append_bos, c->prefix, static_cast<long long>(P + extra) * d, P, d);
+    RUN(launch_check());
+  }
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------ continuous batching
+// Decode iterations per round of ccb_caption_dataset: one replay of a captured graph, then one host read of the slots'
+// state.  A slot that finishes waits 1.5 rounds on average for its refill (the rest of its round, then the round already
+// enqueued while the host reads), so a round trades that idle decode work against refills of fewer images each.  On GPT2-XL
+// with 64 slots (DESIGN.md §6b) a refill costs about 5-6 ms, and 4 steps per round gave 697 captions/s against 625 for 2.
+constexpr int kRoundSteps = 4;
+
+// every slot empty (finished, no image) at position S0 of its own pages [r * ppr, (r+1) * ppr); the outputs' pointers
+__global__ void cont_init_kernel(int* block_table, int max_pages, int rows, int pages_per_row, int S0, int* ctx_len,
+                                 int* row_step, int* slot_image, int* next_tokens, int* lengths, int* stops,
+                                 uint8_t* finished, int** cont_out, int* tokens_out, int* lengths_out) {
+  const int tid = blockIdx.x * blockDim.x + threadIdx.x;
+  const int nth = gridDim.x * blockDim.x;
+  for (int i = tid; i < rows * pages_per_row; i += nth)
+    block_table[static_cast<long long>(i / pages_per_row) * max_pages + i % pages_per_row] = i;
+  for (int r = tid; r < rows; r += nth) {
+    ctx_len[r] = S0;
+    row_step[r] = 0;
+    slot_image[r] = -1;
+    next_tokens[r] = 0;
+    lengths[r] = 0;
+    stops[r] = 0;
+    finished[r] = 1;
+  }
+  if (tid == 0) {
+    cont_out[0] = tokens_out;
+    cont_out[1] = lengths_out;
+  }
+}
+
+// prefill row i of a refill chunk -> slot slots[i], image img0 + i: its pages in the prefill block table, its state reset
+__global__ void cont_refill_kernel(const int* __restrict__ slots, int k, int img0, long long first_row_id, int max_pages,
+                                   int pages_per_row, int S0, int* block_table_prefill, int* ctx_len, int* row_step,
+                                   int* slot_image, long long* slot_ids, long long* refill_ids, int* lengths, int* stops,
+                                   uint8_t* finished) {
+  for (int i = threadIdx.x; i < k * pages_per_row; i += blockDim.x) {
+    const int b = i / pages_per_row, j = i % pages_per_row;
+    block_table_prefill[static_cast<long long>(b) * max_pages + j] = slots[b] * pages_per_row + j;
+  }
+  for (int i = threadIdx.x; i < k; i += blockDim.x) {
+    const int r = slots[i];
+    ctx_len[r] = S0;
+    row_step[r] = 0;
+    slot_image[r] = img0 + i;
+    slot_ids[r] = refill_ids[i] = first_row_id + img0 + i;
+    lengths[r] = 0;
+    stops[r] = 0;
+    finished[r] = 0;
+  }
+}
+
+RowAdvance row_advance(ccb_ctx* c, const int* slots, int* next_tokens) {
+  RowAdvance ra;
+  ra.row_step = c->row_step;
+  ra.row_image = c->slot_image;
+  ra.slots = slots;
+  ra.next_tokens = next_tokens;
+  ra.out = c->cont_out;
+  return ra;
+}
+
+// one decode iteration over all slots: the step, token selection keyed by (seed, image id, row step), per-row advance
+int cont_iteration(ccb_ctx* c, const ccb_gen_params* p, int rows, int T, cudaStream_t s) {
+  if (lm_decode_step(c, rows, s)) return -1;
+  if (p->mode == CCB_GEN_GREEDY) {
+    RUN(sample_greedy(c->logits, c->ldv, rows, c->desc.lm_vocab, c->next_tokens, s));
+  } else {
+    SampleParams sp = sample_params(c, p, rows);
+    sp.history = c->gen_tokens;
+    sp.ld_hist = T;
+    sp.row_ids = c->slot_ids;
+    sp.row_step = c->row_step;
+    RUN(sample_top_p(c->logits, c->ldv, rows, c->desc.lm_vocab, sp, c->next_tokens, s));
+  }
+  const RowAdvance ra = row_advance(c, nullptr, nullptr);
+  RUN(advance_rows(c->next_tokens, rows, c->gen_tokens, T, c->lengths, c->stops, c->finished, c->ctx_len, nullptr,
+                   p->stop_token, p->max_stops, p->eos_token, s, &ra));
+  return 0;
+}
+
+// k consecutive images from img0 into slots c->refill_slots[off, off + k): prefix, prefill into the slots' pages, first token
+int cont_refill(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int append_bos, long long first_row_id,
+                int off, int k, int img0, int S0, int T, int pages_per_row, cudaStream_t s) {
+  const ccb_model_desc& D = c->desc;
+  const size_t image_bytes = static_cast<size_t>(3) * D.vit_image * D.vit_image * (dtype == CCB_DTYPE_F32 ? 4 : 2);
+  if (image_prefix(c, static_cast<const char*>(images) + image_bytes * img0, dtype, k, append_bos, s)) return -1;
+  cont_refill_kernel<<<1, 256, 0, s>>>(c->refill_slots + off, k, img0, first_row_id, c->max_pages_per_row, pages_per_row, S0,
+                                       c->block_table_prefill, c->ctx_len, c->row_step, c->slot_image, c->slot_ids,
+                                       c->refill_ids, c->lengths, c->stops, c->finished);
+  RUN(launch_check());
+  if (lm_prefill_layers(c, c->prefix, k, S0, nullptr, true, s)) return -1;
+  if (lm_logits(c, k, S0, 1, c->logits, c->ldv, s)) return -1;
+  if (p->mode == CCB_GEN_GREEDY) {
+    RUN(sample_greedy(c->logits, c->ldv, k, D.lm_vocab, c->refill_next, s));
+  } else {
+    SampleParams sp = sample_params(c, p, k);   // step 0: no history yet
+    sp.row_ids = c->refill_ids;
+    RUN(sample_top_p(c->logits, c->ldv, k, D.lm_vocab, sp, c->refill_next, s));
+  }
+  const RowAdvance ra = row_advance(c, c->refill_slots + off, c->next_tokens);
+  RUN(advance_rows(c->refill_next, k, c->gen_tokens, T, c->lengths, c->stops, c->finished, nullptr, nullptr, p->stop_token,
+                   p->max_stops, p->eos_token, s, &ra));
+  return 0;
+}
+
+int caption_dataset_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int n, int rows,
+                                   int append_bos, long long first_row_id, int32_t* tokens_out, int32_t* lengths_out,
+                                   int64_t* steps_out) {
+  const ccb_model_desc& D = c->desc;
+  cudaStream_t s = c->work;
+  const int T = p->max_new_tokens;
+  const int S0 = D.map_prefix_len + (append_bos >= 0 ? 1 : 0);
+  if (p->mode == CCB_GEN_BEAM) return fail(c, "ccb_caption_dataset: beam search is not supported (ccb_caption_images has it)");
+  if (p->mode != CCB_GEN_GREEDY && p->mode != CCB_GEN_SAMPLE) return fail(c, "ccb_caption_dataset: unknown mode %d", p->mode);
+  if (p->q_noise) return fail(c, "ccb_caption_dataset: q_noise is not supported (its [step, row] layout has no meaning here)");
+  if (p->row_ids || p->top_p_rows || p->top_k_rows || p->typ_p_rows)
+    return fail(c, "ccb_caption_dataset: per-row arrays (row_ids, top_p_rows, top_k_rows, typ_p_rows) are not supported; "
+                   "image ids are first_row_id + image index");
+  if (dtype != CCB_DTYPE_F32 && dtype != CCB_DTYPE_F16 && dtype != CCB_DTYPE_BF16)
+    return fail(c, "ccb_caption_dataset: unknown image dtype %d", dtype);
+  if (n <= 0) return fail(c, "ccb_caption_dataset: n_images=%d must be positive", n);
+  if (rows < 1 || rows > c->max_rows)
+    return fail(c, "ccb_caption_dataset: rows=%d outside [1, max_images * max_beam = %d]", rows, c->max_rows);
+  if (T <= 0 || S0 + T > D.max_ctx)
+    return fail(c, "ccb_caption_dataset: S0=%d + max_new_tokens=%d exceeds max_ctx=%d", S0, T, D.max_ctx);
+  if (S0 > D.max_lm_tokens) return fail(c, "ccb_caption_dataset: S0=%d exceeds max_lm_tokens=%d", S0, D.max_lm_tokens);
+  if (const char* why = image_path_unsupported(c, append_bos)) return fail(c, "ccb_caption_dataset: %s", why);
+  if (const char* why = attention_prefill_unsupported(S0, D.lm_d / D.lm_heads, 1, true, D.lm_rotary_dim, false))
+    return fail(c, "ccb_caption_dataset: prefix of S0=%d tokens with head_dim %d: %s", S0, D.lm_d / D.lm_heads, why);
+  const int page_tokens = D.page_tokens;
+  const int pages_per_row = (S0 + T + page_tokens - 1) / page_tokens;
+  if (static_cast<long long>(rows) * pages_per_row * page_tokens > c->kv_pool_tokens)
+    return fail(c, "ccb_caption_dataset: KV pool too small");
+  c->kv.page_tokens = page_tokens;
+  c->kv.num_pages = static_cast<int>(c->kv_pool_tokens / page_tokens);
+  c->kv.max_pages_per_row = c->max_pages_per_row;
+
+  CUDA_OK(cudaMemsetAsync(tokens_out, 0, sizeof(int32_t) * static_cast<size_t>(n) * T, s));
+  CUDA_OK(cudaMemsetAsync(lengths_out, 0, sizeof(int32_t) * static_cast<size_t>(n), s));
+  cont_init_kernel<<<148, 256, 0, s>>>(c->block_table, c->max_pages_per_row, rows, pages_per_row, S0, c->ctx_len, c->row_step,
+                                       c->slot_image, c->next_tokens, c->lengths, c->stops, c->finished, c->cont_out,
+                                       tokens_out, lengths_out);
+  RUN(launch_check());
+  const GraphEntry* ge = captured_graph(c, "cont" + std::to_string(kRoundSteps) + " " + graph_key(p, 0, rows, T, c->mega.enabled ? 1 : 0),
+                                        s, [&]() {
+                                          for (int i = 0; i < kRoundSteps; ++i)
+                                            if (cont_iteration(c, p, rows, T, s)) return -1;
+                                          return 0;
+                                        });
+  if (!ge) return -1;
+
+  // The host keeps one round ahead: it reads round j's slot state while round j + 1 runs, and refills the slots that had
+  // finished by round j at the boundary after round j + 1.  A finished slot is frozen, so nothing it holds changes in
+  // between; a slot shows as free when its snapshot is finished with the image the host last gave it.
+  const int chunk = std::min(D.max_images, D.max_lm_tokens / S0);
+  std::vector<int> occupant(rows, -1);   // image the host gave each slot, -1 = free
+  int next_image = 0;
+  auto refill = [&](int boundary) -> int {
+    int* list = c->h_refill + (boundary % 2) * c->max_rows;
+    int m = 0;
+    for (int r = 0; r < rows && next_image + m < n; ++r)
+      if (occupant[r] < 0) list[m++] = r;
+    if (m == 0) return 0;
+    CUDA_OK(cudaMemcpyAsync(c->refill_slots, list, sizeof(int) * m, cudaMemcpyHostToDevice, s));
+    for (int off = 0; off < m; off += chunk)
+      if (cont_refill(c, p, images, dtype, append_bos, first_row_id, off, std::min(chunk, m - off), next_image + off, S0, T,
+                      pages_per_row, s))
+        return -1;
+    for (int i = 0; i < m; ++i) occupant[list[i]] = next_image + i;
+    next_image += m;
+    return 0;
+  };
+  auto round = [&](int j) -> int {
+    CUDA_OK(cudaGraphLaunch(ge->exec, s));
+    c->launches += ge->nodes;
+    CUDA_OK(cudaMemcpyAsync(c->h_finished + (j % 2) * c->max_rows, c->finished, rows, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaMemcpyAsync(c->h_slot_image + (j % 2) * c->max_rows, c->slot_image, sizeof(int) * rows, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaEventRecord(c->ev_round[j % 2], s));
+    return 0;
+  };
+  if (refill(0) || round(0) || round(1)) return -1;
+  long long rounds = 2;
+  for (int j = 0;; ++j) {
+    CUDA_OK(cudaEventSynchronize(c->ev_round[j % 2]));
+    const uint8_t* fin = c->h_finished + (j % 2) * c->max_rows;
+    const int* img = c->h_slot_image + (j % 2) * c->max_rows;
+    bool busy = false;
+    for (int r = 0; r < rows; ++r) {
+      if (occupant[r] < 0) continue;
+      if (fin[r] && img[r] == occupant[r]) occupant[r] = -1;
+      else busy = true;
+    }
+    if (!busy && next_image == n) {
+      // round j + 1 is still running: the pinned ring is free for the next call once it has read its last refill list
+      CUDA_OK(cudaEventSynchronize(c->ev_round[(j + 1) % 2]));
+      break;
+    }
+    if (refill(j + 1) || round(j + 2)) return -1;
+    ++rounds;
+  }
+  *steps_out = rounds * kRoundSteps;
   return 0;
 }
 
@@ -734,8 +979,9 @@ void ccb_destroy(ccb_ctx* c) {
   cudaDeviceSynchronize();
   for (auto& kvp : c->graphs) cudaGraphExecDestroy(kvp.second.exec);
   for (void* p : c->allocs) cudaFree(p);
+  if (c->host_pinned) cudaFreeHost(c->host_pinned);
   if (c->work) cudaStreamDestroy(c->work);
-  for (cudaEvent_t e : {c->ev_in, c->ev_out})
+  for (cudaEvent_t e : {c->ev_in, c->ev_out, c->ev_round[0], c->ev_round[1]})
     if (e) cudaEventDestroy(e);
   for (int i = 0; i < ccb_ctx::kTimingSlots; ++i)
     for (cudaEvent_t e : {c->ev_t0[i], c->ev_t1[i], c->ev_t2[i]})
@@ -1052,6 +1298,13 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   c->seq_lengths = a.arr<float>(c->max_rows);
   c->has_stopped = a.arr<uint8_t>(c->max_rows);
   c->bos_token = a.arr<int>(D.max_images);
+  c->row_step = a.arr<int>(c->max_rows);
+  c->slot_image = a.arr<int>(c->max_rows);
+  c->slot_ids = a.arr<long long>(c->max_rows);
+  c->refill_slots = a.arr<int>(c->max_rows);
+  c->refill_ids = a.arr<long long>(D.max_images);
+  c->refill_next = a.arr<int>(D.max_images);
+  c->cont_out = a.arr<int*>(2);
 
   // ---- persistent decode kernel: GPT-2 blocks with head_dim 64 (every GPT-2 size), up to 256 rows per step
   MegaState& mg = c->mega;
@@ -1100,11 +1353,17 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   if (cudaStreamCreateWithFlags(&c->work, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_in, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_out, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&c->ev_round[0], cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&c->ev_round[1], cudaEventDisableTiming) != cudaSuccess ||
+      cudaMallocHost(&c->host_pinned, static_cast<size_t>(2) * c->max_rows * (1 + 2 * sizeof(int))) != cudaSuccess ||
       cudaDeviceSynchronize() != cudaSuccess) {
     fail(nullptr, "ccb_create: stream / event creation failed: %s", cudaGetErrorString(cudaGetLastError()));
     ccb_destroy(c);
     return -1;
   }
+  c->h_slot_image = static_cast<int*>(c->host_pinned);
+  c->h_refill = c->h_slot_image + 2 * c->max_rows;
+  c->h_finished = reinterpret_cast<uint8_t*>(c->h_refill + 2 * c->max_rows);
   for (int i = 0; i < ccb_ctx::kTimingSlots; ++i) {
     if (cudaEventCreate(&c->ev_t0[i]) != cudaSuccess || cudaEventCreate(&c->ev_t1[i]) != cudaSuccess ||
         cudaEventCreate(&c->ev_t2[i]) != cudaSuccess) {
@@ -1246,25 +1505,23 @@ int ccb_caption_images(ccb_ctx* c, const ccb_gen_params* p, const void* images, 
   DeviceGuard dev_guard(c->device);
   cudaStream_t caller = static_cast<cudaStream_t>(stream);
   if (fence_in(c, caller)) return -1;
-  cudaStream_t s = c->work;
-  const int P = c->desc.map_prefix_len, d = c->desc.lm_d;
-  const int extra = append_bos >= 0 ? 1 : 0;
-  const bool all_tokens = c->desc.map_kind == CCB_MAP_TRANSFORMER_ALL;
-  if (all_tokens && c->desc.vit_present && c->desc.map_clip_len != (c->desc.vit_image / c->desc.vit_patch) * (c->desc.vit_image / c->desc.vit_patch) + 1)
-    return fail(c, "ccb_caption_images: map_clip_len=%d does not match the ViT's token count", c->desc.map_clip_len);
-  int r = vit_forward(c, images, dtype, N, c->feat, s, all_tokens);
-  if (r == 0) r = map_forward(c, c->feat, N, c->prefix, P + extra, s);
-  if (r == 0 && extra) {
-    if (append_bos >= c->desc.lm_vocab) {
-      r = fail(c, "ccb_caption_images: BOS id %d outside the vocabulary", append_bos);
-    } else {
-      token_rows_kernel<<<N, 256, 0, s>>>(c->wte, append_bos, c->prefix, static_cast<long long>(P + extra) * d, P, d);
-      const int lc = launch_check();
-      if (lc) r = fail(c, "token_rows_kernel: %s", cudaGetErrorString(static_cast<cudaError_t>(lc)));
-      else c->launches++;
-    }
-  }
-  if (r == 0) r = generate_on_work_stream(c, p, c->prefix, N, P + extra, tokens_out, lengths_out, scores_out);
+  const char* why = image_path_unsupported(c, append_bos);
+  int r = why ? fail(c, "ccb_caption_images: %s", why) : image_prefix(c, images, dtype, N, append_bos, c->work);
+  if (r == 0) r = generate_on_work_stream(c, p, c->prefix, N, c->desc.map_prefix_len + (append_bos >= 0 ? 1 : 0), tokens_out,
+                                          lengths_out, scores_out);
+  if (fence_out(c, caller)) return -1;
+  return r;
+}
+
+int ccb_caption_dataset(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int n_images, int rows,
+                        int append_bos, int64_t first_row_id, int32_t* tokens_out, int32_t* lengths_out,
+                        int64_t* decode_steps_out, void* stream) {
+  if (!c || !p || !images || !tokens_out || !lengths_out || !decode_steps_out) return fail(c, "ccb_caption_dataset: null argument");
+  DeviceGuard dev_guard(c->device);
+  cudaStream_t caller = static_cast<cudaStream_t>(stream);
+  if (fence_in(c, caller)) return -1;
+  const int r = caption_dataset_on_work_stream(c, p, images, dtype, n_images, rows, append_bos, first_row_id, tokens_out,
+                                               lengths_out, decode_steps_out);
   if (fence_out(c, caller)) return -1;
   return r;
 }

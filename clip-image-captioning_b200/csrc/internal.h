@@ -194,6 +194,8 @@ struct SampleParams {
   const long long* row_ids = nullptr;  // global image ids for the Philox key (null -> row index)
   const int* step = nullptr;           // device step counter (null -> step_scalar)
   int step_scalar = 0;
+  const int* row_step = nullptr;       // per-row steps [B] (continuous batching): where non-null, row b's Philox step and
+                                       // history length are row_step[b], overriding step / hist_len
   float* filtered_out = nullptr;       // optional [B, ld] masked logits (for parity tests of the processors)
   int* alt_out = nullptr;              // optional second sample (multinomial(p, 2) column 1)
 };
@@ -215,10 +217,25 @@ int beam_step(const float* logits, long long ld, int N, int beam, int V, float t
               const BeamState& st, int* next_tokens /*[N*beam]*/, int* src_rows /*[N*beam] global row ids*/,
               int* block_table /*[N*beam, max_pages] permuted in place, or null*/, int max_pages,
               const int* ctx_len /*[N*beam] cached tokens per row*/, cudaStream_t s);
+// Per-row mode of advance_rows (continuous batching: every row decodes its own image at its own step).  Entry i of
+// `next` belongs to row r = slots[i] (slots null: r = i).  A row whose image is < 0 or that is finished is frozen: nothing
+// is written and neither ctx_len nor its step advances.  Otherwise, with st = row_step[r]: tokens_out[r, st] (the row's
+// sampling history) and out[0][image * max_len + st] = the token, out[1][image] = st + 1, stop counting as below, the
+// row finishes at its stop rule or when st + 1 == max_len, ctx_len[r] += 1 (when non-null), row_step[r] = st + 1, and
+// with next_tokens non-null next_tokens[r] = the token (the scatter of a refill's first tokens).
+struct RowAdvance {
+  int* row_step = nullptr;          // [rows]
+  const int* row_image = nullptr;   // [rows]
+  const int* slots = nullptr;       // [entries of next] or null
+  int* next_tokens = nullptr;       // [rows] or null
+  int* const* out = nullptr;        // device {tokens [n_images, max_len], lengths [n_images]}: caller output pointers
+};
 // Per-step bookkeeping after a sampled token: tokens_out[r, *step] = next[r]; stop counting (stop_token up to
-// max_stops, eos_token) -> lengths / finished; *step += 1.  Null pointers skip the corresponding part.
+// max_stops, eos_token) -> lengths / finished; *step += 1.  Null pointers skip the corresponding part.  With `per_row`
+// the rows advance as RowAdvance describes and `step` is not used.
 int advance_rows(const int* next, int rows, int* tokens_out, int max_len, int* lengths, int* stops, uint8_t* finished,
-                 int* ctx_len, int* step, int stop_token, int max_stops, int eos_token, cudaStream_t s);
+                 int* ctx_len, int* step, int stop_token, int max_stops, int eos_token, cudaStream_t s,
+                 const RowAdvance* per_row = nullptr);
 // x[r] += 1 for r < rows; *scalar += 1 when non-null
 int increment_rows(int* x, int rows, int* scalar, cudaStream_t s);
 

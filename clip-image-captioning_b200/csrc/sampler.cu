@@ -373,6 +373,7 @@ struct TopPArgs {
   const long long* row_ids;
   const int* step;
   int step_scalar;
+  const int* row_step;
   float* filtered_out;
   int* alt_out;
   int* next;
@@ -526,7 +527,8 @@ __global__ void __launch_bounds__(kSampThreads) top_p_kernel(const TopPArgs a) {
   __syncthreads();
   // repetition penalty (values computed from the ORIGINAL logits, like gather -> where -> scatter_)
   if (a.rep_pen != 1.0f && a.history != nullptr) {
-    const int hl = a.hist_len ? a.hist_len[b] : (a.hist_len_from_step && a.step ? *a.step : a.hist_len_scalar);
+    const int hl = a.row_step ? a.row_step[b]
+                 : a.hist_len ? a.hist_len[b] : (a.hist_len_from_step && a.step ? *a.step : a.hist_len_scalar);
     for (int t = threadIdx.x; t < hl; t += blockDim.x) {
       const int tok = a.history[static_cast<long long>(b) * a.ld_hist + t];
       if (tok >= 0 && tok < V) {
@@ -567,7 +569,8 @@ __global__ void __launch_bounds__(kSampThreads) top_p_kernel(const TopPArgs a) {
     const bool typ_on = (a.typ_p_rows != nullptr && typ >= 0.f) || (a.typ_p_rows == nullptr && typ > 0.f);
     if (a.fast && top_p > 0.f && !typ_on && a.filtered_out == nullptr && a.alt_out == nullptr) {
       const unsigned long long rid_f = a.row_ids ? static_cast<unsigned long long>(a.row_ids[b]) : static_cast<unsigned long long>(b);
-      const uint32_t step_f = a.step ? static_cast<uint32_t>(*a.step) : static_cast<uint32_t>(a.step_scalar);
+      const uint32_t step_f = a.row_step ? static_cast<uint32_t>(a.row_step[b])
+                            : a.step ? static_cast<uint32_t>(*a.step) : static_cast<uint32_t>(a.step_scalar);
       const float* qrow_f = a.q_noise ? a.q_noise + static_cast<long long>(step_f) * a.q_step_stride + static_cast<long long>(b) * a.ldq : nullptr;
       const int tok = nucleus_sample_fast(vals, V, mx, 1.0f / sum, top_p, qrow_f, a.seed, rid_f, step_f, ascratch, dscratch, iscratch);
       if (tok >= 0) {
@@ -664,7 +667,8 @@ __global__ void __launch_bounds__(kSampThreads) top_p_kernel(const TopPArgs a) {
   for (int v = threadIdx.x; v < V; v += blockDim.x) ksum += expf(vals[v] - mx);
   ksum = block_sum(ksum, fscratch);
   const unsigned long long rid = a.row_ids ? static_cast<unsigned long long>(a.row_ids[b]) : static_cast<unsigned long long>(b);
-  const uint32_t step = a.step ? static_cast<uint32_t>(*a.step) : static_cast<uint32_t>(a.step_scalar);
+  const uint32_t step = a.row_step ? static_cast<uint32_t>(a.row_step[b])
+                      : a.step ? static_cast<uint32_t>(*a.step) : static_cast<uint32_t>(a.step_scalar);
   const float* qrow = a.q_noise ? a.q_noise + static_cast<long long>(step) * a.q_step_stride + static_cast<long long>(b) * a.ldq : nullptr;
   ArgMax best;
   best.v = -INFINITY;
@@ -1141,6 +1145,33 @@ __global__ void advance_kernel(const int* __restrict__ next, int rows, int* toke
   if (threadIdx.x == 0) *step = st + 1;
 }
 
+// the per-row mode (internal.h: RowAdvance)
+__global__ void advance_rows_kernel(const int* __restrict__ next, int n, int* hist, int max_len, int* lengths, int* stops,
+                                    uint8_t* finished, int* ctx_len, int stop_token, int max_stops, int eos_token,
+                                    const RowAdvance ra) {
+  ptx::grid_dep_wait();
+  ptx::grid_dep_launch();
+  int* out_tokens = ra.out[0];
+  int* out_lengths = ra.out[1];
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const int r = ra.slots ? ra.slots[i] : i;
+    const int img = ra.row_image[r];
+    if (img < 0 || finished[r]) continue;
+    const int tok = next[i];
+    const int st = ra.row_step[r];
+    hist[static_cast<long long>(r) * max_len + st] = tok;
+    out_tokens[static_cast<long long>(img) * max_len + st] = tok;
+    out_lengths[img] = st + 1;
+    const int sc = stops[r] + (tok == stop_token ? 1 : 0);
+    stops[r] = sc;
+    lengths[r] = st + 1;
+    if ((max_stops > 0 && sc >= max_stops) || (eos_token >= 0 && tok == eos_token) || st + 1 >= max_len) finished[r] = 1;
+    if (ctx_len) ctx_len[r] += 1;
+    ra.row_step[r] = st + 1;
+    if (ra.next_tokens) ra.next_tokens[r] = tok;
+  }
+}
+
 }  // namespace
 
 int sample_greedy(const float* logits, long long ld, int B, int V, int* next, cudaStream_t s) {
@@ -1178,7 +1209,7 @@ int sample_top_p(const float* logits, long long ld, int B, int V, const SamplePa
   a.rep_pen = sp.repetition_penalty; a.history = sp.history; a.ld_hist = sp.ld_hist;
   a.hist_len = sp.hist_len; a.hist_len_scalar = sp.hist_len_scalar; a.hist_len_from_step = sp.hist_len_from_step;
   a.q_noise = sp.q_noise; a.ldq = sp.ldq; a.q_step_stride = sp.q_step_stride; a.seed = sp.seed; a.row_ids = sp.row_ids;
-  a.step = sp.step; a.step_scalar = sp.step_scalar;
+  a.step = sp.step; a.step_scalar = sp.step_scalar; a.row_step = sp.row_step;
   a.filtered_out = sp.filtered_out; a.alt_out = sp.alt_out; a.next = next;
   static const bool fast_on = [] {   // CCB_SAMPLER_FAST=0: always the radix select (A/B)
     const char* e = getenv("CCB_SAMPLER_FAST");
@@ -1231,7 +1262,15 @@ int increment_rows(int* x, int rows, int* scalar, cudaStream_t s) {
 }
 
 int advance_rows(const int* next, int rows, int* tokens_out, int max_len, int* lengths, int* stops, uint8_t* finished,
-                 int* ctx_len, int* step, int stop_token, int max_stops, int eos_token, cudaStream_t s) {
+                 int* ctx_len, int* step, int stop_token, int max_stops, int eos_token, cudaStream_t s,
+                 const RowAdvance* per_row) {
+  if (per_row) {
+    if (!per_row->row_step || !per_row->row_image || !per_row->out || !tokens_out || !lengths || !stops || !finished)
+      return (int)cudaErrorInvalidValue;
+    const cudaError_t e = launch_kernel(advance_rows_kernel, dim3(1), dim3(1024), 0, s, true, next, rows, tokens_out, max_len,
+                                        lengths, stops, finished, ctx_len, stop_token, max_stops, eos_token, *per_row);
+    return e == cudaSuccess ? 0 : (int)e;
+  }
   cudaError_t e = launch_kernel(advance_kernel, dim3(1), dim3(1024), 0, s, true, next, rows, tokens_out, max_len, lengths,
                                 stops, finished, ctx_len, step, stop_token, max_stops, eos_token);
   return e == cudaSuccess ? 0 : (int)e;

@@ -447,6 +447,27 @@ class Engine:
         scores = torch.cat(scs, 0) if scs and scs[0] is not None else None
         return tokens, lengths, scores
 
+    def caption_dataset_continuous(self, images: torch.Tensor, p: GenParams, rows: Optional[int] = None,
+                                   first_row_id: int = 0, append_bos: int = -1):
+        """`caption_dataset` with continuous batching (ccb_caption_dataset), greedy or sampling: `rows` decode slots
+        (default `micro_batch_for(p)`) stay busy, and a slot whose caption has finished takes the next image instead of
+        decoding to max_new_tokens.  Returns (tokens [n, T], lengths [n], decode steps run).  Per image the caption equals
+        `caption_dataset`'s; positions at or past a caption's length are 0.  Sampling keys the Philox streams by
+        first_row_id + image index, as `caption_dataset` does.  Synchronises the host once per round of decode steps."""
+        images = self._dev(images)
+        if images.dtype not in _TORCH_DTYPE:
+            images = images.float()
+        n = images.shape[0]
+        rows = rows or self.micro_batch_for(p)
+        tokens = torch.empty(n, p.max_new_tokens, device=self.device, dtype=torch.int32)
+        lengths = torch.empty(n, device=self.device, dtype=torch.int32)
+        steps = C.c_int64()
+        self._check(self.lib.ccb_caption_dataset(self._h, C.byref(p), _ptr(images), _TORCH_DTYPE[images.dtype], n, rows,
+                                                 append_bos, first_row_id, _ptr(tokens), _ptr(lengths), C.byref(steps),
+                                                 self._stream()))
+        self._keep = [images, p]
+        return tokens, lengths, int(steps.value)
+
     # ------------------------------------------------------------------------------------------ samplers
     def sample(self, logits: torch.Tensor, p: GenParams, history: Optional[torch.Tensor] = None, step: int = 0,
                return_filtered: bool = False, return_alt: bool = False):

@@ -63,3 +63,16 @@ def caption_images_sharded(engine, images: torch.Tensor, params, n_items: Option
     # micro-batches sized for the fastest decode path (Engine.micro_batch_for); Philox streams keyed by global image id
     tokens, lengths, _ = engine.caption_dataset(images, params, first_row_id=lo)
     return gather_captions(tokens, lengths, n_items, group)
+
+
+def caption_images_sharded_continuous(engine, images: torch.Tensor, params, n_items: Optional[int] = None, group=None,
+                                      rows: Optional[int] = None):
+    """`caption_images_sharded` on Engine.caption_dataset_continuous (greedy / sampling): finished rows take the next
+    image of this rank's shard.  Same result up to near-ties, and positions past a caption's length are 0."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    if n_items is None:
+        n_items = images.shape[0] * world
+    lo, _ = shard_range(n_items, rank, world)
+    tokens, lengths, _ = engine.caption_dataset_continuous(images, params, rows=rows, first_row_id=lo)
+    return gather_captions(tokens, lengths, n_items, group)

@@ -11,7 +11,7 @@
  *   - every data pointer is a DEVICE pointer to a contiguous row-major tensor owned by the caller (PyTorch);
  *     the library never frees caller memory and allocates only inside ccb_create.
  *   - every call is asynchronous on `stream` (a cudaStream_t passed as void*); no host synchronisation except
- *     where stated.  A ccb_ctx is bound to one device and is not thread-safe (one ctx per rank / GPU).
+ *     where stated (ccb_caption_dataset, ccb_beam_step).  A ccb_ctx is bound to one device and is not thread-safe (one ctx per rank / GPU).
  *   - there is no CPU fallback: without an sm_100 device ccb_create fails.
  */
 #ifndef CLIPCAP_B200_H_
@@ -153,6 +153,20 @@ CCB_API int ccb_generate(ccb_ctx* ctx, const ccb_gen_params* params, const float
  * append_bos >= 0, evaluate_model.py:124-133) + ccb_generate.  Same outputs as ccb_generate. */
 CCB_API int ccb_caption_images(ccb_ctx* ctx, const ccb_gen_params* params, const void* images, int dtype, int N,
                        int append_bos, int32_t* tokens_out, int32_t* lengths_out, float* scores_out, void* stream);
+/* A whole shard of images -> captions with continuous batching, greedy or sampling: `rows` decode slots stay busy, and a
+ * slot whose caption has finished takes the next image.  images [n_images, 3, H, W] (device); tokens_out
+ * [n_images, max_new_tokens] and lengths_out [n_images] in image order (device); *decode_steps_out (HOST) = decode steps run.
+ * Per image, (tokens[:len], len) is what ccb_caption_images gives; unlike there, positions at or past a caption's length
+ * are 0.  Sampling keys each image's Philox stream by (seed, first_row_id + image index, step), so the result depends
+ * neither on `rows` nor on the order in which images are taken.
+ * The call synchronises the host once per round of a few decode steps, to learn which slots have finished; it returns
+ * once the last round has completed.  ccb_last_timing / ccb_timing_sum do not count it.
+ * Rejected with a message, nothing launched: beam mode, q_noise, the per-row arrays (row_ids, top_p_rows, top_k_rows,
+ * typ_p_rows), rows outside [1, max_images * max_beam], map_prefix_len (+ 1 with append_bos >= 0) + max_new_tokens above
+ * max_ctx, and the prefix shapes ccb_caption_images rejects. */
+CCB_API int ccb_caption_dataset(ccb_ctx* ctx, const ccb_gen_params* params, const void* images, int dtype, int n_images,
+                                int rows, int append_bos, int64_t first_row_id, int32_t* tokens_out, int32_t* lengths_out,
+                                int64_t* decode_steps_out, void* stream);
 /* number of kernels launched by the library on this context since creation (CUDA-graph replays count the
  * kernels inside the graph) */
 CCB_API int64_t ccb_launch_count(const ccb_ctx* ctx);
