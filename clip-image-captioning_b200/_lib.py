@@ -58,6 +58,7 @@ PROTOTYPES = {
     "ccb_generate": (_I, [_P, C.POINTER(GenParams), _P, _I, _I, _P, _P, _P, _P]),
     "ccb_caption_images": (_I, [_P, C.POINTER(GenParams), _P, _I, _I, _I, _P, _P, _P, _P]),
     "ccb_caption_dataset": (_I, [_P, C.POINTER(GenParams), _P, _I, _I, _I, _I, _L, _P, _P, C.POINTER(_L), _P]),
+    "ccb_caption_dataset_beam": (_I, [_P, C.POINTER(GenParams), _P, _I, _I, _I, _I, _P, _P, _P, C.POINTER(_L), _P]),
     "ccb_launch_count": (_L, [_P]),
     "ccb_last_timing": (_I, [_P, C.POINTER(_F), C.POINTER(_F), C.POINTER(_I)]),
     "ccb_timing_sum": (_I, [_P, _I, C.POINTER(_F), C.POINTER(_F), C.POINTER(_I)]),

@@ -50,6 +50,14 @@ int fail(ccb_ctx* c, const char* fmt, ...) {
   } while (0)
 
 // ------------------------------------------------------------------------------------------ small kernels
+// Beam search with token-granular pages (page_tokens == 1).  Image (group) g owns pages [g * ppi, (g+1) * ppi),
+// ppi = S0 + beam * T: the first S0 hold the prefix shared by all beams; row k's token written at step j - S0 goes to
+// S0 + (j - S0) * beam + k.  The KV page of position j of row k:
+__device__ __forceinline__ int beam_page(int g, int k, int j, int beam, int S0, int T) {
+  const int base = g * (S0 + beam * T);
+  return j < S0 ? base + j : base + S0 + (j - S0) * beam + k;
+}
+
 __global__ void init_state_kernel(int* block_table, int* block_table_prefill, int max_pages, int rows, int N, int beam,
                                   int S0, int T, int page_tokens, int pages_per_row, int* ctx_len, int* step,
                                   int* lengths, int* stops, uint8_t* finished, float* scores, float* seq_lengths,
@@ -64,14 +72,11 @@ __global__ void init_state_kernel(int* block_table, int* block_table_prefill, in
       block_table_prefill[static_cast<long long>(r) * max_pages + j] = i;
     }
   } else {
-    // token-granular pages (page_tokens == 1).  Image n owns pages [n * ppi, (n+1) * ppi), ppi = S0 + beam * T:
-    // the first S0 hold the prefix shared by all beams; row k's token written at step j goes to
-    // S0 + j * beam + k.  beam_step permutes the entries [0, ctx) of a row, never the fresh ones.
-    const int ppi = S0 + beam * T;
+    // image n is group n of beam_page; beam_step permutes the entries [0, ctx) of a row, never the fresh ones
     for (int i = tid; i < rows * (S0 + T); i += nth) {
       const int r = i / (S0 + T), j = i % (S0 + T);
       const int n = r / beam, k = r % beam;
-      const int page = (j < S0) ? n * ppi + j : n * ppi + S0 + (j - S0) * beam + k;
+      const int page = beam_page(n, k, j, beam, S0, T);
       block_table[static_cast<long long>(r) * max_pages + j] = page;
       if (k == 0 && j < S0) block_table_prefill[static_cast<long long>(n) * max_pages + j] = page;
     }
@@ -558,9 +563,12 @@ int select_step(ccb_ctx* c, const ccb_gen_params* p, int rows, int T, bool after
   return 0;
 }
 
-int beam_select(ccb_ctx* c, const ccb_gen_params* p, int N, int T, bool first, cudaStream_t s) {
+// one beam step over N images; with `groups` over N launch entries in beam_step's per-group mode, which advances
+// ctx_len and the step itself
+int beam_select(ccb_ctx* c, const ccb_gen_params* p, int N, int T, bool first, cudaStream_t s,
+                const BeamGroups* groups = nullptr) {
   const int beam = p->beam_size, rows = N * beam;
-  if (!first) RUN(increment_rows(c->ctx_len, rows, c->step, s));
+  if (!first && !groups) RUN(increment_rows(c->ctx_len, rows, c->step, s));
   BeamState st;
   st.scores = c->scores;
   st.seq_lengths = c->seq_lengths;
@@ -572,7 +580,7 @@ int beam_select(ccb_ctx* c, const ccb_gen_params* p, int N, int T, bool first, c
   st.cand_rows = c->max_rows;
   if (c->capturing) c->capture_launches++; else c->launches++;   // (beam_step launches two kernels)
   RUN(beam_step(c->logits, c->ldv, N, beam, c->desc.lm_vocab, p->temperature, p->stop_token, st, c->next_tokens,
-                c->src_rows, c->block_table, c->max_pages_per_row, c->ctx_len, s));
+                c->src_rows, c->block_table, c->max_pages_per_row, c->ctx_len, s, groups));
   return 0;
 }
 
@@ -736,7 +744,7 @@ constexpr int kRoundSteps = 4;
 // every slot empty (finished, no image) at position S0 of its own pages [r * ppr, (r+1) * ppr); the outputs' pointers
 __global__ void cont_init_kernel(int* block_table, int max_pages, int rows, int pages_per_row, int S0, int* ctx_len,
                                  int* row_step, int* slot_image, int* next_tokens, int* lengths, int* stops,
-                                 uint8_t* finished, int** cont_out, int* tokens_out, int* lengths_out) {
+                                 uint8_t* finished, void** cont_out, void* tokens_out, void* lengths_out) {
   const int tid = blockIdx.x * blockDim.x + threadIdx.x;
   const int nth = gridDim.x * blockDim.x;
   for (int i = tid; i < rows * pages_per_row; i += nth)
@@ -787,6 +795,65 @@ RowAdvance row_advance(ccb_ctx* c, const int* slots, int* next_tokens) {
   return ra;
 }
 
+// The round protocol of continuous batching, shared by ccb_caption_dataset (a unit is one decode row) and
+// ccb_caption_dataset_beam (a unit is the group of beam rows of one image).  Unit u reports c->finished[u] and
+// c->slot_image[u]; `ge` runs one round of kRoundSteps decode iterations; refill_chunk(off, k, img0) enqueues images
+// img0 .. img0 + k - 1 into the units c->refill_slots[off, off + k).
+//
+// The host keeps one round ahead: it reads round j's state while round j + 1 runs, and refills the units that had
+// finished by round j at the boundary after round j + 1.  A finished unit is frozen, so nothing it holds changes in
+// between; a unit shows as free when its snapshot is finished with the image the host last gave it.
+template <class RefillChunk>
+int continuous_rounds(ccb_ctx* c, const GraphEntry* ge, int n, int units, int chunk, int64_t* steps_out,
+                      RefillChunk refill_chunk) {
+  cudaStream_t s = c->work;
+  std::vector<int> occupant(units, -1);   // image the host gave each unit, -1 = free
+  int next_image = 0;
+  auto refill = [&](int boundary) -> int {
+    int* list = c->h_refill + (boundary % 2) * c->max_rows;
+    int m = 0;
+    for (int u = 0; u < units && next_image + m < n; ++u)
+      if (occupant[u] < 0) list[m++] = u;
+    if (m == 0) return 0;
+    CUDA_OK(cudaMemcpyAsync(c->refill_slots, list, sizeof(int) * m, cudaMemcpyHostToDevice, s));
+    for (int off = 0; off < m; off += chunk)
+      if (refill_chunk(off, std::min(chunk, m - off), next_image + off)) return -1;
+    for (int i = 0; i < m; ++i) occupant[list[i]] = next_image + i;
+    next_image += m;
+    return 0;
+  };
+  auto round = [&](int j) -> int {
+    CUDA_OK(cudaGraphLaunch(ge->exec, s));
+    c->launches += ge->nodes;
+    CUDA_OK(cudaMemcpyAsync(c->h_finished + (j % 2) * c->max_rows, c->finished, units, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaMemcpyAsync(c->h_slot_image + (j % 2) * c->max_rows, c->slot_image, sizeof(int) * units, cudaMemcpyDeviceToHost, s));
+    CUDA_OK(cudaEventRecord(c->ev_round[j % 2], s));
+    return 0;
+  };
+  if (refill(0) || round(0) || round(1)) return -1;
+  long long rounds = 2;
+  for (int j = 0;; ++j) {
+    CUDA_OK(cudaEventSynchronize(c->ev_round[j % 2]));
+    const uint8_t* fin = c->h_finished + (j % 2) * c->max_rows;
+    const int* img = c->h_slot_image + (j % 2) * c->max_rows;
+    bool busy = false;
+    for (int u = 0; u < units; ++u) {
+      if (occupant[u] < 0) continue;
+      if (fin[u] && img[u] == occupant[u]) occupant[u] = -1;
+      else busy = true;
+    }
+    if (!busy && next_image == n) {
+      // round j + 1 is still running: the pinned ring is free for the next call once it has read its last refill list
+      CUDA_OK(cudaEventSynchronize(c->ev_round[(j + 1) % 2]));
+      break;
+    }
+    if (refill(j + 1) || round(j + 2)) return -1;
+    ++rounds;
+  }
+  *steps_out = rounds * kRoundSteps;
+  return 0;
+}
+
 // one decode iteration over all slots: the step, token selection keyed by (seed, image id, row step), per-row advance
 int cont_iteration(ccb_ctx* c, const ccb_gen_params* p, int rows, int T, cudaStream_t s) {
   if (lm_decode_step(c, rows, s)) return -1;
@@ -806,12 +873,17 @@ int cont_iteration(ccb_ctx* c, const ccb_gen_params* p, int rows, int T, cudaStr
   return 0;
 }
 
+// image i of images [n, 3, H, W]
+const void* image_at(ccb_ctx* c, const void* images, int dtype, int i) {
+  const size_t image_bytes = static_cast<size_t>(3) * c->desc.vit_image * c->desc.vit_image * (dtype == CCB_DTYPE_F32 ? 4 : 2);
+  return static_cast<const char*>(images) + image_bytes * i;
+}
+
 // k consecutive images from img0 into slots c->refill_slots[off, off + k): prefix, prefill into the slots' pages, first token
 int cont_refill(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int append_bos, long long first_row_id,
                 int off, int k, int img0, int S0, int T, int pages_per_row, cudaStream_t s) {
   const ccb_model_desc& D = c->desc;
-  const size_t image_bytes = static_cast<size_t>(3) * D.vit_image * D.vit_image * (dtype == CCB_DTYPE_F32 ? 4 : 2);
-  if (image_prefix(c, static_cast<const char*>(images) + image_bytes * img0, dtype, k, append_bos, s)) return -1;
+  if (image_prefix(c, image_at(c, images, dtype, img0), dtype, k, append_bos, s)) return -1;
   cont_refill_kernel<<<1, 256, 0, s>>>(c->refill_slots + off, k, img0, first_row_id, c->max_pages_per_row, pages_per_row, S0,
                                        c->block_table_prefill, c->ctx_len, c->row_step, c->slot_image, c->slot_ids,
                                        c->refill_ids, c->lengths, c->stops, c->finished);
@@ -838,7 +910,7 @@ int caption_dataset_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const vo
   cudaStream_t s = c->work;
   const int T = p->max_new_tokens;
   const int S0 = D.map_prefix_len + (append_bos >= 0 ? 1 : 0);
-  if (p->mode == CCB_GEN_BEAM) return fail(c, "ccb_caption_dataset: beam search is not supported (ccb_caption_images has it)");
+  if (p->mode == CCB_GEN_BEAM) return fail(c, "ccb_caption_dataset: beam search is not supported (ccb_caption_dataset_beam has it)");
   if (p->mode != CCB_GEN_GREEDY && p->mode != CCB_GEN_SAMPLE) return fail(c, "ccb_caption_dataset: unknown mode %d", p->mode);
   if (p->q_noise) return fail(c, "ccb_caption_dataset: q_noise is not supported (its [step, row] layout has no meaning here)");
   if (p->row_ids || p->top_p_rows || p->top_k_rows || p->typ_p_rows)
@@ -877,57 +949,145 @@ int caption_dataset_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const vo
                                         });
   if (!ge) return -1;
 
-  // The host keeps one round ahead: it reads round j's slot state while round j + 1 runs, and refills the slots that had
-  // finished by round j at the boundary after round j + 1.  A finished slot is frozen, so nothing it holds changes in
-  // between; a slot shows as free when its snapshot is finished with the image the host last gave it.
-  const int chunk = std::min(D.max_images, D.max_lm_tokens / S0);
-  std::vector<int> occupant(rows, -1);   // image the host gave each slot, -1 = free
-  int next_image = 0;
-  auto refill = [&](int boundary) -> int {
-    int* list = c->h_refill + (boundary % 2) * c->max_rows;
-    int m = 0;
-    for (int r = 0; r < rows && next_image + m < n; ++r)
-      if (occupant[r] < 0) list[m++] = r;
-    if (m == 0) return 0;
-    CUDA_OK(cudaMemcpyAsync(c->refill_slots, list, sizeof(int) * m, cudaMemcpyHostToDevice, s));
-    for (int off = 0; off < m; off += chunk)
-      if (cont_refill(c, p, images, dtype, append_bos, first_row_id, off, std::min(chunk, m - off), next_image + off, S0, T,
-                      pages_per_row, s))
-        return -1;
-    for (int i = 0; i < m; ++i) occupant[list[i]] = next_image + i;
-    next_image += m;
-    return 0;
-  };
-  auto round = [&](int j) -> int {
-    CUDA_OK(cudaGraphLaunch(ge->exec, s));
-    c->launches += ge->nodes;
-    CUDA_OK(cudaMemcpyAsync(c->h_finished + (j % 2) * c->max_rows, c->finished, rows, cudaMemcpyDeviceToHost, s));
-    CUDA_OK(cudaMemcpyAsync(c->h_slot_image + (j % 2) * c->max_rows, c->slot_image, sizeof(int) * rows, cudaMemcpyDeviceToHost, s));
-    CUDA_OK(cudaEventRecord(c->ev_round[j % 2], s));
-    return 0;
-  };
-  if (refill(0) || round(0) || round(1)) return -1;
-  long long rounds = 2;
-  for (int j = 0;; ++j) {
-    CUDA_OK(cudaEventSynchronize(c->ev_round[j % 2]));
-    const uint8_t* fin = c->h_finished + (j % 2) * c->max_rows;
-    const int* img = c->h_slot_image + (j % 2) * c->max_rows;
-    bool busy = false;
-    for (int r = 0; r < rows; ++r) {
-      if (occupant[r] < 0) continue;
-      if (fin[r] && img[r] == occupant[r]) occupant[r] = -1;
-      else busy = true;
-    }
-    if (!busy && next_image == n) {
-      // round j + 1 is still running: the pinned ring is free for the next call once it has read its last refill list
-      CUDA_OK(cudaEventSynchronize(c->ev_round[(j + 1) % 2]));
-      break;
-    }
-    if (refill(j + 1) || round(j + 2)) return -1;
-    ++rounds;
+  return continuous_rounds(c, ge, n, rows, std::min(D.max_images, D.max_lm_tokens / S0), steps_out,
+                           [&](int off, int k, int img0) {
+                             return cont_refill(c, p, images, dtype, append_bos, first_row_id, off, k, img0, S0, T,
+                                                pages_per_row, s);
+                           });
+}
+
+// ---- beam search (ccb_caption_dataset_beam): a unit is the group of beam rows [g * beam, (g+1) * beam) of one image,
+// on the pages beam_page gives group g.  c->row_step / c->slot_image / c->finished hold the groups' state.
+//
+// Entry i < k resets group g = slots[i] (slots null: g = i) to take image img0 + i from its first beam step on or, with
+// img0 < 0, to be empty (image -1, finished): the block tables of its rows over its own pages (the previous occupant's
+// beam steps permuted them), ctx_len = S0, zeroed token rows (a stopped beam leaves zeros behind its length), fresh
+// scores, and prefill row i's block table on its prefix pages.  Non-null outputs are stored for the captured rounds.
+__global__ void beam_group_reset_kernel(const int* __restrict__ slots, int k, int img0, int beam, int S0, int T,
+                                        int max_pages, int* block_table, int* block_table_prefill, int* ctx_len,
+                                        int* next_tokens, int* gen_tokens, float* scores, float* seq_lengths,
+                                        uint8_t* has_stopped, int* group_step, int* group_image, uint8_t* finished,
+                                        void** cont_out, void* tokens_out, void* lengths_out, void* scores_out) {
+  const int tid = blockIdx.x * blockDim.x + threadIdx.x;
+  const int nth = gridDim.x * blockDim.x;
+  const int W = S0 + T;
+  for (int i = tid; i < k * beam * W; i += nth) {
+    const int e = i / (beam * W), kk = (i / W) % beam, j = i % W;
+    const int g = slots ? slots[e] : e;
+    block_table[static_cast<long long>(g * beam + kk) * max_pages + j] = beam_page(g, kk, j, beam, S0, T);
+    if (kk == 0 && j < S0) block_table_prefill[static_cast<long long>(e) * max_pages + j] = beam_page(g, 0, j, beam, S0, T);
   }
-  *steps_out = rounds * kRoundSteps;
-  return 0;
+  for (int i = tid; i < k * beam * T; i += nth) {
+    const int g = slots ? slots[i / (beam * T)] : i / (beam * T);
+    gen_tokens[static_cast<long long>(g) * beam * T + i % (beam * T)] = 0;
+  }
+  for (int i = tid; i < k * beam; i += nth) {
+    const int r = (slots ? slots[i / beam] : i / beam) * beam + i % beam;
+    ctx_len[r] = S0;
+    next_tokens[r] = 0;
+    scores[r] = 0.f;
+    seq_lengths[r] = 1.f;
+    has_stopped[r] = 0;
+  }
+  for (int i = tid; i < k; i += nth) {
+    const int g = slots ? slots[i] : i;
+    group_step[g] = 0;
+    group_image[g] = img0 < 0 ? -1 : img0 + i;
+    finished[g] = img0 < 0 ? 1 : 0;
+  }
+  if (tid == 0 && tokens_out) {
+    cont_out[0] = tokens_out;
+    cont_out[1] = lengths_out;
+    cont_out[2] = scores_out;
+  }
+}
+
+BeamGroups beam_groups(ccb_ctx* c, const int* slots) {
+  BeamGroups bg;
+  bg.group_step = c->row_step;
+  bg.group_image = c->slot_image;
+  bg.finished = c->finished;
+  bg.slots = slots;
+  bg.out = c->cont_out;
+  return bg;
+}
+
+void beam_group_reset(ccb_ctx* c, const int* slots, int k, int img0, int beam, int S0, int T, cudaStream_t s,
+                      void* tokens_out = nullptr, void* lengths_out = nullptr, void* scores_out = nullptr) {
+  beam_group_reset_kernel<<<148, 256, 0, s>>>(slots, k, img0, beam, S0, T, c->max_pages_per_row, c->block_table,
+                                              c->block_table_prefill, c->ctx_len, c->next_tokens, c->gen_tokens, c->scores,
+                                              c->seq_lengths, c->has_stopped, c->row_step, c->slot_image, c->finished,
+                                              c->cont_out, tokens_out, lengths_out, scores_out);
+}
+
+// k consecutive images from img0 into groups c->refill_slots[off, off + k): prefix, reset, prefill into the groups' prefix
+// pages (once per group, shared by its beams), the first beam step
+int beam_refill(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int append_bos, int off, int k, int img0,
+                int S0, int T, cudaStream_t s) {
+  if (image_prefix(c, image_at(c, images, dtype, img0), dtype, k, append_bos, s)) return -1;
+  const int* slots = c->refill_slots + off;
+  beam_group_reset(c, slots, k, img0, p->beam_size, S0, T, s);
+  RUN(launch_check());
+  if (lm_prefill_layers(c, c->prefix, k, S0, nullptr, true, s)) return -1;
+  if (lm_logits(c, k, S0, 1, c->logits, c->ldv, s)) return -1;
+  const BeamGroups bg = beam_groups(c, slots);
+  return beam_select(c, p, k, T, true, s, &bg);
+}
+
+int caption_dataset_beam_on_work_stream(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int n,
+                                        int groups, int append_bos, int32_t* tokens_out, int32_t* lengths_out,
+                                        float* scores_out, int64_t* steps_out) {
+  const ccb_model_desc& D = c->desc;
+  cudaStream_t s = c->work;
+  const int T = p->max_new_tokens, beam = p->beam_size;
+  const int S0 = D.map_prefix_len + (append_bos >= 0 ? 1 : 0);
+  const int max_beam = std::min(D.max_beam, 8);
+  if (p->mode != CCB_GEN_BEAM)
+    return fail(c, "ccb_caption_dataset_beam: mode %d is not beam search (ccb_caption_dataset takes greedy and sampling)", p->mode);
+  if (beam < 1 || beam > max_beam)
+    return fail(c, "ccb_caption_dataset_beam: beam_size=%d outside [1, min(max_beam, 8) = %d]", beam, max_beam);
+  if (dtype != CCB_DTYPE_F32 && dtype != CCB_DTYPE_F16 && dtype != CCB_DTYPE_BF16)
+    return fail(c, "ccb_caption_dataset_beam: unknown image dtype %d", dtype);
+  if (n <= 0) return fail(c, "ccb_caption_dataset_beam: n_images=%d must be positive", n);
+  if (groups < 1 || groups > D.max_images || groups * beam > c->max_rows)
+    return fail(c, "ccb_caption_dataset_beam: groups=%d outside [1, max_images = %d] (or groups * beam_size above %d rows)",
+                groups, D.max_images, c->max_rows);
+  if (T <= 0 || S0 + T > D.max_ctx)
+    return fail(c, "ccb_caption_dataset_beam: S0=%d + max_new_tokens=%d exceeds max_ctx=%d", S0, T, D.max_ctx);
+  if (S0 > D.max_lm_tokens) return fail(c, "ccb_caption_dataset_beam: S0=%d exceeds max_lm_tokens=%d", S0, D.max_lm_tokens);
+  if (const char* why = image_path_unsupported(c, append_bos)) return fail(c, "ccb_caption_dataset_beam: %s", why);
+  if (const char* why = attention_prefill_unsupported(S0, D.lm_d / D.lm_heads, 1, true, D.lm_rotary_dim, false))
+    return fail(c, "ccb_caption_dataset_beam: prefix of S0=%d tokens with head_dim %d: %s", S0, D.lm_d / D.lm_heads, why);
+  const long long need_tokens = static_cast<long long>(groups) * (S0 + static_cast<long long>(beam) * T);
+  if (need_tokens > c->kv_pool_tokens)
+    return fail(c, "ccb_caption_dataset_beam: KV pool too small (%lld > %lld tokens)", need_tokens, c->kv_pool_tokens);
+  const size_t smem = beam_merge_smem(beam, T, c->max_pages_per_row);
+  if (smem > kBeamMergeMaxSmem)
+    return fail(c, "ccb_caption_dataset_beam: the beam merge needs %zu bytes of shared memory for beam %d over max_ctx=%d "
+                   "positions, above its %zu", smem, beam, c->max_pages_per_row, kBeamMergeMaxSmem);
+  c->kv.page_tokens = 1;
+  c->kv.num_pages = static_cast<int>(c->kv_pool_tokens);
+  c->kv.max_pages_per_row = c->max_pages_per_row;
+
+  // every group empty, with valid block tables: the decode step runs its rows and appends their K/V on its own pages
+  beam_group_reset(c, nullptr, groups, -1, beam, S0, T, s, tokens_out, lengths_out, scores_out);
+  RUN(launch_check());
+  const int rows = groups * beam;
+  const BeamGroups bg = beam_groups(c, nullptr);
+  const GraphEntry* ge = captured_graph(c, "contbeam" + std::to_string(kRoundSteps) + " " +
+                                               graph_key(p, groups, rows, T, c->mega.enabled ? 1 : 0),
+                                        s, [&]() {
+                                          for (int i = 0; i < kRoundSteps; ++i) {
+                                            if (lm_decode_step(c, rows, s)) return -1;
+                                            if (beam_select(c, p, groups, T, false, s, &bg)) return -1;
+                                          }
+                                          return 0;
+                                        });
+  if (!ge) return -1;
+  return continuous_rounds(c, ge, n, groups, std::min(D.max_images, D.max_lm_tokens / S0), steps_out,
+                           [&](int off, int k, int img0) {
+                             return beam_refill(c, p, images, dtype, append_bos, off, k, img0, S0, T, s);
+                           });
 }
 
 int fence_in(ccb_ctx* c, cudaStream_t caller) {
@@ -1304,7 +1464,7 @@ int ccb_create(ccb_ctx** out, const ccb_model_desc* desc, int device) {
   c->refill_slots = a.arr<int>(c->max_rows);
   c->refill_ids = a.arr<long long>(D.max_images);
   c->refill_next = a.arr<int>(D.max_images);
-  c->cont_out = a.arr<int*>(2);
+  c->cont_out = a.arr<void*>(3);
 
   // ---- persistent decode kernel: GPT-2 blocks with head_dim 64 (every GPT-2 size), up to 256 rows per step
   MegaState& mg = c->mega;
@@ -1522,6 +1682,20 @@ int ccb_caption_dataset(ccb_ctx* c, const ccb_gen_params* p, const void* images,
   if (fence_in(c, caller)) return -1;
   const int r = caption_dataset_on_work_stream(c, p, images, dtype, n_images, rows, append_bos, first_row_id, tokens_out,
                                                lengths_out, decode_steps_out);
+  if (fence_out(c, caller)) return -1;
+  return r;
+}
+
+int ccb_caption_dataset_beam(ccb_ctx* c, const ccb_gen_params* p, const void* images, int dtype, int n_images, int groups,
+                             int append_bos, int32_t* tokens_out, int32_t* lengths_out, float* scores_out,
+                             int64_t* decode_steps_out, void* stream) {
+  if (!c || !p || !images || !tokens_out || !lengths_out || !scores_out || !decode_steps_out)
+    return fail(c, "ccb_caption_dataset_beam: null argument");
+  DeviceGuard dev_guard(c->device);
+  cudaStream_t caller = static_cast<cudaStream_t>(stream);
+  if (fence_in(c, caller)) return -1;
+  const int r = caption_dataset_beam_on_work_stream(c, p, images, dtype, n_images, groups, append_bos, tokens_out,
+                                                    lengths_out, scores_out, decode_steps_out);
   if (fence_out(c, caller)) return -1;
   return r;
 }

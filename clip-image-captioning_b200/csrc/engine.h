@@ -133,14 +133,15 @@ struct ccb_ctx {
   float* seq_lengths = nullptr;   // [max_rows]
   uint8_t* has_stopped = nullptr; // [max_rows]
   int* bos_token = nullptr;       // [max_images] scratch for the BOS embedding gather
-  // continuous batching (ccb_caption_dataset): a slot (decode row) holds one image at a time
+  // continuous batching (ccb_caption_dataset): a slot (decode row) holds one image at a time; ccb_caption_dataset_beam
+  // keeps the same per-unit state for its groups of beam rows (row_step = the group's beam steps)
   int* row_step = nullptr;        // [max_rows] tokens generated so far by the slot's image
   int* slot_image = nullptr;      // [max_rows] image index of the slot, -1 = none
   long long* slot_ids = nullptr;  // [max_rows] first_row_id + image index: the slot's Philox key
   int* refill_slots = nullptr;    // [max_rows] slots refilled at one round boundary, in refill order
   long long* refill_ids = nullptr;  // [max_images] Philox keys of one refill chunk's prefill rows
   int* refill_next = nullptr;     // [max_images] first tokens of one refill chunk
-  int** cont_out = nullptr;       // [2] the caller's tokens / lengths outputs, read by the captured rounds
+  void** cont_out = nullptr;      // [3] the caller's tokens / lengths (/ scores) outputs, read by the captured rounds
   // pinned host ring (two halves): per round the finished flags and images of the slots, per boundary the refill list
   uint8_t* h_finished = nullptr;  // [2, max_rows]
   int* h_slot_image = nullptr;    // [2, max_rows]

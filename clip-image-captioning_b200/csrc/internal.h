@@ -213,10 +213,31 @@ struct BeamState {
   int cand_rows = 0;
 };
 constexpr int kBeamCandPerRow = 8;   // == kMaxBeam of sampler.cu
+// Per-group mode of beam_step (continuous batching: group g is the beam rows [g * beam, (g+1) * beam) of one image, at
+// its own step).  Launch entry i (logits row i on a first step, rows [i * beam, (i+1) * beam) otherwise) belongs to group
+// g = slots[i] (slots null: g = i); the state arrays, block tables, ctx_len and next_tokens are indexed by g.  A group
+// whose image is < 0 or that is finished is frozen: nothing is written and neither its ctx_len nor its step advances.
+// Otherwise step = group_step[g] replaces *step; a later step counts the token the decode step has just appended
+// (ctx = ctx_len + 1 is permuted and stored), and group_step[g] = step + 1.  The group finishes when all its beams have
+// stopped or at step + 1 == max_len; it then writes out[0][image, k, :max_len] = its token rows, out[1][image, k] =
+// seq_lengths and out[2][image, k] = scores / seq_lengths (finalize_beam_kernel's values), and sets finished[g].
+struct BeamGroups {
+  int* group_step = nullptr;         // [groups] beam steps the group's image has taken
+  const int* group_image = nullptr;  // [groups] image index, -1 = none
+  uint8_t* finished = nullptr;       // [groups]
+  const int* slots = nullptr;        // [entries] or null
+  void* const* out = nullptr;        // device {tokens int [n, beam, max_len], lengths int [n, beam], scores float [n, beam]}
+};
+// dynamic shared memory beam_merge_kernel needs; beam_step refuses more than kBeamMergeMaxSmem
+constexpr size_t kBeamMergeMaxSmem = 64 * 1024;
+inline size_t beam_merge_smem(int beam, int max_len, int max_pages) {
+  return static_cast<size_t>(beam) * (max_len > max_pages ? max_len : max_pages) * sizeof(int);
+}
 int beam_step(const float* logits, long long ld, int N, int beam, int V, float temperature, int stop_token,
               const BeamState& st, int* next_tokens /*[N*beam]*/, int* src_rows /*[N*beam] global row ids*/,
               int* block_table /*[N*beam, max_pages] permuted in place, or null*/, int max_pages,
-              const int* ctx_len /*[N*beam] cached tokens per row*/, cudaStream_t s);
+              int* ctx_len /*[N*beam] cached tokens per row (advanced in per-group mode)*/, cudaStream_t s,
+              const BeamGroups* groups = nullptr);
 // Per-row mode of advance_rows (continuous batching: every row decodes its own image at its own step).  Entry i of
 // `next` belongs to row r = slots[i] (slots null: r = i).  A row whose image is < 0 or that is finished is frozen: nothing
 // is written and neither ctx_len nor its step advances.  Otherwise, with st = row_step[r]: tokens_out[r, st] (the row's
@@ -228,7 +249,7 @@ struct RowAdvance {
   const int* row_image = nullptr;   // [rows]
   const int* slots = nullptr;       // [entries of next] or null
   int* next_tokens = nullptr;       // [rows] or null
-  int* const* out = nullptr;        // device {tokens [n_images, max_len], lengths [n_images]}: caller output pointers
+  void* const* out = nullptr;       // device {tokens int [n_images, max_len], lengths int [n_images]}: caller outputs
 };
 // Per-step bookkeeping after a sampled token: tokens_out[r, *step] = next[r]; stop counting (stop_token up to
 // max_stops, eos_token) -> lengths / finished; *step += 1.  Null pointers skip the corresponding part.  With `per_row`

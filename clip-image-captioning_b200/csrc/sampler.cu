@@ -763,8 +763,15 @@ struct BeamArgs {
   int* src_rows;            // [N*beam]
   int* block_table;         // [N*beam, max_pages] permuted in place (may be null)
   int max_pages;
-  const int* ctx_len;       // [N*beam] tokens currently cached per row (entries < ctx are permuted)
+  int* ctx_len;             // [N*beam] tokens currently cached per row (entries < ctx are permuted)
+  BeamGroups grp;           // per-group mode (internal.h) when grp.group_step is non-null
 };
+
+// group of launch entry n in per-group mode (the entry itself otherwise); true when that group is frozen
+__device__ __forceinline__ bool beam_group(const BeamArgs& a, int n, int& g) {
+  g = a.grp.slots ? a.grp.slots[n] : n;
+  return a.grp.group_step && (a.grp.group_image[g] < 0 || a.grp.finished[g]);
+}
 
 // Two launches per step.  beam_rows_kernel: one CTA per (image, beam row) -- the row's log-softmax statistics and its
 // best kMaxBeam candidates (255 rows keep every SM busy where one CTA per image used 51 of 148).  beam_merge_kernel: one
@@ -777,16 +784,18 @@ __global__ void __launch_bounds__(kBeamRowThreads, 2) beam_rows_kernel(const Bea
   __shared__ Cand wcand[(kBeamRowThreads / 32) * kMaxBeam];
   const int beam = a.beam, V = a.V;
   const int n = blockIdx.x / beam, r = blockIdx.x - n * beam;
-  const int step = *a.step;
+  int g;
+  if (beam_group(a, n, g)) return;
+  const int step = a.grp.group_step ? a.grp.group_step[g] : *a.step;
   const bool first = (step == 0);
   if (first && r > 0) return;          // the first step ranks the single prefill row of the image
   Cand* out = a.cand + static_cast<long long>(blockIdx.x) * kMaxBeam;
   const float T = a.temperature > 0.f ? a.temperature : 1.0f;
   const bool unit_T = T == 1.0f;       // x / 1.0f == x: skip the division
-  const float score = first ? 0.f : a.scores[n * beam + r];
-  const bool stopped = !first && a.has_stopped[n * beam + r];
+  const float score = first ? 0.f : a.scores[g * beam + r];
+  const bool stopped = !first && a.has_stopped[g * beam + r];
   // seq_lengths[~has_stopped] += 1  (not on the first step)
-  const float len = first ? 1.f : a.seq_lengths[n * beam + r] + (stopped ? 0.f : 1.f);
+  const float len = first ? 1.f : a.seq_lengths[g * beam + r] + (stopped ? 0.f : 1.f);
   if (stopped) {
     // logits[has_stopped] = -inf; logits[has_stopped, 0] = 0  -> only token 0 is a finite candidate
     if (threadIdx.x < kMaxBeam) {
@@ -1030,14 +1039,16 @@ __global__ void __launch_bounds__(256) beam_merge_kernel(const BeamArgs a) {
   __shared__ uint8_t s_stop[kMaxBeam];
   extern __shared__ int perm_buf[];  // beam * max(max_len, max_pages) ints
   const int n = blockIdx.x;
+  int g;
+  if (beam_group(a, n, g)) return;
   const int beam = a.beam, V = a.V;
-  const int step = *a.step;
+  const int step = a.grp.group_step ? a.grp.group_step[g] : *a.step;
   const bool first = (step == 0);
   const int rows = first ? 1 : beam;
   if (threadIdx.x < beam) {
-    const uint8_t st = first ? 0 : a.has_stopped[n * beam + threadIdx.x];
+    const uint8_t st = first ? 0 : a.has_stopped[g * beam + threadIdx.x];
     s_stop[threadIdx.x] = st;
-    s_len[threadIdx.x] = first ? 1.f : a.seq_lengths[n * beam + threadIdx.x] + (st ? 0.f : 1.f);
+    s_len[threadIdx.x] = first ? 1.f : a.seq_lengths[g * beam + threadIdx.x] + (st ? 0.f : 1.f);
   }
   if (threadIdx.x == 0) {
     // merge of the rows' sorted candidate lists
@@ -1065,6 +1076,8 @@ __global__ void __launch_bounds__(256) beam_merge_kernel(const BeamArgs a) {
 
   // bookkeeping
   __shared__ int s_src[kMaxBeam], s_tok[kMaxBeam];
+  __shared__ float s_new_len[kMaxBeam], s_new_score[kMaxBeam];
+  __shared__ uint8_t s_new_stop[kMaxBeam];
   if (threadIdx.x < beam) {
     const int k = threadIdx.x;
     const Cand c = top[k];
@@ -1087,16 +1100,19 @@ __global__ void __launch_bounds__(256) beam_merge_kernel(const BeamArgs a) {
     stopped = stopped | (tok == a.stop_token ? 1 : 0);
     s_src[k] = src;
     s_tok[k] = tok;
-    a.scores[n * beam + k] = new_score;
-    a.seq_lengths[n * beam + k] = new_len;
-    a.has_stopped[n * beam + k] = stopped;
-    a.next_tokens[n * beam + k] = tok;
-    a.src_rows[n * beam + k] = n * beam + src;
+    a.scores[g * beam + k] = new_score;
+    a.seq_lengths[g * beam + k] = new_len;
+    a.has_stopped[g * beam + k] = stopped;
+    a.next_tokens[g * beam + k] = tok;
+    a.src_rows[g * beam + k] = g * beam + src;
+    s_new_stop[k] = stopped;
+    s_new_len[k] = new_len;
+    s_new_score[k] = new_score;
   }
   __syncthreads();
   // tokens = cat(tokens[src], tok)
+  int* tk = a.tokens + static_cast<long long>(g) * beam * a.max_len;
   {
-    int* tk = a.tokens + static_cast<long long>(n) * beam * a.max_len;
     if (!first) {
       for (int idx = threadIdx.x; idx < beam * step; idx += blockDim.x) perm_buf[idx] = tk[(idx / step) * a.max_len + idx % step];
       __syncthreads();
@@ -1108,10 +1124,12 @@ __global__ void __launch_bounds__(256) beam_merge_kernel(const BeamArgs a) {
     if (threadIdx.x < beam && step < a.max_len) tk[threadIdx.x * a.max_len + step] = s_tok[threadIdx.x];
   }
   // block tables: row k inherits the cached-token entries of its source row
+  // (in per-group mode including the token the decode step has just appended: ctx_len has not been advanced yet)
+  int ctx = 0;
   if (!first && a.block_table != nullptr) {
     __syncthreads();
-    const int ctx = a.ctx_len[n * beam];
-    int* bt = a.block_table + static_cast<long long>(n) * beam * a.max_pages;
+    ctx = a.ctx_len[g * beam] + (a.grp.group_step ? 1 : 0);
+    int* bt = a.block_table + static_cast<long long>(g) * beam * a.max_pages;
     for (int idx = threadIdx.x; idx < beam * ctx; idx += blockDim.x) perm_buf[idx] = bt[(idx / ctx) * a.max_pages + idx % ctx];
     __syncthreads();
     for (int idx = threadIdx.x; idx < beam * ctx; idx += blockDim.x) {
@@ -1119,6 +1137,23 @@ __global__ void __launch_bounds__(256) beam_merge_kernel(const BeamArgs a) {
       bt[k * a.max_pages + t] = perm_buf[s_src[k] * ctx + t];
     }
   }
+  if (a.grp.group_step == nullptr) return;
+  // per-group mode: advance the group; at its end (generate_beam's `if has_stopped.all(): break`, inference.py:70-148,
+  // or max_len tokens) hand its beams to the caller's outputs
+  __syncthreads();
+  if (!first && threadIdx.x < beam) a.ctx_len[g * beam + threadIdx.x] = ctx;
+  if (threadIdx.x == 0) a.grp.group_step[g] = step + 1;
+  bool all_stopped = true;
+  for (int k = 0; k < beam; ++k) all_stopped = all_stopped && s_new_stop[k];
+  if (!all_stopped && step + 1 < a.max_len) return;
+  const int img = a.grp.group_image[g];
+  int* out_tokens = static_cast<int*>(a.grp.out[0]) + static_cast<long long>(img) * beam * a.max_len;
+  for (int idx = threadIdx.x; idx < beam * a.max_len; idx += blockDim.x) out_tokens[idx] = tk[idx];
+  if (threadIdx.x < beam) {
+    static_cast<int*>(a.grp.out[1])[img * beam + threadIdx.x] = static_cast<int>(s_new_len[threadIdx.x]);
+    static_cast<float*>(a.grp.out[2])[img * beam + threadIdx.x] = s_new_score[threadIdx.x] / s_new_len[threadIdx.x];
+  }
+  if (threadIdx.x == 0) a.grp.finished[g] = 1;
 }
 
 // ------------------------------------------------------------------------------------------------ bookkeeping
@@ -1151,8 +1186,8 @@ __global__ void advance_rows_kernel(const int* __restrict__ next, int n, int* hi
                                     const RowAdvance ra) {
   ptx::grid_dep_wait();
   ptx::grid_dep_launch();
-  int* out_tokens = ra.out[0];
-  int* out_lengths = ra.out[1];
+  int* out_tokens = static_cast<int*>(ra.out[0]);
+  int* out_lengths = static_cast<int*>(ra.out[1]);
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     const int r = ra.slots ? ra.slots[i] : i;
     const int img = ra.row_image[r];
@@ -1223,7 +1258,7 @@ int sample_top_p(const float* logits, long long ld, int B, int V, const SamplePa
 
 int beam_step(const float* logits, long long ld, int N, int beam, int V, float temperature, int stop_token,
               const BeamState& st, int* next_tokens, int* src_rows, int* block_table, int max_pages,
-              const int* ctx_len, cudaStream_t s) {
+              int* ctx_len, cudaStream_t s, const BeamGroups* groups) {
   if (N <= 0) return 0;
   if (beam < 1 || beam > kMaxBeam) return (int)cudaErrorInvalidValue;
   BeamArgs a;
@@ -1231,15 +1266,19 @@ int beam_step(const float* logits, long long ld, int N, int beam, int V, float t
   a.scores = st.scores; a.seq_lengths = st.seq_lengths; a.has_stopped = st.has_stopped; a.tokens = st.tokens;
   a.max_len = st.max_len; a.step = st.step; a.next_tokens = next_tokens; a.src_rows = src_rows;
   a.block_table = block_table; a.max_pages = max_pages; a.ctx_len = ctx_len;
+  if (groups) {
+    if (!groups->group_step || !groups->group_image || !groups->finished || !groups->out || !block_table || !ctx_len)
+      return (int)cudaErrorInvalidValue;
+    a.grp = *groups;
+  }
   if (st.cand_scratch == nullptr || st.cand_rows < N * beam) return (int)cudaErrorInvalidValue;
   a.cand = static_cast<Cand*>(st.cand_scratch);
-  const int m = st.max_len > max_pages ? st.max_len : max_pages;
-  const size_t smem = static_cast<size_t>(beam) * m * sizeof(int);
-  if (smem > 64 * 1024) return (int)cudaErrorInvalidValue;
+  const size_t smem = beam_merge_smem(beam, st.max_len, max_pages);
+  if (smem > kBeamMergeMaxSmem) return (int)cudaErrorInvalidValue;
   static bool configured_dev[kMaxDevices] = {};
   bool& configured = configured_dev[current_device_slot()];
   if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(beam_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(beam_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kBeamMergeMaxSmem));
     if (e != cudaSuccess) return (int)e;
     configured = true;
   }

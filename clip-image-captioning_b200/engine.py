@@ -468,6 +468,31 @@ class Engine:
         self._keep = [images, p]
         return tokens, lengths, int(steps.value)
 
+    def caption_dataset_continuous_beam(self, images: torch.Tensor, p: GenParams, groups: Optional[int] = None,
+                                        append_bos: int = -1):
+        """`caption_dataset` in beam mode with continuous batching (ccb_caption_dataset_beam): `groups` images (default
+        `micro_batch_for(p)`) are in flight with beam_size decode rows each, and an image whose beams have all stopped,
+        or that has max_new_tokens tokens, gives its group to the next image (generate_beam, inference.py:70-148, stops
+        there too).  Returns (tokens [n, beam, T], lengths [n, beam], scores [n, beam], decode steps run), the layout of
+        `caption_dataset` in beam mode; positions past a beam's length are 0.  Synchronises the host once per round of
+        decode steps."""
+        images = self._dev(images)
+        if images.dtype not in _TORCH_DTYPE:
+            images = images.float()
+        n = images.shape[0]
+        groups = groups or self.micro_batch_for(p)
+        # (non-empty even for the arguments the library rejects, so that it names the reason)
+        beam, T = max(p.beam_size, 1), max(p.max_new_tokens, 1)
+        tokens = torch.empty(n, beam, T, device=self.device, dtype=torch.int32)
+        lengths = torch.empty(n, beam, device=self.device, dtype=torch.int32)
+        scores = torch.empty(n, beam, device=self.device, dtype=torch.float32)
+        steps = C.c_int64()
+        self._check(self.lib.ccb_caption_dataset_beam(self._h, C.byref(p), _ptr(images), _TORCH_DTYPE[images.dtype], n,
+                                                      groups, append_bos, _ptr(tokens), _ptr(lengths), _ptr(scores),
+                                                      C.byref(steps), self._stream()))
+        self._keep = [images, p]
+        return tokens, lengths, scores, int(steps.value)
+
     # ------------------------------------------------------------------------------------------ samplers
     def sample(self, logits: torch.Tensor, p: GenParams, history: Optional[torch.Tensor] = None, step: int = 0,
                return_filtered: bool = False, return_alt: bool = False):

@@ -11,7 +11,7 @@
  *   - every data pointer is a DEVICE pointer to a contiguous row-major tensor owned by the caller (PyTorch);
  *     the library never frees caller memory and allocates only inside ccb_create.
  *   - every call is asynchronous on `stream` (a cudaStream_t passed as void*); no host synchronisation except
- *     where stated (ccb_caption_dataset, ccb_beam_step).  A ccb_ctx is bound to one device and is not thread-safe (one ctx per rank / GPU).
+ *     where stated (ccb_caption_dataset, ccb_caption_dataset_beam, ccb_beam_step).  A ccb_ctx is bound to one device and is not thread-safe (one ctx per rank / GPU).
  *   - there is no CPU fallback: without an sm_100 device ccb_create fails.
  */
 #ifndef CLIPCAP_B200_H_
@@ -167,6 +167,23 @@ CCB_API int ccb_caption_images(ccb_ctx* ctx, const ccb_gen_params* params, const
 CCB_API int ccb_caption_dataset(ccb_ctx* ctx, const ccb_gen_params* params, const void* images, int dtype, int n_images,
                                 int rows, int append_bos, int64_t first_row_id, int32_t* tokens_out, int32_t* lengths_out,
                                 int64_t* decode_steps_out, void* stream);
+/* A whole shard of images -> beam-search captions with continuous batching (generate_beam, inference.py:70-148, per
+ * image): `groups` images are in flight, each holding beam_size decode rows, and an image's group takes the next image
+ * once all of its beams have stopped (the reference's `if has_stopped.all(): break`) or it has produced max_new_tokens
+ * tokens.  images [n_images, 3, H, W] (device); in image order (device): tokens_out [n_images, beam, max_new_tokens] int32,
+ * lengths_out [n_images, beam] (seq_lengths), scores_out [n_images, beam] (scores / seq_lengths, inference.py:138), the
+ * layout of ccb_caption_images in beam mode: the caller picks argmax like inference.py:143-144.  Positions past a beam's
+ * length are 0.  *decode_steps_out (HOST) = decode steps run.
+ * The call synchronises the host once per round of a few decode steps, to learn which groups have finished; it returns
+ * once the last round has completed.  ccb_last_timing / ccb_timing_sum do not count it.  max_stops, eos_token, seed
+ * and the sampling fields are ignored, as ccb_generate ignores them in beam mode.
+ * Rejected with a message, nothing launched: a mode other than beam, beam_size outside [1, min(max_beam, 8)], groups
+ * outside [1, max_images], map_prefix_len (+ 1 with append_bos >= 0) + max_new_tokens above max_ctx, the prefix shapes
+ * ccb_caption_images rejects, and beam_size * max(max_new_tokens, max_ctx) * 4 bytes above the 64 KB of shared memory
+ * of the beam merge. */
+CCB_API int ccb_caption_dataset_beam(ccb_ctx* ctx, const ccb_gen_params* params, const void* images, int dtype,
+                                     int n_images, int groups, int append_bos, int32_t* tokens_out, int32_t* lengths_out,
+                                     float* scores_out, int64_t* decode_steps_out, void* stream);
 /* number of kernels launched by the library on this context since creation (CUDA-graph replays count the
  * kernels inside the graph) */
 CCB_API int64_t ccb_launch_count(const ccb_ctx* ctx);
